@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the hot path on synthetic Pfam-shaped data (BASELINE.json config 3).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one counting pass over one batch: bucket table + LG transition histogram of
 F families x 1024 sequences x 300 sites into K=100 time buckets (+ the all-reduce of the raw
@@ -9,6 +9,10 @@ integer histogram when N > 1, + symmetrisation).  Per-GPU work is fixed (weak sc
 rank counts its own F families).  ``value`` = transitions examined per second with the batch
 resident in HBM; ``e2e`` = the same through the host-buffer C-ABI entry point
 (pinned host arrays -> H2D -> kernels -> D2H).  One JSON line is printed by rank 0.
+
+``--dump-outputs DIR`` writes what the last timed step returned, the symmetrised fp64 count
+tensor [K, 20, 20] (320 KB), as ``DIR/counts.npy``.  The batch is generated from a fixed seed, so
+two builds run with the same arguments can be compared output for output.
 
 ``--impl reference`` times the reference's own CPU implementation (the unmodified C++
 program compiled into oracle/_ref, one process per host core on the reference's own family
@@ -63,7 +67,14 @@ def parse_args():
     ap.add_argument("--no-likelihood", action="store_true")
     ap.add_argument("--no-siterm", action="store_true")
     ap.add_argument("--no-public-api", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output of the last timed step to DIR/counts.npy (--impl ours)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def workload_name(families):
@@ -387,6 +398,10 @@ def run_ours(args):
     value = examined * world / (ms_per_step * 1e-3)
     _log(f"timed steps done: {ms_per_step:.3f} ms per step")
     counted = float(counts.sum().item())
+    if args.dump_outputs is not None and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "counts.npy"), counts.cpu().numpy())
+        _log(f"outputs of the last timed step written to {args.dump_outputs}")
 
     # ---- strong scaling (BASELINE config 3 as stated: 16k families in total on 1/2/4/8 GPUs): the SAME
     # step, all-reduce inside, on F/N families per rank (the first 1/N of this rank's resident tiles)

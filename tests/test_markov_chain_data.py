@@ -10,6 +10,8 @@ from cherryml_b200 import markov_chain as mc
 from cherryml_b200.utils import amino_acids
 
 REF_DATA = "/root/reference/data/rate_matrices"
+# byte copies of the reference's data/rate_matrices/lg.txt and equ.txt (tests/golden/make_golden_fit.py)
+REF_COPIES = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fit", "inputs")
 PAIRS = [a + b for a in amino_acids for b in amino_acids]
 
 
@@ -37,6 +39,13 @@ def test_derived_files_are_consistent_with_their_matrices():
     w = mc.wag_matrix().to_numpy()
     assert abs(mc.compute_mutation_rate(w) - 1.0) < 1e-12
     assert abs(float(mc.wag_stationary_distribution().to_numpy().sum()) - 1.0) < 1e-12
+
+
+def test_values_equal_stored_copies_of_the_reference_data_files():
+    for mine, ref in ((mc.get_lg_path(), "lg.txt"), (mc.get_equ_path(), "equ.txt")):
+        a, b = io.read_rate_matrix(mine), io.read_rate_matrix(os.path.join(REF_COPIES, ref))
+        assert list(a.index) == list(b.index) and list(a.columns) == list(b.columns)
+        assert np.array_equal(a.to_numpy(), b.to_numpy())
 
 
 @pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="the reference checkout is only present in the build container")
