@@ -19,12 +19,8 @@ int check_args(const cherry_fit_args* a, bool training) {
 
 int one_epoch(const cherry_fit_args& a, cudaStream_t stream) {
   int rc;
-  if (a.S <= cherry::kSmallFitMaxS) {
-    // ONE launch per epoch: the last CTA of every problem runs its parameter update (fit_small.cu)
-    static const bool no_fuse = getenv("CHERRY_FIT_SMALL_UNFUSED") != nullptr;  // A/B switch
-    if ((rc = cherry::fit_small_expm(a, stream, nullptr, !no_fuse))) return rc;
-    return no_fuse ? cherry::fit_small_update(a, 1, stream) : 0;
-  }
+  // S <= 32: ONE launch per epoch, the last CTA of every problem runs its parameter update (fit_small.cu)
+  if (a.S <= cherry::kSmallFitMaxS) return cherry::fit_small_expm(a, stream, nullptr, true);
   if ((rc = cherry::fit_large_expm(a, stream, true))) return rc;
   return cherry::fit_large_update(a, 1, stream);
 }

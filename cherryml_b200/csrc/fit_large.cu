@@ -40,8 +40,11 @@ constexpr double kTheta = 2.2;    // tau*mu bound: 2.2^25/25! ~ 2e-17 (all terms
 constexpr int kSStore = 8;        // squarings kept per bucket: covers t*mu up to 2.2 * 2^8 = 563
 constexpr int BT = 80, BK = 16, NSTAGE = 2;  // two stages (51 KB per CTA): THREE CTAs share an SM; three stages with two CTAs
                                               // measured 0.851 ms per epoch against 0.820 (gpurun_out/r02_fit_stage2_sweep.txt)
-constexpr int KGROUPS = 1;  // >1: warp groups split every k chunk (lower tile latency, measured 30% less throughput)
-constexpr int GEMM_THREADS = 128 * KGROUPS;
+constexpr int GEMM_THREADS = 128;  // 4 warps, one 40x40 quadrant of the tile each
+constexpr int kCtasPerSm = 3;      // persistent grids of the tile kernels: 2-stage pipeline, 51 KB and ~20 K registers per CTA
+// split-K cap of the squaring kernels (graph-replayed epochs, general form, 25 tiles per product: 1 -> 1.04 ms,
+// 2 -> 0.94, 5 -> 0.96; symmetric form, 15 tiles: 2 -> 0.764, 3 -> 0.741, 4 -> 0.744, 6 -> 0.749)
+constexpr int kSqKsplitGeneral = 2, kSqKsplitSym = 3;
 constexpr int LD_ROW = 20;        // tile stored [80][16]: k contiguous
 constexpr int LD_COL = 84;        // tile stored [16][80]: m (or n) contiguous
 constexpr int TILE_ELEMS = BT * LD_ROW;  // 1600 >= 16 * 84
@@ -50,8 +53,7 @@ constexpr int kTaylorStagesS = 16;     // count loads in flight per thread of it
 constexpr int kTaylorThreads = 256;    // threads per CTA of the shared-memory variant of the fused Taylor pass (288 would make
                                        // 160 000 elements two passes of 296 CTAs instead of 2.11, but needs <= 113 registers: 96 with
                                        // 300 bytes of spills measured 213 us against 180)
-constexpr int kTaylorTailUnits = 2560;  // (chunk, share) CTAs of the split shared-memory Taylor pass (625 chunks x 4)
-constexpr int kTaylorParts = 1;         // default split (1: persistent, every chunk one CTA)
+constexpr int kTaylorTailUnits = 512;   // (chunk, share) CTAs of the tail split: at most 2 CTAs per SM (296 on a B200)
 constexpr int kTaylorInterleave = 2;  // buckets whose dependent chains a thread of the fused Taylor pass interleaves
 constexpr int kTaylorStages = 16;  // count loads in flight per thread of the fused Taylor pass
 static_assert(kDeg % 4 == 0, "the elementwise kernels skip Taylor terms in blocks of four");
@@ -63,13 +65,7 @@ struct GemmTerm {
 };
 struct GemmTask {
   double* C;
-  const int* cond;  // active iff cond == nullptr || *cond > level
-  int term_begin, n_terms, accumulate, level;
-  int ksplit = 0;        // > 0: this task's own split-K factor (<= the launch's grid.z)
-  int partial_off = -1;  // >= 0: index of this task's first partial matrix (else blockIdx.y * ksplit)
-};
-struct Group {
-  int task_begin, n_tasks, ksplit;
+  int term_begin, n_terms, accumulate;
 };
 
 __device__ __forceinline__ void dmma884(double& d0, double& d1, double a, double b) {
@@ -102,10 +98,9 @@ __device__ __forceinline__ void load_col_tile(double* s, const double* g, int ld
 
 template <bool TA, bool TB>
 __device__ __forceinline__ void compute_chunk(const double* As, const double* Bs, double (&acc)[5][5][2],
-                                              int rbase, int cbase, int g, int tg, int kgroup) {
+                                              int rbase, int cbase, int g, int tg) {
 #pragma unroll
-  for (int kq = 0; kq < BK / 4 / KGROUPS; ++kq) {
-    const int kk = (kq * KGROUPS + kgroup) * 4;  // this warp group's k-steps of the chunk
+  for (int kk = 0; kk < BK; kk += 4) {
     double a[5], b[5];
 #pragma unroll
     for (int i = 0; i < 5; ++i) {
@@ -138,8 +133,7 @@ __device__ __forceinline__ void gemm_tile(TermFn get_term, int Sp, int m0, int n
   if (ld_out == 0) ld_out = Sp;
   const int cpt = Sp / BK;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, tg = lane & 3;
-  const int kgroup = warp >> 2, wq = warp & 3;  // 4 warps (2x2 quadrants of 40x40) per k group
-  const int rbase = (wq >> 1) * 40, cbase = (wq & 1) * 40;
+  const int rbase = (warp >> 1) * 40, cbase = (warp & 1) * 40;  // 4 warps: 2x2 quadrants of 40x40
   double acc[5][5][2];
 #pragma unroll
   for (int i = 0; i < 5; ++i)
@@ -169,39 +163,14 @@ __device__ __forceinline__ void gemm_tile(TermFn get_term, int Sp, int m0, int n
     const double* As = smem + (size_t)(i % NSTAGE) * 2 * TILE_ELEMS;
     const double* Bs = As + TILE_ELEMS;
     if (t.ta) {
-      if (t.tb) compute_chunk<true, true>(As, Bs, acc, rbase, cbase, g, tg, kgroup);
-      else compute_chunk<true, false>(As, Bs, acc, rbase, cbase, g, tg, kgroup);
+      if (t.tb) compute_chunk<true, true>(As, Bs, acc, rbase, cbase, g, tg);
+      else compute_chunk<true, false>(As, Bs, acc, rbase, cbase, g, tg);
     } else {
-      if (t.tb) compute_chunk<false, true>(As, Bs, acc, rbase, cbase, g, tg, kgroup);
-      else compute_chunk<false, false>(As, Bs, acc, rbase, cbase, g, tg, kgroup);
+      if (t.tb) compute_chunk<false, true>(As, Bs, acc, rbase, cbase, g, tg);
+      else compute_chunk<false, false>(As, Bs, acc, rbase, cbase, g, tg);
     }
   }
   cp_async_wait<0>();
-  if (KGROUPS > 1) {
-    // fold the k groups: groups 1.. park their accumulators in the (now idle) pipeline buffers,
-    // group 0 adds them.  Layout [value][thread of group] keeps the accesses conflict free.
-    __syncthreads();
-    double* park = smem;  // 50 * 128 doubles = 51 KB <= NSTAGE * 2 * TILE_ELEMS * 8 B
-    const int tq = threadIdx.x & 127;
-    if (kgroup == 1) {
-#pragma unroll
-      for (int i = 0; i < 5; ++i)
-#pragma unroll
-        for (int j = 0; j < 5; ++j) {
-          park[((i * 5 + j) * 2 + 0) * 128 + tq] = acc[i][j][0];
-          park[((i * 5 + j) * 2 + 1) * 128 + tq] = acc[i][j][1];
-        }
-    }
-    __syncthreads();
-    if (kgroup != 0) return;
-#pragma unroll
-    for (int i = 0; i < 5; ++i)
-#pragma unroll
-      for (int j = 0; j < 5; ++j) {
-        acc[i][j][0] += park[((i * 5 + j) * 2 + 0) * 128 + tq];
-        acc[i][j][1] += park[((i * 5 + j) * 2 + 1) * 128 + tq];
-      }
-  }
 #pragma unroll
   for (int i = 0; i < 5; ++i)
 #pragma unroll
@@ -227,55 +196,17 @@ __device__ __forceinline__ void gemm_tile(TermFn get_term, int Sp, int m0, int n
 // writes its partial product to `partial[(task*ksplit + z)]` and splitk_reduce_kernel finishes.
 __global__ void __launch_bounds__(GEMM_THREADS)
 gemm_tasks_kernel(const GemmTask* __restrict__ tasks, const GemmTerm* __restrict__ terms, int Sp,
-                  int ksplit, double* __restrict__ partial, int* __restrict__ arrive) {
+                  int ksplit, double* __restrict__ partial) {
   extern __shared__ double smem[];
-  __shared__ int s_last;
   const GemmTask task = tasks[blockIdx.y];
-  if (task.cond != nullptr && *task.cond <= task.level) return;
   const int tiles_n = Sp / BT;
   const int m0 = (blockIdx.x / tiles_n) * BT, n0 = (blockIdx.x % tiles_n) * BT;
   const int total = task.n_terms * (Sp / BK);
   const int z = blockIdx.z;
-  const int launch_ksplit = ksplit;
-  if (task.ksplit > 0) ksplit = task.ksplit;  // tasks of one launch may split K differently
-  if (z >= ksplit) return;
-  const size_t pbase = task.partial_off >= 0 ? (size_t)task.partial_off : (size_t)blockIdx.y * launch_ksplit;
   const int c_begin = (int)((long long)total * z / ksplit), c_end = (int)((long long)total * (z + 1) / ksplit);
-  double* out = (ksplit == 1) ? task.C : partial + (pbase + z) * (size_t)Sp * Sp;
+  double* out = (ksplit == 1) ? task.C : partial + ((size_t)blockIdx.y * ksplit + z) * (size_t)Sp * Sp;
   gemm_tile([&](int idx) { return terms[task.term_begin + idx]; }, Sp, m0, n0, c_begin, c_end, smem, out,
             (ksplit == 1) && task.accumulate);
-  if (ksplit == 1 || arrive == nullptr) return;
-  // Split-K without a second launch: the CTA that arrives last at this tile adds the ksplit
-  // partial tiles in z order (so the result does not depend on who is last) and writes C.
-  __threadfence();
-  __syncthreads();
-  int* ctr = arrive + blockIdx.y * gridDim.x + blockIdx.x;
-  if (threadIdx.x == 0) {
-    const int old = atomicAdd(ctr, 1);
-    s_last = (old == ksplit - 1);
-    if (s_last) *ctr = 0;  // ready for the next launch
-  }
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  const size_t n_p = (size_t)Sp * Sp;
-  const double* base = partial + pbase * n_p;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, tg = lane & 3;
-  const int wq = warp & 3, rbase = (wq >> 1) * 40, cbase = (wq & 1) * 40;
-  if (warp >= 4) return;
-#pragma unroll
-  for (int i = 0; i < 5; ++i)
-#pragma unroll
-    for (int j = 0; j < 5; ++j) {
-      const size_t pos = (size_t)(m0 + rbase + 8 * i + g) * Sp + n0 + cbase + 8 * j + 2 * tg;
-      double2 v = task.accumulate ? *reinterpret_cast<const double2*>(task.C + pos) : make_double2(0.0, 0.0);
-      for (int zz = 0; zz < ksplit; ++zz) {
-        const double2 pz = __ldcg(reinterpret_cast<const double2*>(base + (size_t)zz * n_p + pos));
-        v.x += pz.x;
-        v.y += pz.y;
-      }
-      *reinterpret_cast<double2*>(task.C + pos) = v;
-    }
 }
 
 // ----------------------------------------------------------- dataflow squaring chains
@@ -301,7 +232,7 @@ __device__ __forceinline__ int* sq_done_fwd(SqSchedule* s, int K) { return sq_ac
 __device__ __forceinline__ int* sq_done_bwd(SqSchedule* s, int K) { return sq_done_fwd(s, K) + kSStore * K; }
 __device__ __forceinline__ int* sq_rank(SqSchedule* s, int K) { return sq_done_bwd(s, K) + (kSStore + 1) * K; }
 __device__ __forceinline__ int* sq_tile_arrive(SqSchedule* s, int K) { return sq_rank(s, K) + K; }
-constexpr int kSqPartialSlots = 96;  // matrices in the split-K partial buffer (Plan::n_partial)
+constexpr int kSqPartialSlots = 96;  // matrices of the split-K partial buffer (Plan::off_partial) the squarings may use
 
 // Bounded spin (about a second): a scheduling bug must surface as an error flag, not as a hung GPU.
 __device__ __forceinline__ void wait_counter(const int* ctr, int target, int* status_flag) {
@@ -495,8 +426,10 @@ __host__ __device__ inline size_t df_state_ints(int n_mats, int tiles, int n_gro
 }
 constexpr int kDfReduceLag = 1 << 20;  // groups between a product and its reduction items in the queue: effectively "all
                                         // of a level's products first, then its reductions" -- sweeps of 10..1000 groups
-                                        // (gpurun_out/r02_fit_reduce_lag_sweep.txt, r02_fit_chain_sweep2/3.txt): a reduction
-                                        // taken before its products are done idles a CTA that could have run a product
+                                        // (profiles/timelines/r02_fit_reduce_lag_sweep.txt, r02_fit_chain_sweep2/3.txt): a
+                                        // reduction taken before its products are done idles a CTA that could have run a product
+constexpr int kDfChainTarget = 500;  // work items per level of a power chain (sweeps 300..4000:
+                                     // profiles/timelines/r02_fit_chain_target_sweep.txt, r02_fit_chain_sweep3.txt)
 
 __device__ __forceinline__ void df_wait_tile(const int* v, int target, int* status_flag) {
   unsigned spins = 0;
@@ -664,15 +597,11 @@ chain_dataflow_kernel(const DfItem* __restrict__ items, int n_items, int n_group
   }
 }
 
-// grid = (blocks over elements, n_tasks): C = (accumulate ? C : 0) + sum_z partial[task][z], z ascending
+// grid = (blocks over elements, n_tasks), ksplit > 1: C = (accumulate ? C : 0) + sum_z partial[task][z], z ascending
 __global__ void splitk_reduce_kernel(const GemmTask* __restrict__ tasks, int ksplit, size_t n_p,
                                      const double* __restrict__ partial) {
   const GemmTask task = tasks[blockIdx.y];
-  if (task.cond != nullptr && *task.cond <= task.level) return;
-  const size_t pbase = task.partial_off >= 0 ? (size_t)task.partial_off : (size_t)blockIdx.y * ksplit;
-  if (task.ksplit > 0) ksplit = task.ksplit;
-  if (ksplit == 1) return;  // the GEMM wrote (or accumulated into) C itself
-  const double* base = partial + pbase * n_p;
+  const double* base = partial + (size_t)blockIdx.y * ksplit * n_p;
   for (size_t e = blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < n_p; e += (size_t)gridDim.x * blockDim.x) {
     double v = task.accumulate ? task.C[e] : 0.0;
     for (int z = 0; z < ksplit; ++z) v += base[(size_t)z * n_p + e];
@@ -724,7 +653,7 @@ __global__ void coef_kernel(const double* __restrict__ t, int K, LargeScalars* _
                             double* __restrict__ tau_arr,
                             int* __restrict__ status_flag, SqSchedule* __restrict__ sched, int tiles,
                             int n_ctas, int* __restrict__ df_state_fwd, int n_fwd_ints,
-                            int* __restrict__ df_state_bwd, int n_bwd_ints, int full_degree, int sq_ksplit_max) {
+                            int* __restrict__ df_state_bwd, int n_bwd_ints, int sq_ksplit_max) {
   // the power chains' queues, tile versions and arrival counters start every epoch at zero
   for (int i = threadIdx.x; i < n_fwd_ints; i += blockDim.x) df_state_fwd[i] = 0;
   for (int i = threadIdx.x; i < n_bwd_ints; i += blockDim.x) df_state_bwd[i] = 0;
@@ -751,7 +680,6 @@ __global__ void coef_kernel(const double* __restrict__ t, int K, LargeScalars* _
         term *= x / (double)(d + 2);
       }
     }
-    if (full_degree) d = kDeg;
     deg_arr[k] = d;
     const double e = exp(-tau * mu);
     double c = e;
@@ -856,25 +784,7 @@ poly_eval_kernel(const double* __restrict__ powers, size_t n_p, int S, int Sp, i
   }
 }
 
-// One (element, bucket) of the fused Taylor pass with the first D Taylor terms: value, loss term, and the
-// bucket's contribution to the power adjoints.  LPE lanes share an element: lane h owns the powers
-// j = h, h + LPE, ... (NP = kDeg / LPE of them, in pw / acc), the value is summed over the lanes of the element.
-template <int D, int LPE>
-__device__ __forceinline__ void taylor_term(const double* __restrict__ wk, const double (&pw)[kDeg / LPE],
-                                            double (&acc)[kDeg / LPE], double c, double diag, int h, double& part) {
-  double v = h == 0 ? wk[0] * diag : 0.0;
-#pragma unroll
-  for (int i = 0; i < D / LPE; ++i) v = fma(wk[i * LPE + h + 1], pw[i], v);
-#pragma unroll
-  for (int o = 1; o < LPE; o <<= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  const bool live = c != 0.0;  // with LPE > 1 the whole warp comes here if any of its elements has a count
-  if (live && h == 0) part -= c * log(v);
-  const double g = live ? -c / v : 0.0;
-#pragma unroll
-  for (int i = 0; i < D / LPE; ++i) acc[i] = fma(wk[i * LPE + h + 1], g, acc[i]);
-}
-
-// Several buckets at once (LPE = 1): the polynomial, the logarithm and the quotient of one (element, bucket) are
+// Several buckets at once: the polynomial, the logarithm and the quotient of one (element, bucket) are
 // ONE dependent chain of ~60 FP64 operations, and the pass runs 8 warps per SM (178 registers), so a bucket at a
 // time leaves the FP64 pipe idle for most of every operation's latency (issue slots 25 % busy, r02_taylor_fused_v1).
 // kTaylorInterleave independent chains interleave (four of them spill: 255 registers).  The weights beyond a bucket's degree are zero, so the four share the
@@ -934,9 +844,10 @@ __device__ __forceinline__ void taylor_term_n_s(const double* const (&w)[U], con
   }
 }
 
-// Fused Taylor pass (training): LPE lanes per matrix element, the m power values split over their registers
-// (one thread per element holds 48 doubles of state = 186 registers = one 256-thread block per SM: the pass
-// was latency bound at 12 % of the warp slots, profiles/r02_taylor_fused_v1.txt).
+// Fused Taylor pass (training), one thread per matrix element with its m power values in registers (48 doubles
+// of state = 186 registers = one 256-thread block per SM: the pass was latency bound at 12 % of the warp slots,
+// profiles/r02_taylor_fused_v1.txt).  taylor_fused_smem_kernel is the same pass with the powers in shared memory;
+// this variant runs where two CTAs' weight tables do not fit an SM (large K).
 //   buckets WITHOUT squarings (most of them): P_k(e) is the polynomial itself, so the loss term
 //     and the bucket's whole contribution to the power adjoints, Pbar_j(e) += w[k][j] * (-C/P),
 //     are formed on the spot -- nothing is stored per bucket, and an element with C_k(e) == 0
@@ -944,13 +855,12 @@ __device__ __forceinline__ void taylor_term_n_s(const double* const (&w)[U], con
 //   buckets WITH squarings: X0_k(e) is stored for the squaring chain.
 // Outputs: Pbar_j (j = 1..m) initialised with the no-squaring buckets' contributions, X0 of
 // the squared buckets, one loss partial per block.
-template <int LPE, int UI>
 __global__ void __launch_bounds__(EW_THREADS)
 taylor_fused_kernel(const double* __restrict__ powers, size_t n_p, int S, int Sp, int K,
                     const double* __restrict__ w, const int* __restrict__ s_arr,
                     const int* __restrict__ deg_arr, const double* __restrict__ C, double* __restrict__ X0,
                     double* __restrict__ Pbar, double* __restrict__ loss_partial_fused) {
-  constexpr int NP = kDeg / LPE;
+  constexpr int U = kTaylorInterleave;
   extern __shared__ double sw[];  // [K][m+1] weights, then int lists
   __shared__ double red[EW_THREADS / 32];
   __shared__ int n_zero, n_sq;
@@ -969,20 +879,19 @@ taylor_fused_kernel(const double* __restrict__ powers, size_t n_p, int S, int Sp
   }
   __syncthreads();
   // persistent: the weight table and the lists are staged once per CTA, the CTA walks over chunks of elements
-  const size_t n_chunks = (n_p * LPE + blockDim.x - 1) / blockDim.x;
+  const size_t n_chunks = (n_p + blockDim.x - 1) / blockDim.x;
   double part = 0.0;
   for (size_t chunk = blockIdx.x; chunk < n_chunks; chunk += gridDim.x) {
-    const int h = threadIdx.x & (LPE - 1);
-    const size_t e = (chunk * (size_t)blockDim.x + threadIdx.x) / LPE;
+    const size_t e = chunk * (size_t)blockDim.x + threadIdx.x;
     const bool in_range = e < n_p;
     const size_t ee = in_range ? e : 0;
     const int row = (int)(ee / Sp), col = (int)(ee - (size_t)row * Sp);
     const bool real = in_range && row < S && col < S;
     const double diag = (row == col && row < S) ? 1.0 : 0.0;
-    double pw[NP], acc[NP];
+    double pw[kDeg], acc[kDeg];
 #pragma unroll
-    for (int i = 0; i < NP; ++i) {
-      pw[i] = in_range ? powers[(size_t)(i * LPE + h) * n_p + ee] : 0.0;
+    for (int i = 0; i < kDeg; ++i) {
+      pw[i] = in_range ? powers[(size_t)i * n_p + ee] : 0.0;
       acc[i] = 0.0;
     }
     const size_t cidx = (size_t)row * S + col;
@@ -1000,66 +909,45 @@ taylor_fused_kernel(const double* __restrict__ powers, size_t n_p, int S, int Sp
     };
 #pragma unroll
     for (int i = 0; i < kTaylorStages; ++i) issue(i);
-    if constexpr (LPE == 1) {
-      constexpr int U = UI;
-      for (int i = 0; i < n_zero; i += U) {
-        cp_async_wait<kTaylorStages - U>();
-        double c[U];
+    for (int i = 0; i < n_zero; i += U) {
+      cp_async_wait<kTaylorStages - U>();
+      double c[U];
 #pragma unroll
-        for (int u = 0; u < U; ++u)
-          c[u] = (real && i + u < n_zero) ? ring[((i + u) % kTaylorStages) * EW_THREADS + threadIdx.x] : 0.0;
+      for (int u = 0; u < U; ++u)
+        c[u] = (real && i + u < n_zero) ? ring[((i + u) % kTaylorStages) * EW_THREADS + threadIdx.x] : 0.0;
 #pragma unroll
-        for (int u = 0; u < U; ++u) issue(i + u + kTaylorStages);  // the slots just read are this thread's own
-        bool nz = false;
+      for (int u = 0; u < U; ++u) issue(i + u + kTaylorStages);  // the slots just read are this thread's own
+      bool nz = false;
 #pragma unroll
-        for (int u = 0; u < U; ++u) nz |= c[u] != 0.0;
-        if (!__any_sync(0xffffffffu, nz)) continue;
-        const double* wu[U];
-        int d = 0;
+      for (int u = 0; u < U; ++u) nz |= c[u] != 0.0;
+      if (!__any_sync(0xffffffffu, nz)) continue;
+      const double* wu[U];
+      int d = 0;
 #pragma unroll
-        for (int u = 0; u < U; ++u) {
-          const int k = zlist[min(i + u, n_zero - 1)];
-          wu[u] = sw + k * (kDeg + 1);
-          d = max(d, sdeg[k]);
-        }
-        if (d <= 8) taylor_term_n<8, U>(wu, pw, acc, c, diag, part);
-        else if (d <= 12) taylor_term_n<12, U>(wu, pw, acc, c, diag, part);
-        else if (d <= 16) taylor_term_n<16, U>(wu, pw, acc, c, diag, part);
-        else if (d <= 20) taylor_term_n<20, U>(wu, pw, acc, c, diag, part);
-        else taylor_term_n<24, U>(wu, pw, acc, c, diag, part);
+      for (int u = 0; u < U; ++u) {
+        const int k = zlist[min(i + u, n_zero - 1)];
+        wu[u] = sw + k * (kDeg + 1);
+        d = max(d, sdeg[k]);
       }
-    } else {
-      for (int i = 0; i < n_zero; ++i) {
-        cp_async_wait<kTaylorStages - 1>();
-        const double c = real ? ring[(i % kTaylorStages) * EW_THREADS + threadIdx.x] : 0.0;
-        issue(i + kTaylorStages);  // the slot just read is this thread's own: no barrier needed
-        // the shuffles inside need every lane of the warp: the branch is warp-uniform
-        if (__any_sync(0xffffffffu, c != 0.0) != 0) {
-          const double* wk = sw + zlist[i] * (kDeg + 1);
-          const int d = sdeg[zlist[i]];  // block-uniform: the weights beyond d are zero
-          if (d <= 8) taylor_term<8, LPE>(wk, pw, acc, c, diag, h, part);
-          else if (d <= 12) taylor_term<12, LPE>(wk, pw, acc, c, diag, h, part);
-          else if (d <= 16) taylor_term<16, LPE>(wk, pw, acc, c, diag, h, part);
-          else if (d <= 20) taylor_term<20, LPE>(wk, pw, acc, c, diag, h, part);
-          else taylor_term<24, LPE>(wk, pw, acc, c, diag, h, part);
-        }
-      }
+      if (d <= 8) taylor_term_n<8, U>(wu, pw, acc, c, diag, part);
+      else if (d <= 12) taylor_term_n<12, U>(wu, pw, acc, c, diag, part);
+      else if (d <= 16) taylor_term_n<16, U>(wu, pw, acc, c, diag, part);
+      else if (d <= 20) taylor_term_n<20, U>(wu, pw, acc, c, diag, part);
+      else taylor_term_n<24, U>(wu, pw, acc, c, diag, part);
     }
     cp_async_wait<0>();
     // ---- buckets with squarings: store X0
     for (int i = 0; i < n_sq; ++i) {
       const int k = qlist[i];
       const double* wk = sw + k * (kDeg + 1);
-      double v = h == 0 ? wk[0] * diag : 0.0;
+      double v = wk[0] * diag;
 #pragma unroll
-      for (int j = 0; j < NP; ++j) v = fma(wk[j * LPE + h + 1], pw[j], v);
-#pragma unroll
-      for (int o = 1; o < LPE; o <<= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-      if (in_range && h == 0) X0[(size_t)k * n_p + e] = v;
+      for (int j = 0; j < kDeg; ++j) v = fma(wk[j + 1], pw[j], v);
+      if (in_range) X0[(size_t)k * n_p + e] = v;
     }
     if (in_range) {
 #pragma unroll
-      for (int i = 0; i < NP; ++i) Pbar[(size_t)(i * LPE + h) * n_p + e] = acc[i];
+      for (int i = 0; i < kDeg; ++i) Pbar[(size_t)i * n_p + e] = acc[i];
     }
   }
   for (int o = 16; o > 0; o >>= 1) part += __shfl_xor_sync(0xffffffffu, part, o);
@@ -1110,7 +998,7 @@ taylor_fused_smem_kernel(const double* __restrict__ powers, size_t n_p, int S, i
                     double* __restrict__ Pbar, double* __restrict__ loss_partial_fused, int* __restrict__ chunk_counter,
                     int chunk_begin, int chunk_end, double* __restrict__ tailbuf) {
   constexpr bool sym = SYM;
-  constexpr int LPE = 1, NP = kDeg;
+  constexpr int NP = kDeg;
   extern __shared__ double sw[];  // [K][m+1] weights, then int lists
   __shared__ double red[NT / 32];
   __shared__ int n_zero, n_sq;
@@ -1137,8 +1025,7 @@ taylor_fused_smem_kernel(const double* __restrict__ powers, size_t n_p, int S, i
   // PARTS == 1: the first chunk of a CTA is its block index, the others come from a counter (coef_kernel zeroes it
   // every epoch): the CTAs that finish first take what is left
   for (int chunk = chunk_begin + (PARTS == 1 ? (int)blockIdx.x : (int)(blockIdx.x / PARTS)); chunk < chunk_end;) {
-    const int h = threadIdx.x & (LPE - 1);
-    const size_t v_idx = ((size_t)chunk * blockDim.x + threadIdx.x) / LPE;
+    const size_t v_idx = (size_t)chunk * blockDim.x + threadIdx.x;
     const bool in_range = v_idx < n_visit;
     int row, col;
     taylor_visit<SYM>(in_range ? v_idx : 0, Sp, row, col);
@@ -1206,12 +1093,10 @@ taylor_fused_smem_kernel(const double* __restrict__ powers, size_t n_p, int S, i
     for (int i = unit; i < n_sq; i += PARTS) {
       const int k = qlist[i];
       const double* wk = sw + k * (kDeg + 1);
-      double v = h == 0 ? wk[0] * diag : 0.0;
+      double v = wk[0] * diag;
 #pragma unroll
       for (int j = 0; j < NP; ++j) v = fma(wk[j + 1], spw[j * NT], v);
-#pragma unroll
-      for (int o = 1; o < LPE; o <<= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-      if (in_range && h == 0) {
+      if (in_range) {
         X0[(size_t)k * n_p + e] = v;
         if (mirror) X0[(size_t)k * n_p + et] = v;
       }
@@ -1219,10 +1104,10 @@ taylor_fused_smem_kernel(const double* __restrict__ powers, size_t n_p, int S, i
     if (PARTS == 1) {
       if (in_range) {
 #pragma unroll
-        for (int i = 0; i < NP; ++i) Pbar[(size_t)(i * LPE + h) * n_p + e] = acc[i];
+        for (int i = 0; i < NP; ++i) Pbar[(size_t)i * n_p + e] = acc[i];
         if (mirror) {
 #pragma unroll
-          for (int i = 0; i < NP; ++i) Pbar[(size_t)(i * LPE + h) * n_p + et] = acc[i];
+          for (int i = 0; i < NP; ++i) Pbar[(size_t)i * n_p + et] = acc[i];
         }
       }
     } else if (in_range) {
@@ -1273,8 +1158,8 @@ __global__ void taylor_tail_reduce_kernel(const double* __restrict__ tailbuf, in
   if (SYM && row != col) Pbar[(size_t)j * n_p + (size_t)col * Sp + row] = v;
 }
 
-// Loss and G_k = -C_k / P_k (into chain slot s_k + 1) for the squared buckets of the list coef_kernel built
-// (training) or for all buckets; P_k = X0_k if s_k == 0 else chain slot s_k.  1-D grid: block = (chunk of
+// Loss and G_k = -C_k / P_k (into chain slot s_k + 1) for the squared buckets of the list coef_kernel built (the
+// fused Taylor pass did the others); P_k = X0_k if s_k == 0 else chain slot s_k.  1-D grid: block = (chunk of
 // 4 * EW_THREADS elements, list position mod kLossLanes); one loss partial per block (only the SUM over the buckets
 // is used downstream: loss_reduce_kernel puts it into loss_part[0]).  A grid of (blocks, K) launched 7 900 CTAs of
 // which 87 % returned at once: 36 us for 13 buckets of work.
@@ -1282,14 +1167,14 @@ constexpr int kLossLanes = 16;  // list positions processed side by side
 __global__ void __launch_bounds__(EW_THREADS)
 loss_grad_kernel(const double* __restrict__ C, int S, int Sp, size_t n_p, int K, const int* __restrict__ s_arr,
                  const int* __restrict__ deg_arr, const double* __restrict__ X0, double* __restrict__ chain,
-                 int slots_per_bucket, double* __restrict__ loss_partial, int skip_unsquared) {
+                 int slots_per_bucket, double* __restrict__ loss_partial) {
   __shared__ double red[EW_THREADS / 32];
-  const int n_list = skip_unsquared ? deg_arr[3 * K + 1] : K;
+  const int n_list = deg_arr[3 * K + 1];
   const int n_chunks = (int)((n_p + 4 * EW_THREADS - 1) / (4 * EW_THREADS));
   const int chunk = blockIdx.x % n_chunks, lane0 = blockIdx.x / n_chunks;
   double part = 0.0;
   for (int i = lane0; i < n_list; i += kLossLanes) {
-    const int k = skip_unsquared ? deg_arr[2 * K + i] : i;
+    const int k = deg_arr[2 * K + i];
     const int s = s_arr[k];
     const double* P = (s == 0) ? X0 + (size_t)k * n_p
                                : chain + ((size_t)k * slots_per_bucket + (s - 1)) * n_p;
@@ -1346,20 +1231,20 @@ __global__ void loss_reduce_kernel(const double* __restrict__ loss_partial, int 
   }
 }
 
-// Pbar_j = sum_k w[k][j] * X0bar_k (chain slot 1 of bucket k), j = 1..m; buckets in order.  Persistent: a CTA
-// stages the weights of the buckets it will read (only the squared ones in training: the list coef_kernel
-// built) once and walks over chunks of elements.
+// Pbar_j += sum_k w[k][j] * X0bar_k (chain slot 1 of bucket k), j = 1..m, over the squared buckets in order (the
+// list coef_kernel built; the fused Taylor pass wrote the others' share).  Persistent: a CTA stages the weights of
+// those buckets once and walks over chunks of elements.
 __global__ void __launch_bounds__(EW_THREADS)
 accumulate_M_kernel(const double* __restrict__ chain, int slots_per_bucket, size_t n_p, int K,
                     const double* __restrict__ w, double* __restrict__ Pbar,
-                    const int* __restrict__ deg_arr, int squared_only) {
+                    const int* __restrict__ deg_arr) {
   extern __shared__ double sw[];  // [n_list][m+1] weights, then the bucket list
   __shared__ int n_list_s;
-  if (threadIdx.x == 0) n_list_s = squared_only ? deg_arr[3 * K + 1] : K;
+  if (threadIdx.x == 0) n_list_s = deg_arr[3 * K + 1];
   __syncthreads();
   const int n_list = n_list_s;
   int* list = reinterpret_cast<int*>(sw + (size_t)K * (kDeg + 1));
-  for (int i = threadIdx.x; i < n_list; i += blockDim.x) list[i] = squared_only ? deg_arr[2 * K + i] : i;
+  for (int i = threadIdx.x; i < n_list; i += blockDim.x) list[i] = deg_arr[2 * K + i];
   __syncthreads();
   for (int i = threadIdx.x; i < n_list * (kDeg + 1); i += blockDim.x)
     sw[i] = w[(size_t)list[i / (kDeg + 1)] * (kDeg + 1) + i % (kDeg + 1)];
@@ -1370,7 +1255,7 @@ accumulate_M_kernel(const double* __restrict__ chain, int slots_per_bucket, size
     if (e >= n_p) continue;
     double acc[kDeg];
 #pragma unroll
-    for (int j = 0; j < kDeg; ++j) acc[j] = squared_only ? Pbar[(size_t)j * n_p + e] : 0.0;
+    for (int j = 0; j < kDeg; ++j) acc[j] = Pbar[(size_t)j * n_p + e];
     for (int i0 = 0; i0 < n_list; i0 += 4) {
       double x[4];
 #pragma unroll
@@ -1653,15 +1538,10 @@ struct Plan {
   int S, Sp, K, tiles;
   size_t n_p;
   // workspace offsets in bytes
-  size_t off_arrive, off_sched, off_scalars, off_s, off_deg, off_tau, off_w, off_loss_partial, off_grad_theta, off_dpi, off_pibuf, off_tasks, off_terms;
+  size_t off_sym_flag, off_sched, off_scalars, off_s, off_deg, off_tau, off_w, off_loss_partial, off_grad_theta, off_dpi, off_pibuf;
   size_t off_P, off_Pbar, off_X0, off_chain, off_partial, off_prof, total_bytes;
   int slots_per_bucket;   // chain slots 1..kSStore+1
   int loss_blocks;
-  int n_partial;
-  bool n_partial_overflow = false;
-  std::vector<GemmTask> tasks;   // device pointers filled relative to base
-  std::vector<GemmTerm> terms;
-  std::vector<Group> pow_fwd, sq_fwd, sq_bwd, pow_bwd;
   DfList df_fwd, df_bwd;  // the two power chains as dataflow item lists
   DfList df_fwd_sym;      // forward chain of a symmetric B: upper tiles only, mirrored (shares df_fwd's state words)
   size_t off_sr = 0;      // [S] sqrt(pi) of the current parameters (symmetric mode)
@@ -1671,17 +1551,7 @@ struct Plan {
 
 size_t align256(size_t x) { return (x + 255) / 256 * 256; }
 
-int choose_ksplit(int n_tasks, int tiles, int chunks_per_task) {
-  static const int target = getenv("CHERRY_FIT_KSPLIT_TARGET") ? atoi(getenv("CHERRY_FIT_KSPLIT_TARGET")) : 296;
-  int want = (target + n_tasks * tiles - 1) / (n_tasks * tiles);
-  int cap = chunks_per_task / 2;
-  if (cap < 1) cap = 1;
-  if (want > cap) want = cap;
-  if (want < 1) want = 1;
-  return want;
-}
-
-// Builds the layout and (if base != nullptr) the task lists with absolute device pointers.
+// Builds the layout and the item lists of the power chains (absolute device pointers if base != nullptr).
 void make_plan(Plan& p, int S, int K, char* base) {
   p.S = S;
   p.K = K;
@@ -1692,13 +1562,10 @@ void make_plan(Plan& p, int S, int K, char* base) {
   p.loss_blocks = (int)((p.n_p + 4 * EW_THREADS - 1) / (4 * EW_THREADS)) * kLossLanes;  // blocks of loss_grad_kernel
   const size_t mat = p.n_p * sizeof(double);
   const int n_theta = S + S * (S - 1) / 2;
-  // upper bounds on descriptor counts: powers (2m tasks, 4m terms) + squarings (2 * kSStore * K tasks, 3x terms)
-  const size_t max_tasks = 4 * kDeg + 2 * (size_t)kSStore * K + 16;
-  const size_t max_terms = 8 * kDeg + 3 * (size_t)kSStore * K + 16;
   size_t off = 0;
   auto carve = [&](size_t bytes) { size_t o = off; off = align256(off + bytes); return o; };
   p.off_scalars = carve(sizeof(LargeScalars));
-  p.off_arrive = carve(sizeof(int) * 64 * (size_t)p.tiles);
+  p.off_sym_flag = carve(sizeof(int));  // result word of symmetric_inputs_kernel
   p.off_sched = carve(sizeof(SqSchedule) + sizeof(int) * ((size_t)kSStore * K * 2 + (size_t)K * (kSStore + 1) +
                                                             (size_t)K + (size_t)K * p.tiles));
   p.off_s = carve(sizeof(int) * K);
@@ -1709,8 +1576,6 @@ void make_plan(Plan& p, int S, int K, char* base) {
   p.off_grad_theta = carve(sizeof(double) * n_theta);
   p.off_dpi = carve(sizeof(double) * S);
   p.off_pibuf = carve(sizeof(double) * S);
-  p.off_tasks = carve(sizeof(GemmTask) * max_tasks);
-  p.off_terms = carve(sizeof(GemmTerm) * max_terms);
   // dataflow lists: upper bounds (fine slices everywhere): items <= 3 * (m-1) * tiles * slices
   {
     const size_t max_groups = 3 * (size_t)kDeg * p.tiles + 64;
@@ -1752,7 +1617,6 @@ void make_plan(Plan& p, int S, int K, char* base) {
         if (count > 0) --count;
       }
     };
-    static const int reduce_lag = getenv("CHERRY_FIT_REDUCE_LAG") ? atoi(getenv("CHERRY_FIT_REDUCE_LAG")) : kDfReduceLag;  // A/B switch
     // one output matrix update C (+)= sum of terms, for every tile; slices of 80 (fine) or whole K per term (coarse)
     auto add_update = [&](DfList& L, double* C, int c_mat, int need_ver, int accumulate,
                           const std::vector<TermSpec>& terms, int per_term, bool upper_only = false) {
@@ -1782,16 +1646,15 @@ void make_plan(Plan& p, int S, int K, char* base) {
           L.groups.push_back(g);
           const bool direct = (g.n_slices == 1) && !g.accumulate;
           if (!direct) L.pending.push_back(gi);
-          if ((int)L.pending.size() > reduce_lag) emit_reduce(L, 1);
+          if ((int)L.pending.size() > kDfReduceLag) emit_reduce(L, 1);
         }
     };
     // K slices per term of a level with `term_tiles` (term, output tile) products: as few as keep about
-    // `target` work items in the level (every item pays ~3 us of queue / fence / reduction latency, a
+    // kDfChainTarget work items in the level (every item pays ~3 us of queue / fence / reduction latency, a
     // 80-deep slice is only 10 us of arithmetic), at most 5 (80-deep)
-    static const int chain_target = getenv("CHERRY_FIT_CHAIN_TARGET") ? atoi(getenv("CHERRY_FIT_CHAIN_TARGET")) : 500;  // sweeps 300..4000: gpurun_out/r02_fit_chain_target_sweep.txt, r02_fit_chain_sweep3.txt
     auto slices_for = [&](int term_tiles) {
       for (int n : {1, 2, 3, 4})
-        if (term_tiles * n >= chain_target) return n;
+        if (term_tiles * n >= kDfChainTarget) return n;
       return 5;
     };
     // forward: P_{b+r} = P_b P_r, r = 1..min(b, m-b); matrix id of P_j is j-1, version 1 once written (P_1: given).
@@ -1849,102 +1712,14 @@ void make_plan(Plan& p, int S, int K, char* base) {
   }
   // split-K partial buffers: the squaring dataflow kernels need kSqPartialSlots matrices, the chain
   // lists one compact 80x80 tile per (group, slice); the launches are stream ordered and share it
-  p.n_partial = kSqPartialSlots;
   {
     const size_t tile_doubles = (size_t)BT * BT;
     const size_t need = (size_t)std::max(std::max(p.df_fwd.partial_tiles, p.df_fwd_sym.partial_tiles), p.df_bwd.partial_tiles) * tile_doubles;
-    size_t doubles = p.n_p * p.n_partial;
+    size_t doubles = p.n_p * kSqPartialSlots;
     if (need > doubles) doubles = need;
     p.off_partial = carve(doubles * sizeof(double));
   }
   p.total_bytes = off;
-  if (!base) return;
-
-  auto Pj = [&](int j) { return reinterpret_cast<double*>(base + p.off_P) + (size_t)(j - 1) * p.n_p; };
-  auto Pbar = [&](int j) { return reinterpret_cast<double*>(base + p.off_Pbar) + (size_t)(j - 1) * p.n_p; };
-  auto X0 = [&](int k) { return reinterpret_cast<double*>(base + p.off_X0) + (size_t)k * p.n_p; };
-  auto chain = [&](int k, int slot) {  // slot 1..kSStore+1
-    return reinterpret_cast<double*>(base + p.off_chain) + ((size_t)k * p.slots_per_bucket + (slot - 1)) * p.n_p;
-  };
-  const int* s_arr = reinterpret_cast<const int*>(base + p.off_s);
-  const int cpt = p.Sp / BK;
-  auto begin_group = [&]() { Group g; g.task_begin = (int)p.tasks.size(); g.n_tasks = 0; g.ksplit = 1; return g; };
-  auto add_task = [&](Group& g, double* C, const int* cond, int level, int accumulate,
-                      std::initializer_list<GemmTerm> ts) {
-    GemmTask t;
-    t.C = C; t.cond = cond; t.level = level; t.accumulate = accumulate;
-    t.term_begin = (int)p.terms.size(); t.n_terms = (int)ts.size();
-    for (const GemmTerm& x : ts) p.terms.push_back(x);
-    p.tasks.push_back(t);
-    g.n_tasks++;
-  };
-  // ---- powers forward: level with base b: P_{b+r} = P_b P_r, r = 1..min(b, m-b)
-  for (int b = 1; b < kDeg; b *= 2) {
-    Group g = begin_group();
-    for (int r = 1; r <= b && b + r <= kDeg; ++r)
-      add_task(g, Pj(b + r), nullptr, 0, 0, {GemmTerm{Pj(b), Pj(r), 0, 0}});
-    g.ksplit = choose_ksplit(g.n_tasks, p.tiles, cpt);
-    p.pow_fwd.push_back(g);
-  }
-  // ---- squarings forward, level i: X_{i+1} = X_i X_i for buckets with s_k > i
-  for (int i = 0; i < kSStore; ++i) {
-    Group g = begin_group();
-    for (int k = 0; k < K; ++k) {
-      double* Xi = (i == 0) ? X0(k) : chain(k, i);
-      add_task(g, chain(k, i + 1), s_arr + k, i, 0, {GemmTerm{Xi, Xi, 0, 0}});
-    }
-    p.sq_fwd.push_back(g);
-  }
-  // ---- squarings backward, level i: Xbar_i = Xbar_{i+1} X_i^T + X_i^T Xbar_{i+1} -> slot i+1
-  for (int i = kSStore - 1; i >= 0; --i) {
-    Group g = begin_group();
-    for (int k = 0; k < K; ++k) {
-      double* Xi = (i == 0) ? X0(k) : chain(k, i);
-      double* Xb = chain(k, i + 2);
-      add_task(g, chain(k, i + 1), s_arr + k, i, 0, {GemmTerm{Xb, Xi, 0, 1}, GemmTerm{Xi, Xb, 1, 0}});
-    }
-    p.sq_bwd.push_back(g);
-  }
-  // ---- powers backward, levels in reverse.  For P_{b+r} = P_b P_r:
-  //      Pbar_r += P_b^T Pbar_{b+r}  (r != b),   Pbar_b += sum_r Pbar_{b+r} P_r^T (+ P_b^T Pbar_{2b})
-  std::vector<int> bases;
-  for (int b = 1; b < kDeg; b *= 2) bases.push_back(b);
-  for (int li = (int)bases.size() - 1; li >= 0; --li) {
-    const int b = bases[li];
-    const int rmax = (b + b <= kDeg) ? b : kDeg - b;
-    // The two kinds of products of a level only read adjoints of HIGHER powers and write
-    // different ones (Pbar_r, r < b, vs Pbar_b), so they go into ONE launch; each task splits
-    // K by its own length (the Pbar_b task concatenates up to b + 1 products).
-    Group g = begin_group();
-    int n_small = 0;
-    for (int r = 1; r <= rmax; ++r)
-      if (r != b) ++n_small;
-    const int ks_small = n_small ? choose_ksplit(n_small, p.tiles, cpt) : 1;
-    int poff = 0;
-    for (int r = 1; r <= rmax; ++r)
-      if (r != b) {
-        add_task(g, Pbar(r), nullptr, 0, 1, {GemmTerm{Pj(b), Pbar(b + r), 1, 0}});
-        p.tasks.back().ksplit = ks_small;
-        p.tasks.back().partial_off = poff;
-        poff += ks_small;
-      }
-    {
-      GemmTask t;
-      t.C = Pbar(b); t.cond = nullptr; t.level = 0; t.accumulate = 1;
-      t.term_begin = (int)p.terms.size();
-      for (int r = 1; r <= rmax; ++r) p.terms.push_back(GemmTerm{Pbar(b + r), Pj(r), 0, 1});
-      if (rmax == b) p.terms.push_back(GemmTerm{Pj(b), Pbar(2 * b), 1, 0});
-      t.n_terms = (int)p.terms.size() - t.term_begin;
-      t.ksplit = choose_ksplit(1, p.tiles, cpt * t.n_terms);
-      t.partial_off = poff;
-      poff += t.ksplit;
-      p.tasks.push_back(t);
-      g.n_tasks++;
-      g.ksplit = t.ksplit > ks_small ? t.ksplit : ks_small;
-    }
-    if (poff > p.n_partial) p.n_partial_overflow = true;
-    p.pow_bwd.push_back(g);
-  }
 }
 
 // make_plan builds ~6000 work items; the evaluation entry points run once per epoch (and per
@@ -1960,30 +1735,6 @@ const Plan& get_plan(int S, int K, char* base) {
     cS[slot] = S; cK[slot] = K; cbase[slot] = base;
   }
   return cache[slot];
-}
-
-int launch_group(const Plan& p, const Group& g, char* base, cudaStream_t stream) {
-  const GemmTask* tasks = reinterpret_cast<const GemmTask*>(base + p.off_tasks) + g.task_begin;
-  const GemmTerm* terms = reinterpret_cast<const GemmTerm*>(base + p.off_terms);
-  double* partial = reinterpret_cast<double*>(base + p.off_partial);
-  const GemmTask* host_tasks = p.tasks.data() + g.task_begin;
-  const bool own_offsets = g.n_tasks > 0 && !p.tasks.empty() && host_tasks[0].partial_off >= 0;
-  if (p.n_partial_overflow || (!own_offsets && g.ksplit > 1 && g.n_tasks * g.ksplit > p.n_partial))
-    return cherry::fail(CHERRY_ELIMIT, "fit_large: split-K partial buffer too small");
-  const size_t smem = (size_t)NSTAGE * 2 * TILE_ELEMS * sizeof(double);
-  dim3 grid(p.tiles, g.n_tasks, g.ksplit);
-  // A/B switch: the in-kernel "last CTA reduces" variant measured SLOWER (one CTA per tile re-reads
-  // ksplit partial tiles at low memory parallelism), so the separate reduce launch is the default.
-  static const bool separate_reduce = getenv("CHERRY_FIT_FUSED_REDUCE") == nullptr;
-  int* arrive = (separate_reduce || g.n_tasks > 64) ? nullptr : reinterpret_cast<int*>(base + p.off_arrive);
-  gemm_tasks_kernel<<<grid, GEMM_THREADS, smem, stream>>>(tasks, terms, p.Sp, g.ksplit, partial, arrive);
-  CHERRY_LAUNCH_CHECK("gemm_tasks_kernel");
-  if (g.ksplit > 1 && arrive == nullptr) {
-    int bx = (int)((p.n_p + EW_THREADS * 4 - 1) / (EW_THREADS * 4));
-    splitk_reduce_kernel<<<dim3(bx, g.n_tasks), EW_THREADS, 0, stream>>>(tasks, g.ksplit, p.n_p, partial);
-    CHERRY_LAUNCH_CHECK("splitk_reduce_kernel");
-  }
-  return 0;
 }
 
 int ensure_gemm_attr() {
@@ -2051,35 +1802,30 @@ static int symmetric_mode_of(const cherry_fit_args& a) {
   return it == g_sym_mode.end() ? 0 : it->second;
 }
 
-int fit_large_symmetric_form(const cherry_fit_args& a) {
-  static const bool legacy_schedule = getenv("CHERRY_FIT_LEVEL_LAUNCH") != nullptr || getenv("CHERRY_FIT_LEVEL_SYNC") != nullptr;
-  return (!legacy_schedule && symmetric_mode_of(a) == 1) ? 1 : 0;
-}
+int fit_large_symmetric_form(const cherry_fit_args& a) { return symmetric_mode_of(a) == 1 ? 1 : 0; }
 
-// Uploads the GEMM task lists (absolute pointers into this workspace).  Synchronous.
+// Uploads the item lists of the power chains (absolute pointers into this workspace) and decides the symmetric
+// form.  Synchronous.
 int fit_large_prepare(const cherry_fit_args& a, cudaStream_t stream) {
   int rc = check_large(a);
   if (rc) return rc;
   char* base = reinterpret_cast<char*>(a.workspace);
   const Plan& p = get_plan(a.S, a.K, base);
   CHERRY_CUDA(cudaStreamSynchronize(stream));
-  CHERRY_CUDA(cudaMemcpy(base + p.off_tasks, p.tasks.data(), p.tasks.size() * sizeof(GemmTask), cudaMemcpyHostToDevice));
-  CHERRY_CUDA(cudaMemcpy(base + p.off_terms, p.terms.data(), p.terms.size() * sizeof(GemmTerm), cudaMemcpyHostToDevice));
   for (const DfList* L : {&p.df_fwd, &p.df_bwd, &p.df_fwd_sym}) {
     CHERRY_CUDA(cudaMemcpy(base + L->off_items, L->items.data(), L->items.size() * sizeof(DfItem), cudaMemcpyHostToDevice));
   }
   CHERRY_CUDA(cudaMemset(base + p.off_scalars, 0, sizeof(LargeScalars)));
-  CHERRY_CUDA(cudaMemset(base + p.off_arrive, 0, sizeof(int) * 64 * (size_t)p.tiles));
   {
     const bool sym_allowed = !(getenv("CHERRY_FIT_SYMMETRIC") && atoi(getenv("CHERRY_FIT_SYMMETRIC")) == 0);  // read per fit: tests toggle it
     int mode = 0;
     if (sym_allowed && a.theta && a.mask && a.C) {
-      int* flag = reinterpret_cast<int*>(base + p.off_arrive);  // zeroed above, zeroed again below
+      int* flag = reinterpret_cast<int*>(base + p.off_sym_flag);
+      CHERRY_CUDA(cudaMemset(flag, 0, sizeof(int)));
       symmetric_inputs_kernel<<<256, 256>>>(a.mask, a.C, a.S, a.K, flag);
       CHERRY_LAUNCH_CHECK("symmetric_inputs_kernel");
       int bad = 1;
       CHERRY_CUDA(cudaMemcpy(&bad, flag, sizeof(int), cudaMemcpyDeviceToHost));
-      CHERRY_CUDA(cudaMemset(flag, 0, sizeof(int)));
       mode = bad ? 0 : 1;
     }
     std::lock_guard<std::mutex> lock(g_sym_mutex);
@@ -2127,13 +1873,8 @@ static int fit_large_impl(const cherry_fit_args& a, cudaStream_t stream, double*
   const Plan& p = get_plan(a.S, a.K, base);  // host-side tables; the device copies were uploaded by prepare
   // symmetric form (see build_B_sym_kernel): only where Q is known to be the reversible model of a.theta -- the
   // training entry points -- and fit_large_prepare found mask and counts symmetric
-  static const bool legacy_schedule = getenv("CHERRY_FIT_LEVEL_LAUNCH") != nullptr || getenv("CHERRY_FIT_LEVEL_SYNC") != nullptr;
-  const bool sym = allow_sym && P_out == nullptr && !legacy_schedule && symmetric_mode_of(a) == 1;
+  const bool sym = allow_sym && P_out == nullptr && symmetric_mode_of(a) == 1;
   const int tn = p.Sp / BT, sq_tiles = sym ? tn * (tn + 1) / 2 : p.tiles;
-  // A/B switch (graph-replayed epochs, general form, 25 tiles per product: 1 -> 1.04 ms, 2 -> 0.94, 5 -> 0.96; symmetric
-  // form, 15 tiles: 2 -> 0.764, 3 -> 0.741, 4 -> 0.744, 6 -> 0.749)
-  static const int sq_ksplit_env = getenv("CHERRY_FIT_SQ_KSPLIT") ? atoi(getenv("CHERRY_FIT_SQ_KSPLIT")) : 0;
-  const int sq_ksplit_max = sq_ksplit_env > 0 ? sq_ksplit_env : (sym ? 3 : 2);
   double* sr = reinterpret_cast<double*>(base + p.off_sr);
   LargeScalars* sc = reinterpret_cast<LargeScalars*>(base + p.off_scalars);
   int* s_arr = reinterpret_cast<int*>(base + p.off_s);
@@ -2159,19 +1900,16 @@ static int fit_large_impl(const cherry_fit_args& a, cudaStream_t stream, double*
   int* df_state_fwd = reinterpret_cast<int*>(base + p.df_fwd.off_state);
   int* df_state_bwd = reinterpret_cast<int*>(base + p.df_bwd.off_state);
   int* deg_arr = reinterpret_cast<int*>(base + p.off_deg);
-  static const int ctas_per_sm = getenv("CHERRY_FIT_CTAS_PER_SM") ? atoi(getenv("CHERRY_FIT_CTAS_PER_SM")) : 3;  // 2-stage pipeline: 51 KB and ~20 K registers per CTA
-  static const bool full_degree = getenv("CHERRY_FIT_FULL_DEGREE") != nullptr;  // A/B switch: round-1 Taylor pass
+  const int persistent_grid = kCtasPerSm * sm_count();
   coef_kernel<<<1, 256, 0, stream>>>(a.t, a.K, sc, s_arr, deg_arr, w, tau, a.status_flag, sched, sq_tiles,
-                                     (KGROUPS == 1 ? ctas_per_sm : 1) * sm_count(), df_state_fwd,
+                                     persistent_grid, df_state_fwd,
                                      (int)df_state_ints(p.df_fwd.n_mats, p.tiles, (int)p.df_fwd.groups.size()),
                                      df_state_bwd,
                                      (int)df_state_ints(p.df_bwd.n_mats, p.tiles, (int)p.df_bwd.groups.size()),
-                                     full_degree ? 1 : 0, sq_ksplit_max);
+                                     sym ? kSqKsplitSym : kSqKsplitGeneral);
   CHERRY_LAUNCH_CHECK("coef_kernel");
   mark("build_B+coef", stream);
-  static const bool level_launch = getenv("CHERRY_FIT_LEVEL_LAUNCH") != nullptr;  // A/B switch: round-1 schedule
   const size_t gemm_smem = (size_t)NSTAGE * 2 * TILE_ELEMS * sizeof(double);
-  const int persistent_grid = (KGROUPS == 1 ? ctas_per_sm : 1) * sm_count();
   auto launch_chain = [&](const DfList& L, int* state, const char* name) -> int {
     long long* prof = nullptr;
     if (g_timeline && persistent_grid <= 1024)
@@ -2183,12 +1921,7 @@ static int fit_large_impl(const cherry_fit_args& a, cudaStream_t stream, double*
     CHERRY_LAUNCH_CHECK(name);
     return 0;
   };
-  if (level_launch) {
-    for (const Group& g : p.pow_fwd)
-      if ((rc = launch_group(p, g, base, stream))) return rc;
-  } else if ((rc = launch_chain(sym ? p.df_fwd_sym : p.df_fwd, df_state_fwd, "chain_dataflow_kernel<fwd>"))) {
-    return rc;
-  }
+  if ((rc = launch_chain(sym ? p.df_fwd_sym : p.df_fwd, df_state_fwd, "chain_dataflow_kernel<fwd>"))) return rc;
   mark("powers_fwd", stream);
   static bool ew_attr[64] = {false};
   {
@@ -2197,10 +1930,7 @@ static int fit_large_impl(const cherry_fit_args& a, cudaStream_t stream, double*
     if (dev < 64 && !ew_attr[dev]) {
       CHERRY_CUDA(cudaFuncSetAttribute(poly_eval_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
       CHERRY_CUDA(cudaFuncSetAttribute(accumulate_M_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-      CHERRY_CUDA(cudaFuncSetAttribute(taylor_fused_kernel<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-      CHERRY_CUDA(cudaFuncSetAttribute(taylor_fused_kernel<1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-      CHERRY_CUDA(cudaFuncSetAttribute(taylor_fused_kernel<1, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-      CHERRY_CUDA(cudaFuncSetAttribute(taylor_fused_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+      CHERRY_CUDA(cudaFuncSetAttribute(taylor_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
 #define CHERRY_TAYLOR_ATTR(SYM_, PARTS_)                                                               \
   CHERRY_CUDA(cudaFuncSetAttribute(taylor_fused_smem_kernel<1, kTaylorThreads, SYM_, PARTS_>,          \
                                    cudaFuncAttributeMaxDynamicSharedMemorySize, 113 * 1024))
@@ -2212,40 +1942,24 @@ static int fit_large_impl(const cherry_fit_args& a, cudaStream_t stream, double*
       ew_attr[dev] = true;
     }
   }
-  static const bool unfused = getenv("CHERRY_FIT_UNFUSED") != nullptr;  // A/B switch
-  const bool fused = (P_out == nullptr) && !unfused;
   double* fused_partial = loss_partial + (size_t)p.loss_blocks;
   int fused_blocks = 0;
-  if (fused) {
-    const size_t fsmem = wsmem + 3 * sizeof(int) * a.K + 8 + sizeof(double) * kTaylorStages * EW_THREADS;
-    static const int lpe = getenv("CHERRY_FIT_TAYLOR_LPE") ? atoi(getenv("CHERRY_FIT_TAYLOR_LPE")) : 1;  // A/B switch
-    int ebl = (int)((p.n_p * (size_t)lpe + EW_THREADS - 1) / EW_THREADS);
-    static const int taylor_ctas = getenv("CHERRY_FIT_TAYLOR_CTAS") ? atoi(getenv("CHERRY_FIT_TAYLOR_CTAS")) : 1;  // per SM
-    if (ebl > taylor_ctas * sm_count()) ebl = taylor_ctas * sm_count();
-    fused_blocks = ebl;
-#define CHERRY_TAYLOR_LAUNCH(L, U)                                                                                  \
-  taylor_fused_kernel<L, U><<<ebl, EW_THREADS, fsmem, stream>>>(P, p.n_p, a.S, p.Sp, a.K, w, s_arr, deg_arr, a.C, X0, \
-                                                                Pbar, fused_partial)
-    static const int tu = getenv("CHERRY_FIT_TAYLOR_U") ? atoi(getenv("CHERRY_FIT_TAYLOR_U")) : kTaylorInterleave;  // A/B switch
-    static const int pws = getenv("CHERRY_FIT_TAYLOR_SMEM") ? atoi(getenv("CHERRY_FIT_TAYLOR_SMEM")) : 1;  // A/B switch (0: powers in registers, one CTA per SM)
+  if (P_out != nullptr) {
+    poly_eval_kernel<<<eb, EW_THREADS, wsmem, stream>>>(P, p.n_p, a.S, p.Sp, a.K, w, X0);
+    CHERRY_LAUNCH_CHECK("poly_eval_kernel");
+  } else {
     const bool two_ctas_fit = 2 * (wsmem + 3 * sizeof(int) * a.K + 8 + sizeof(double) * (kTaylorStagesS + kDeg) * kTaylorThreads + 1024) <=
-                              (size_t)227 * 1024;  // else (K > ~105): the register variant, one CTA per SM
-    if (pws && two_ctas_fit) {
+                              (size_t)227 * 1024;  // else (K >= 157): the register variant, one CTA per SM
+    if (two_ctas_fit) {
       // kTaylorThreads per CTA, two CTAs per SM (128 registers: the powers live in shared memory)
       constexpr int NT = kTaylorThreads;
       const size_t ssmem = wsmem + 3 * sizeof(int) * a.K + 8 + sizeof(double) * (kTaylorStagesS + kDeg) * NT;
       const size_t n_visit = sym ? (size_t)(p.Sp / 2) * (p.Sp + 1) : p.n_p;  // symmetric form: the upper triangle
       const int n_chunks = (int)((n_visit + NT - 1) / NT), slots = 2 * sm_count();
       // the chunks beyond a multiple of the resident CTAs, when they would fill less than half a round, run as
-      // (chunk, share of the buckets) CTAs of their own -- see the kernel.  A/B switch: CHERRY_FIT_TAYLOR_TAIL=0
-      static const bool tail_allowed = !(getenv("CHERRY_FIT_TAYLOR_TAIL") && atoi(getenv("CHERRY_FIT_TAYLOR_TAIL")) == 0);
-      // CHERRY_FIT_TAYLOR_PARTS = 2, 4, 8, 16: EVERY chunk runs as that many (chunk, share of the buckets) CTAs
-      static const int parts_all = getenv("CHERRY_FIT_TAYLOR_PARTS") ? atoi(getenv("CHERRY_FIT_TAYLOR_PARTS")) : kTaylorParts;
+      // (chunk, share of the buckets) CTAs of their own -- see the kernel
       int tail = 0, parts = 1;
-      if ((parts_all == 2 || parts_all == 4 || parts_all == 8 || parts_all == 16) && parts_all * n_chunks <= kTaylorTailUnits) {
-        tail = n_chunks;
-        parts = parts_all;
-      } else if (tail_allowed && n_chunks > slots && n_chunks % slots != 0 && n_chunks % slots <= slots / 2) {
+      if (n_chunks > slots && n_chunks % slots != 0 && n_chunks % slots <= slots / 2) {
         tail = n_chunks % slots;
         for (int cand : {16, 8, 4, 2})
           if (cand * tail <= slots && cand * tail <= kTaylorTailUnits) {
@@ -2290,27 +2004,19 @@ static int fit_large_impl(const cherry_fit_args& a, cudaStream_t stream, double*
                                                                            p.n_p, p.Sp, Pbar);
       }
 #undef CHERRY_TAYLOR_S
-    } else if (lpe == 2) CHERRY_TAYLOR_LAUNCH(2, 1);
-    else if (tu == 4) CHERRY_TAYLOR_LAUNCH(1, 4);
-    else if (tu == 2) CHERRY_TAYLOR_LAUNCH(1, 2);
-    else CHERRY_TAYLOR_LAUNCH(1, 1);
-#undef CHERRY_TAYLOR_LAUNCH
+    } else {
+      const size_t fsmem = wsmem + 3 * sizeof(int) * a.K + 8 + sizeof(double) * kTaylorStages * EW_THREADS;
+      fused_blocks = std::min(eb, sm_count());
+      taylor_fused_kernel<<<fused_blocks, EW_THREADS, fsmem, stream>>>(P, p.n_p, a.S, p.Sp, a.K, w, s_arr, deg_arr, a.C,
+                                                                        X0, Pbar, fused_partial);
+    }
     CHERRY_LAUNCH_CHECK("taylor_fused_kernel");
-  } else {
-    poly_eval_kernel<<<eb, EW_THREADS, wsmem, stream>>>(P, p.n_p, a.S, p.Sp, a.K, w, X0);
-    CHERRY_LAUNCH_CHECK("poly_eval_kernel");
   }
   mark("taylor_fused", stream);
-  static const bool level_sync = getenv("CHERRY_FIT_LEVEL_SYNC") != nullptr;  // A/B switch
-  if (level_sync) {
-    for (const Group& g : p.sq_fwd)
-      if ((rc = launch_group(p, g, base, stream))) return rc;
-  } else {
-    squaring_dataflow_kernel<false><<<persistent_grid, GEMM_THREADS, gemm_smem, stream>>>(
-        sched, s_arr, a.K, p.Sp, X0, chain, p.slots_per_bucket, reinterpret_cast<double*>(base + p.off_partial),
-        a.status_flag, sym ? 1 : 0);
-    CHERRY_LAUNCH_CHECK("squaring_dataflow_kernel<fwd>");
-  }
+  squaring_dataflow_kernel<false><<<persistent_grid, GEMM_THREADS, gemm_smem, stream>>>(
+      sched, s_arr, a.K, p.Sp, X0, chain, p.slots_per_bucket, reinterpret_cast<double*>(base + p.off_partial),
+      a.status_flag, sym ? 1 : 0);
+  CHERRY_LAUNCH_CHECK("squaring_dataflow_kernel<fwd>");
   mark("squarings_fwd", stream);
   if (P_out != nullptr) {
     extract_P_kernel<<<dim3((a.S * a.S + 255) / 256, a.K), 256, 0, stream>>>(s_arr, X0, chain, p.slots_per_bucket,
@@ -2320,32 +2026,21 @@ static int fit_large_impl(const cherry_fit_args& a, cudaStream_t stream, double*
   }
   const int loss_grid = (int)((p.n_p + 4 * EW_THREADS - 1) / (4 * EW_THREADS)) * kLossLanes;
   loss_grad_kernel<<<loss_grid, EW_THREADS, 0, stream>>>(a.C, a.S, p.Sp, p.n_p, a.K, s_arr, deg_arr, X0, chain,
-                                                         p.slots_per_bucket, loss_partial, fused ? 1 : 0);
+                                                         p.slots_per_bucket, loss_partial);
   CHERRY_LAUNCH_CHECK("loss_grad_kernel");
-  loss_reduce_kernel<<<1, 256, 0, stream>>>(loss_partial, a.K, loss_grid, a.loss_part, fused_partial,
-                                            fused ? fused_blocks : 0);
+  loss_reduce_kernel<<<1, 256, 0, stream>>>(loss_partial, a.K, loss_grid, a.loss_part, fused_partial, fused_blocks);
   CHERRY_LAUNCH_CHECK("loss_reduce_kernel");
   mark("loss_grad", stream);
-  if (level_sync) {
-    for (const Group& g : p.sq_bwd)
-      if ((rc = launch_group(p, g, base, stream))) return rc;
-  } else {
-    squaring_dataflow_kernel<true><<<persistent_grid, GEMM_THREADS, gemm_smem, stream>>>(
-        sched, s_arr, a.K, p.Sp, X0, chain, p.slots_per_bucket, reinterpret_cast<double*>(base + p.off_partial),
-        a.status_flag, sym ? 1 : 0);
-    CHERRY_LAUNCH_CHECK("squaring_dataflow_kernel<bwd>");
-  }
+  squaring_dataflow_kernel<true><<<persistent_grid, GEMM_THREADS, gemm_smem, stream>>>(
+      sched, s_arr, a.K, p.Sp, X0, chain, p.slots_per_bucket, reinterpret_cast<double*>(base + p.off_partial),
+      a.status_flag, sym ? 1 : 0);
+  CHERRY_LAUNCH_CHECK("squaring_dataflow_kernel<bwd>");
   mark("squarings_bwd", stream);
   accumulate_M_kernel<<<std::min(eb, 4 * sm_count()), EW_THREADS, wsmem + sizeof(int) * a.K, stream>>>(
-      chain, p.slots_per_bucket, p.n_p, a.K, w, Pbar, deg_arr, fused ? 1 : 0);
+      chain, p.slots_per_bucket, p.n_p, a.K, w, Pbar, deg_arr);
   CHERRY_LAUNCH_CHECK("accumulate_M_kernel");
   mark("accumulate_M", stream);
-  if (level_launch) {
-    for (const Group& g : p.pow_bwd)
-      if ((rc = launch_group(p, g, base, stream))) return rc;
-  } else if ((rc = launch_chain(p.df_bwd, df_state_bwd, "chain_dataflow_kernel<bwd>"))) {
-    return rc;
-  }
+  if ((rc = launch_chain(p.df_bwd, df_state_bwd, "chain_dataflow_kernel<bwd>"))) return rc;
   mark("powers_bwd", stream);
   if (sym)
     unpad_sym_kernel<<<(a.S * a.S + 255) / 256, 256, 0, stream>>>(Pbar, sr, a.S, p.Sp, a.dQ_part);
@@ -2421,8 +2116,7 @@ int gemm_f64_batched(const double* A, const double* B, double* C, int n, int bat
   const size_t nn = (size_t)n * n;
   for (int b = 0; b < batch; ++b) {
     terms[b] = GemmTerm{A + b * nn, B + b * nn, ta, tb};
-    tasks[b].C = C + b * nn; tasks[b].cond = nullptr; tasks[b].term_begin = b; tasks[b].n_terms = 1;
-    tasks[b].accumulate = accumulate; tasks[b].level = 0;
+    tasks[b].C = C + b * nn; tasks[b].term_begin = b; tasks[b].n_terms = 1; tasks[b].accumulate = accumulate;
   }
   char* d = reinterpret_cast<char*>(desc);
   const size_t task_bytes = align256(sizeof(GemmTask) * batch);
@@ -2433,7 +2127,7 @@ int gemm_f64_batched(const double* A, const double* B, double* C, int n, int bat
   const GemmTerm* dm = reinterpret_cast<const GemmTerm*>(d + task_bytes);
   const size_t smem = (size_t)NSTAGE * 2 * TILE_ELEMS * sizeof(double);
   dim3 grid((n / BT) * (n / BT), batch, ksplit);
-  gemm_tasks_kernel<<<grid, GEMM_THREADS, smem, stream>>>(dt, dm, n, ksplit, partial, nullptr);
+  gemm_tasks_kernel<<<grid, GEMM_THREADS, smem, stream>>>(dt, dm, n, ksplit, partial);
   CHERRY_LAUNCH_CHECK("gemm_tasks_kernel");
   if (ksplit > 1) {
     int bx = (int)((nn + EW_THREADS * 4 - 1) / (EW_THREADS * 4));

@@ -15,7 +15,6 @@
 // (estimation/_ratelearn/trainer.py:156-187), RateMatrix.forward (rate.py:167-188), and the
 // batched per-site variant (_siterm/_cherryml_vectorized.py:264-293, 351-383).
 #include "common.cuh"
-#include <cstdlib>
 
 #include "fit_common.cuh"
 
@@ -473,12 +472,7 @@ namespace cherry {
 // TWO CTAs share an SM; slots beyond the resident ones live in the global workspace (sized for the worst
 // case in both shapes, so the caller's workspace does not depend on the shape).
 constexpr int kThroughputThreads = 288, kThroughputSlots = 20;
-static bool throughput_shape(int S, int grid) {
-  static const int forced = getenv("CHERRY_FIT_SMALL_SHAPE") ? atoi(getenv("CHERRY_FIT_SMALL_SHAPE")) : -1;  // A/B switch
-  if (S > 24) return false;
-  if (forced >= 0) return forced == 1;
-  return grid > sm_count();
-}
+static bool throughput_shape(int S, int grid) { return S <= 24 && grid > sm_count(); }
 
 int fit_small_workspace(int S, int* n_smem_slots, int* spill_slots, size_t* slot_bytes,
                         size_t* smem_bytes, int grid) {
@@ -540,8 +534,6 @@ int fit_small_expm(const cherry_fit_args& a, cudaStream_t stream, double* P_out,
   const size_t need = fit_small_workspace_bytes(a.S, a.K, a.n_problems);
   if (!a.workspace || a.workspace_bytes < need)
     return fail(CHERRY_EINVAL, "fit: workspace of %zu bytes required, got %zu", need, a.workspace_bytes);
-  static const bool no_fuse = getenv("CHERRY_FIT_SMALL_UNFUSED") != nullptr;  // A/B switch: two launches per epoch
-  if (no_fuse) fuse_update = false;
   const UpdateArgs ua = make_update_args(a, 1, nullptr);
   int* arrive = fuse_update ? reinterpret_cast<int*>(reinterpret_cast<char*>(a.workspace) +
                                                      small_spill_bytes(sp, sb, a.n_problems, a.K))

@@ -154,7 +154,7 @@ def test_loss_decreases_and_graph_replay_equals_eager():
 CO_COUNTS = os.path.join(os.path.dirname(FIT), "counting/medium3/refcpp_count_co_matrices_dir_cherries_plus_plus/result.npz")
 
 
-@pytest.mark.parametrize("S,K", [(36, 6), (64, 5), (100, 7), (400, 4)])
+@pytest.mark.parametrize("S,K", [(36, 6), (64, 5), (100, 7), (400, 4), (36, 160)])
 @pytest.mark.parametrize("tmin,grad_tol", [(1e-3, 1e-10), (1e-6, 1e-7)])
 def test_large_loss_and_gradient_match_the_oracle(S, K, tmin, grad_tol):
     """With t down to 1e-6 the oracle's own gradient (autograd through torch.matrix_exp's
