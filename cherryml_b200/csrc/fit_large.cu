@@ -57,6 +57,12 @@ constexpr int kTaylorTailUnits = 512;   // (chunk, share) CTAs of the tail split
 constexpr int kTaylorInterleave = 2;  // buckets whose dependent chains a thread of the fused Taylor pass interleaves
 constexpr int kTaylorStages = 16;  // count loads in flight per thread of the fused Taylor pass
 static_assert(kDeg % 4 == 0, "the elementwise kernels skip Taylor terms in blocks of four");
+// The tightest shared-memory budget that depends on K: taylor_fused_kernel (the large-K Taylor pass) stages the
+// weight table, three int lists and the count-load ring in the 200 KB it is allowed (see fit_large_impl).  The
+// other per-K tables (poly_eval_kernel 200 K bytes, accumulate_M_kernel 204 K) fit whenever this one does.
+static_assert(CHERRY_LARGE_FIT_MAX_K ==
+                  (200 * 1024 - 8 - (int)sizeof(double) * kTaylorStages * EW_THREADS) / ((int)sizeof(double) * (kDeg + 1) + 3 * (int)sizeof(int)),
+              "CHERRY_LARGE_FIT_MAX_K must be the K budget of taylor_fused_kernel's shared memory");
 
 struct GemmTerm {
   const double* A;
@@ -699,15 +705,15 @@ __global__ void coef_kernel(const double* __restrict__ t, int K, LargeScalars* _
   int* rank = sq_rank(sched, K);
   int* tile_arrive = sq_tile_arrive(sched, K);
   for (int i = threadIdx.x; i < K * tiles; i += blockDim.x) tile_arrive[i] = 0;
-  __shared__ int ss[256], level_n[kSStore];
-  for (int k = threadIdx.x; k < K; k += blockDim.x) ss[k] = s_arr[k];
-  __syncthreads();
+  // s_arr was written by this CTA before the barrier above, so it is read back from global memory: K is not
+  // bounded by a shared-memory array here
+  __shared__ int level_n[kSStore];
   if (threadIdx.x == kSStore) {  // bucket lists of the fused Taylor pass: without / with squarings, ascending
     int* zl = deg_arr + K;
     int* ql = zl + K;
     int nz = 0, nq = 0;
     for (int k = 0; k < K; ++k) {
-      if (ss[k] == 0) zl[nz++] = k; else ql[nq++] = k;
+      if (s_arr[k] == 0) zl[nz++] = k; else ql[nq++] = k;
     }
     ql[K] = nz;
     ql[K + 1] = nq;
@@ -716,7 +722,7 @@ __global__ void coef_kernel(const double* __restrict__ t, int K, LargeScalars* _
     const int lvl = threadIdx.x;
     int n = 0;
     for (int k = 0; k < K; ++k)
-      if (ss[k] > lvl) {
+      if (s_arr[k] > lvl) {
         if (lvl == 0) rank[k] = n;
         active[lvl * K + n++] = k;
       }
@@ -1540,6 +1546,7 @@ struct Plan {
   // workspace offsets in bytes
   size_t off_sym_flag, off_sched, off_scalars, off_s, off_deg, off_tau, off_w, off_loss_partial, off_grad_theta, off_dpi, off_pibuf;
   size_t off_P, off_Pbar, off_X0, off_chain, off_partial, off_prof, total_bytes;
+  size_t max_items, max_groups;  // capacity of each DfList's item array and state words in the workspace
   int slots_per_bucket;   // chain slots 1..kSStore+1
   int loss_blocks;
   DfList df_fwd, df_bwd;  // the two power chains as dataflow item lists
@@ -1547,6 +1554,7 @@ struct Plan {
   size_t off_sr = 0;      // [S] sqrt(pi) of the current parameters (symmetric mode)
   size_t off_shat = 0;    // [S][S] mask_ij softplus(u_ij) of the current parameters
   size_t off_tailbuf = 0; // shares of the power adjoints written by the tail CTAs of the fused Taylor pass
+  bool lists_fit = true;  // every DfList's items and groups fit the workspace carved for them
 };
 
 size_t align256(size_t x) { return (x + 255) / 256 * 256; }
@@ -1580,6 +1588,8 @@ void make_plan(Plan& p, int S, int K, char* base) {
   {
     const size_t max_groups = 3 * (size_t)kDeg * p.tiles + 64;
     const size_t max_items = 3 * (size_t)kDeg * p.tiles * (p.Sp / BT) + max_groups * kDfSlabs + 64;
+    p.max_items = max_items;
+    p.max_groups = max_groups;
     p.df_fwd.off_items = carve(sizeof(DfItem) * max_items);
     p.df_fwd.off_state = carve(sizeof(int) * df_state_ints(kDeg, p.tiles, (int)max_groups));
     p.df_bwd.off_items = carve(sizeof(DfItem) * max_items);
@@ -1720,6 +1730,10 @@ void make_plan(Plan& p, int S, int K, char* base) {
     p.off_partial = carve(doubles * sizeof(double));
   }
   p.total_bytes = off;
+  // fit_large_prepare uploads the item lists into the arrays carved above, and coef_kernel clears the state words
+  // of groups.size() groups: the bounds are estimates, so they are checked
+  for (const DfList* L : {&p.df_fwd, &p.df_bwd, &p.df_fwd_sym})
+    if (L->items.size() > p.max_items || L->groups.size() > p.max_groups) p.lists_fit = false;
 }
 
 // make_plan builds ~6000 work items; the evaluation entry points run once per epoch (and per
@@ -1770,10 +1784,25 @@ void fill_update_args(LargeUpdateArgs& u, const cherry_fit_args& a, const Plan& 
   u.do_adam = a.do_adam; u.loss_normalization = a.loss_normalization; u.best_mode = a.best_mode;
 }
 
-int check_large(const cherry_fit_args& a) {
-  if (a.n_problems != 1)
+// Sizes the large path supports; the plan of (S, K) in *plan.
+int check_sizes(int S, int K, int n_problems, const Plan** plan) {
+  if (n_problems != 1)
     return cherry::fail(CHERRY_ELIMIT, "fit: batched problems are supported for S <= %d only", cherry::kSmallFitMaxS);
-  const Plan& p = get_plan(a.S, a.K, nullptr);
+  if (K > CHERRY_LARGE_FIT_MAX_K)
+    return cherry::fail(CHERRY_ELIMIT, "fit: K=%d time buckets (or exponents) exceed the limit of %d for S > %d", K,
+                        CHERRY_LARGE_FIT_MAX_K, cherry::kSmallFitMaxS);
+  const Plan& p = get_plan(S, K, nullptr);
+  if (!p.lists_fit)
+    return cherry::fail(CHERRY_ELIMIT, "fit: the power-chain work lists of S=%d exceed their workspace", S);
+  *plan = &p;
+  return 0;
+}
+
+int check_large(const cherry_fit_args& a) {
+  const Plan* pp = nullptr;
+  int rc = check_sizes(a.S, a.K, a.n_problems, &pp);
+  if (rc) return rc;
+  const Plan& p = *pp;
   if (!a.workspace || a.workspace_bytes < p.total_bytes)
     return cherry::fail(CHERRY_EINVAL, "fit: workspace of %zu bytes required, got %zu", p.total_bytes,
                         a.workspace_bytes);
@@ -1785,8 +1814,10 @@ int check_large(const cherry_fit_args& a) {
 namespace cherry {
 
 int fit_large_workspace_bytes(int S, int K, int n_problems, size_t* bytes) {
-  if (n_problems != 1) return fail(CHERRY_ELIMIT, "fit: batched problems are supported for S <= %d only", kSmallFitMaxS);
-  *bytes = get_plan(S, K, nullptr).total_bytes;
+  const Plan* p = nullptr;
+  int rc = check_sizes(S, K, n_problems, &p);
+  if (rc) return rc;
+  *bytes = p->total_bytes;
   return 0;
 }
 
@@ -1886,8 +1917,7 @@ static int fit_large_impl(const cherry_fit_args& a, cudaStream_t stream, double*
   double* X0 = reinterpret_cast<double*>(base + p.off_X0);
   double* chain = reinterpret_cast<double*>(base + p.off_chain);
   const int eb = (int)((p.n_p + EW_THREADS - 1) / EW_THREADS);
-  const size_t wsmem = sizeof(double) * a.K * (kDeg + 1);
-  if (wsmem > 200 * 1024) return fail(CHERRY_ELIMIT, "fit_large: K=%d too large for the weight table", a.K);
+  const size_t wsmem = sizeof(double) * a.K * (kDeg + 1);  // K <= CHERRY_LARGE_FIT_MAX_K (check_large)
 
   mark("start", stream);
   if (sym)

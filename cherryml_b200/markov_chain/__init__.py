@@ -51,20 +51,31 @@ class FactorizedReversibleModel:
         return self.P2 @ self.U @ np.diag(self.D) @ self.U_t @ self.P1
 
 
+# Exponents per cherry_expm_batched call for S > 32 (CHERRY_LARGE_FIT_MAX_K in include/cherryml_b200.h)
+LARGE_MAX_K = 811
+_SMALL_MAX_S = 32
+
+
 def expm_batched(Q, exponents, device="cuda") -> torch.Tensor:
-    """``[K, S, S]`` CUDA fp64 tensor of ``expm(exponents[k] * Q)``."""
+    """``[K, S, S]`` CUDA fp64 tensor of ``expm(exponents[k] * Q)``, for any number of exponents."""
     lib = _lib.load()
     dev = torch.device(device if str(device).startswith("cuda") else "cuda")
     Qt = torch.from_numpy(np.array(Q, dtype=np.float64)).to(dev).contiguous()
     t = torch.from_numpy(np.array(exponents, dtype=np.float64).reshape(-1)).to(dev).contiguous()
     S, K = int(Qt.shape[-1]), int(t.numel())
-    if K == 0:
-        return torch.zeros((0, S, S), dtype=torch.float64, device=dev)
+    out = torch.empty((K, S, S), dtype=torch.float64, device=dev)
+    chunk = LARGE_MAX_K if S > _SMALL_MAX_S else max(K, 1)
+    for k0 in range(0, K, chunk):
+        _expm_call(lib, Qt, t[k0: k0 + chunk], out[k0: k0 + chunk], dev)
+    return out
+
+
+def _expm_call(lib, Qt, t, out, dev) -> None:
+    S, K = int(Qt.shape[-1]), int(t.numel())
     nbytes = ctypes.c_size_t(0)
     _lib.check(lib.cherry_fit_workspace_bytes(S, K, 1, ctypes.byref(nbytes)), "cherry_fit_workspace_bytes")
     ws = torch.empty(max(8, nbytes.value), dtype=torch.uint8, device=dev)
     flag = torch.zeros(1, dtype=torch.int32, device=dev)
-    out = torch.empty((K, S, S), dtype=torch.float64, device=dev)
     a = FitArgs()
     a.S, a.K, a.n_problems = S, K, 1
     a.t, a.Q = _lib.ptr(t), _lib.ptr(Qt)
@@ -73,9 +84,15 @@ def expm_batched(Q, exponents, device="cuda") -> torch.Tensor:
     with torch.cuda.device(dev):
         _lib.check(lib.cherry_expm_batched(ctypes.byref(a), _lib.ptr(out), _lib.current_stream_ptr()),
                    "cherry_expm_batched")
-    if int(flag.item()) != 0:
-        raise _lib.CherryError("expm: exponent * rate is beyond the supported range (t * max|Q_ii| > 279)")
-    return out
+    status = int(flag.item())
+    if status == 3:
+        raise _lib.CherryError("expm: internal scheduling timeout of the squaring kernels (status 3)")
+    if status != 0:
+        if S > _SMALL_MAX_S:  # eight squarings of a Taylor step with t * max|Q_ii| <= 2.2
+            bound = "t * max|Q_ii| > 2.2 * 2^8 = 563.2"
+        else:  # thirty squarings of a Taylor step with t * ||Q||_1 <= 0.0376
+            bound = "t * ||Q||_1 > 0.0376 * 2^30 = 4.0e7"
+        raise _lib.CherryError(f"expm: exponent * rate is beyond the supported range ({bound})")
 
 
 def matrix_exponential_pytorch(exponents: List[float], Q: np.ndarray, device: str) -> np.ndarray:

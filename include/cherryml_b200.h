@@ -287,7 +287,14 @@ typedef struct cherry_fit_args {
   int best_mode;           /* 0: trainer.py:179 (first epoch always taken); 1: best starts at +inf */
 } cherry_fit_args;
 
-/* Bytes of `workspace` the fit needs for these sizes (0 is a valid answer). */
+/* Largest K (time buckets, or exponents of one cherry_expm_batched call) for S > 32: the weight
+ * table, bucket lists and count-load ring of the large-K Taylor pass share one CTA's 200 KB of
+ * shared memory, 212 K + 32 776 bytes.  Beyond it the entry points return CHERRY_ELIMIT; callers
+ * with more exponents split them into calls of at most this many. */
+#define CHERRY_LARGE_FIT_MAX_K 811
+
+/* Bytes of `workspace` the fit needs for these sizes (0 is a valid answer).  CHERRY_ELIMIT for
+ * S > 32 and K > CHERRY_LARGE_FIT_MAX_K. */
 int cherry_fit_workspace_bytes(int S, int K, int n_problems, size_t* bytes);
 /* Q = Q(theta) for every problem (call once before the first epoch). */
 int cherry_fit_init(const cherry_fit_args* args, void* stream);
@@ -318,7 +325,10 @@ int cherry_fit_loss_grad(const cherry_fit_args* args, void* stream);
 
 /* P_out[p*K + k] = expm(t[p*K + k] * Q[p]) (fp64 [S][S] each) with the fit's forward algorithm.
  * Only S, K, n_problems, t, Q, workspace(+bytes, as for the fit) and status_flag of `args` are
- * read.  Replaces matrix_exponential_pytorch (reference markov_chain/_markov_chain.py:22-53). */
+ * read.  Replaces matrix_exponential_pytorch (reference markov_chain/_markov_chain.py:22-53).
+ * For S > 32, K <= CHERRY_LARGE_FIT_MAX_K (else CHERRY_ELIMIT), and *status_flag is set non-zero
+ * when some t * max|Q_ii| exceeds 2.2 * 2^8 = 563.2 (eight squarings).  For S <= 32 the squarings
+ * stop at 30, i.e. t * ||Q||_1 (max column abs sum) up to 0.0376 * 2^30 = 4.0e7. */
 int cherry_expm_batched(const cherry_fit_args* args, double* P_out, void* stream);
 
 /* The FP64 tensor-core GEMM of the large-S fit, stand-alone (unit tests, micro-benchmark):

@@ -72,3 +72,22 @@ def test_product_package_never_imports_the_oracle():
             if re.search(r"^\s*(from|import)\s+oracle\b", text, flags=re.M) or "/root/reference" in text:
                 offenders.append(os.path.relpath(os.path.join(dirpath, fn), REPO))
     assert offenders == []
+
+
+def test_large_fit_sizes_without_gpu():
+    """S > 32: the K limit of the header is enforced by the sizing call, and the power-chain work lists of every
+    padded size up to 800 fit the workspace carved for them (the sizing call fails otherwise)."""
+    import ctypes
+
+    from cherryml_b200.markov_chain import LARGE_MAX_K
+
+    text = open(os.path.join(REPO, "include", "cherryml_b200.h")).read()
+    assert int(re.search(r"#define CHERRY_LARGE_FIT_MAX_K (\d+)", text).group(1)) == LARGE_MAX_K
+    lib = _lib.load()
+    n = ctypes.c_size_t(0)
+    for S in list(range(33, 801, 80)) + list(range(80, 801, 80)):
+        assert lib.cherry_fit_workspace_bytes(S, 4, 1, ctypes.byref(n)) == 0, (S, lib.cherry_last_error())
+        assert n.value > 0
+    assert lib.cherry_fit_workspace_bytes(36, LARGE_MAX_K, 1, ctypes.byref(n)) == 0
+    assert lib.cherry_fit_workspace_bytes(36, LARGE_MAX_K + 1, 1, ctypes.byref(n)) == -3
+    assert b"limit of %d" % LARGE_MAX_K in lib.cherry_last_error()
