@@ -49,21 +49,28 @@ __device__ __forceinline__ void optimizer_step(double& p, double& m, double& v, 
 // threshold covers the norm, else the maximal degree with s = ceil(log2(norm / theta_max)).
 // Thresholds keep the truncation error below 2^-53 * 1e-3 relative to ||A||_1 itself, so
 // that small off-diagonal probabilities keep ~13 significant digits before the log.
+// Returns false when the norm needs more than kMaxSquarings squarings; s is then clamped to
+// kMaxSquarings and the result is outside the accuracy the thresholds promise.  An inf / nan
+// norm gets s = 0 and returns true: the nan propagates to the output instead.
 constexpr int kMaxDegree = 9;
 constexpr int kMaxSquarings = 30;  // covers ||tQ||_1 up to 0.0376 * 2^30 ~ 4e7
-__device__ __forceinline__ void choose_degree(double norm, int& m, int& s) {
+__device__ __forceinline__ bool choose_degree(double norm, int& m, int& s) {
   // theta_m solves theta^m / (m+1)! = 1.1e-19
   const double theta[kMaxDegree + 1] = {0.0,      2.2e-19,  8.1e-10, 1.38e-6, 6.0e-5,
                                         6.0e-4,   2.8e-3,   8.4e-3,  0.0195,  0.0376};
   s = 0;
   for (m = 1; m <= kMaxDegree; ++m)
-    if (norm <= theta[m]) return;
+    if (norm <= theta[m]) return true;
   m = kMaxDegree;
-  if (!(norm < 1e300)) { s = 0; return; }  // inf / nan: let it propagate, do not loop
+  if (!(norm < 1e300)) { s = 0; return true; }  // inf / nan: let it propagate, do not loop
   double r = norm / theta[kMaxDegree];
   s = (int)ceil(log2(r));
   if (s < 0) s = 0;
-  if (s > kMaxSquarings) s = kMaxSquarings;
+  if (s > kMaxSquarings) {
+    s = kMaxSquarings;
+    return false;
+  }
+  return true;
 }
 
 __device__ __forceinline__ double inv_factorial(int j) {

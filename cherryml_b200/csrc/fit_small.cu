@@ -327,7 +327,8 @@ expm_loss_grad_small(const double* __restrict__ Qall, const double* __restrict__
   const double norm = fabs(t) * block_reduce_max<NT>(colsum, red);
   if (tid == 0) {
     int m, s;
-    cherry::choose_degree(norm, m, s);
+    // beyond 30 squarings: report it (status 2, as the large path does) and go on with s = 30
+    if (!cherry::choose_degree(norm, m, s)) atomicExch(overflow_flag, 2);
     sh_m = m;
     sh_s = s;
   }

@@ -280,7 +280,9 @@ typedef struct cherry_fit_args {
   double* workspace;   /* see cherry_fit_workspace_bytes */
   size_t workspace_bytes;
   int* epoch_counter;  /* [n_problems] epochs completed (zero at start) */
-  int* status_flag;    /* [1] set non-zero by a kernel that ran out of workspace */
+  int* status_flag;    /* [1] zero at start; a kernel sets 1 (out of matrix slots), 2 (t * norm of Q
+                          beyond the supported range, see cherry_expm_batched) or 3 (internal
+                          scheduling timeout of the large path); the results are then invalid */
   double lr_pi, lr_upper, beta1, beta2, eps;
   int do_adam;             /* 1: Adam (torch semantics), 0: plain SGD */
   int loss_normalization;  /* divide loss and gradient by sumC */
@@ -326,9 +328,12 @@ int cherry_fit_loss_grad(const cherry_fit_args* args, void* stream);
 /* P_out[p*K + k] = expm(t[p*K + k] * Q[p]) (fp64 [S][S] each) with the fit's forward algorithm.
  * Only S, K, n_problems, t, Q, workspace(+bytes, as for the fit) and status_flag of `args` are
  * read.  Replaces matrix_exponential_pytorch (reference markov_chain/_markov_chain.py:22-53).
- * For S > 32, K <= CHERRY_LARGE_FIT_MAX_K (else CHERRY_ELIMIT), and *status_flag is set non-zero
+ * For S > 32, K <= CHERRY_LARGE_FIT_MAX_K (else CHERRY_ELIMIT), and *status_flag is set to 2
  * when some t * max|Q_ii| exceeds 2.2 * 2^8 = 563.2 (eight squarings).  For S <= 32 the squarings
- * stop at 30, i.e. t * ||Q||_1 (max column abs sum) up to 0.0376 * 2^30 = 4.0e7. */
+ * stop at 30, i.e. t * ||Q||_1 (max column abs sum) up to 0.0376 * 2^30 = 4.0e7; beyond it
+ * *status_flag is set to 2 as well, and that exponent's result is computed with 30 squarings
+ * (outside the accuracy of the path).  The same flag is set by the fit and cherry_fit_loss_grad.
+ * A nan or inf t * norm sets no flag; the nan propagates to the result. */
 int cherry_expm_batched(const cherry_fit_args* args, double* P_out, void* stream);
 
 /* The FP64 tensor-core GEMM of the large-S fit, stand-alone (unit tests, micro-benchmark):

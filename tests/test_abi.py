@@ -91,3 +91,22 @@ def test_large_fit_sizes_without_gpu():
     assert lib.cherry_fit_workspace_bytes(36, LARGE_MAX_K, 1, ctypes.byref(n)) == 0
     assert lib.cherry_fit_workspace_bytes(36, LARGE_MAX_K + 1, 1, ctypes.byref(n)) == -3
     assert b"limit of %d" % LARGE_MAX_K in lib.cherry_last_error()
+
+
+def test_small_fit_sizes_without_gpu():
+    """S <= 32: the sizing call answers for every S, for one and for 400 buckets, one and 331 problems, and the
+    answer covers the matrix slots that do not stay in shared memory for every CTA, plus the arrival counters."""
+    import ctypes
+
+    lib = _lib.load()
+    n = ctypes.c_size_t(0)
+    for S in range(1, 33):
+        spad = (S + 7) // 8 * 8
+        slot_bytes = spad * (spad + 4) * 8
+        resident = min(220 * 1024 // slot_bytes, 43, 20 if S <= 24 else 43)  # 9 Taylor + 30 squaring + 4 slots
+        for K in (1, 400):
+            for P in (1, 331):
+                assert lib.cherry_fit_workspace_bytes(S, K, P, ctypes.byref(n)) == 0, (S, K, P, lib.cherry_last_error())
+                spill = (43 - resident) * slot_bytes * P * K
+                assert n.value >= spill + 4 * P, (S, K, P, n.value)
+                assert n.value <= spill + 4 * P + 512, (S, K, P, n.value)
