@@ -289,7 +289,7 @@ def bench_fit(device, lg_times=None, lg_counts: Optional[torch.Tensor] = None, n
         rank = dist.get_rank(process_group)
     # co-evolution counts from synthetic contact-map families (BASELINE config 4 shape)
     from cherryml_b200 import _lib
-    from cherryml_b200.counting._device import build_bucket_table
+    from cherryml_b200.counting._device import build_bucket_table_tiles
 
     lib = _lib.load()
     dev = as_device_batch(synthetic_co(co_families, 1024, 300, seed=11 + rank, device=device), device)
@@ -309,7 +309,7 @@ def bench_fit(device, lg_times=None, lg_counts: Optional[torch.Tensor] = None, n
         raw.zero_()
         torch.cuda.synchronize(device)
         ev[0].record()
-        tab = build_bucket_table(dev, gd, K)
+        tab = build_bucket_table_tiles(dev, gd, K)
         _lib.check(lib.cherry_sort_pairs_by_bucket(
             _lib.ptr(tab), dev.r_pad, dev.n_pairs, K, _lib.ptr(dev.fams), _lib.ptr(dev.pair_a),
             _lib.ptr(dev.pair_b), _lib.ptr(dev.pair_fam), _lib.ptr(order), _lib.ptr(recs), _lib.ptr(ws), st),

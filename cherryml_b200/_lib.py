@@ -67,10 +67,8 @@ _SIGNATURES = {
     "cherry_version": (c_char_p, []),
     "cherry_launch_count": (c_int64, []),
     "cherry_reset_launch_count": (None, []),
-    "cherry_build_bucket_table": (c_int, [_P, _P, _P, _P, _P, c_int, c_int64, c_int, _P, _P]),
     "cherry_count_lg": (c_int, [_P, _P, _P, _P, _P, c_int, _P, _P, c_int, c_int, c_int, _P, _P]),
     "cherry_build_bucket_table_tiles": (c_int, [_P, _P, c_int, _P, _P, _P, c_int, c_int, _P, _P]),
-    "cherry_count_lg_fused": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, c_int64, c_int, _P, _P, c_int, c_int, c_int, _P, _P, _P]),
     "cherry_sort_pairs_by_bucket": (c_int, [_P, c_int, c_int64, c_int, _P, _P, _P, _P, _P, _P, _P, _P]),
     "cherry_count_co": (c_int, [_P, _P, _P, c_int64, c_int, c_int, c_int, _P, _P]),
     "cherry_validate_residues": (c_int, [_P, c_int64, c_int, _P, _P]),
@@ -114,7 +112,7 @@ _SIGNATURES = {
                               _P, ctypes.c_size_t, _P]),
     "cherry_count_lg_host": (
         c_int,
-        [_P, c_int64, _P, c_int, _P, _P, _P, _P, c_int64, _P, c_int64, _P, c_int64, _P, c_int,
+        [_P, c_int64, _P, c_int, _P, _P, _P, c_int64, _P, c_int64, _P, c_int64, _P, c_int,
          _P, c_int, c_int, c_int, c_int, _P, _P, _P],
     ),
 }

@@ -106,21 +106,8 @@ def validate_residues(msa: torch.Tensor, num_states: int) -> None:
         )
 
 
-def build_bucket_table(dev: DeviceBatch, grid_dev: torch.Tensor, K: int) -> torch.Tensor:
-    lib = _lib.load()
-    tab = torch.empty(max(1, dev.n_pairs * dev.r_pad), dtype=torch.uint8, device=dev.msa.device)
-    if dev.n_pairs:
-        rc = lib.cherry_build_bucket_table(
-            _lib.ptr(dev.pair_t), _lib.ptr(dev.pair_fam), _lib.ptr(dev.fams),
-            _lib.ptr(dev.rate_vals), _lib.ptr(grid_dev), K, dev.n_pairs, dev.r_pad,
-            _lib.ptr(tab), _lib.current_stream_ptr(),
-        )
-        _lib.check(rc, "cherry_build_bucket_table")
-    return tab
-
-
 def build_bucket_table_tiles(dev: DeviceBatch, grid_dev: torch.Tensor, K: int) -> torch.Tensor:
-    """The bucket table of the pairs covered by the batch's tiles, built one CTA per tile."""
+    """The bucket table of the pairs covered by the batch's tiles, built one warp per tile."""
     lib = _lib.load()
     tab = torch.empty(max(1, dev.n_pairs * dev.r_pad), dtype=torch.uint8, device=dev.msa.device)
     if dev.n_tiles:
@@ -160,7 +147,7 @@ def count_raw(
         elo, ehi = max(0, lo - 1), min(K, hi + 1)
         sub = grid_dev[elo:ehi].contiguous()
         ks = ehi - elo
-        sub_tab = build_bucket_table(dev, sub, ks)
+        sub_tab = build_bucket_table_tiles(dev, sub, ks)
         if dev.n_pairs:
             if elo < lo:
                 sub_tab[sub_tab == 0] = _lib.NO_BUCKET
@@ -187,22 +174,8 @@ def _count_raw_one(
     lib = _lib.load()
     device = dev.msa.device
     stream = _lib.current_stream_ptr()
-    if dev.kind == "lg" and tab is None:
-        # one call: bucket table built per tile (one coalesced load per pair), then counted
-        if out is None:
-            out = torch.zeros((K, S, S), dtype=torch.int64, device=device)
-        if dev.n_tiles:
-            scratch = torch.empty(max(1, dev.n_pairs * dev.r_pad), dtype=torch.uint8, device=device)
-            rc = lib.cherry_count_lg_fused(
-                _lib.ptr(dev.msa), _lib.ptr(dev.fams), _lib.ptr(dev.pair_a), _lib.ptr(dev.pair_b),
-                _lib.ptr(dev.pair_t), _lib.ptr(dev.pair_fam), _lib.ptr(dev.rate_vals), _lib.ptr(grid_dev),
-                dev.n_pairs, dev.r_pad, _lib.ptr(dev.aux), _lib.ptr(dev.tiles), dev.n_tiles, K, S,
-                _lib.ptr(scratch), _lib.ptr(out), stream,
-            )
-            _lib.check(rc, "cherry_count_lg_fused")
-        return out
     if tab is None:
-        tab = build_bucket_table(dev, grid_dev, K)
+        tab = build_bucket_table_tiles(dev, grid_dev, K)
     if dev.kind == "lg":
         if out is None:
             out = torch.zeros((K, S, S), dtype=torch.int64, device=device)
@@ -352,8 +325,8 @@ def count_lg_host(batch: CountBatch, quantization_points: Sequence[float], num_s
     h2d, d2h = ctypes.c_int64(0), ctypes.c_int64(0)
     rc = lib.cherry_count_lg_host(
         _lib.ptr(batch.msa), int(batch.msa.size), _lib.ptr(batch.fams), int(batch.fams.shape[0]),
-        _lib.ptr(batch.pair_a), _lib.ptr(batch.pair_b), _lib.ptr(batch.pair_t), _lib.ptr(batch.pair_fam),
-        int(batch.pair_a.shape[0]), _lib.ptr(batch.rate_vals), int(batch.rate_vals.shape[0]),
+        _lib.ptr(batch.pair_a), _lib.ptr(batch.pair_b), _lib.ptr(batch.pair_t), int(batch.pair_a.shape[0]),
+        _lib.ptr(batch.rate_vals), int(batch.rate_vals.shape[0]),
         _lib.ptr(batch.aux), int(batch.aux.shape[0]), _lib.ptr(batch.tiles), int(batch.tiles.shape[0]),
         _lib.ptr(grid), K, S, int(batch.r_pad), int(directed), _lib.ptr(out),
         ctypes.addressof(h2d), ctypes.addressof(d2h),

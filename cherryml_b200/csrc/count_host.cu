@@ -63,11 +63,11 @@ int ensure_state(size_t need_bytes, int n_events) {
 
 extern "C" int cherry_count_lg_host(
     const uint8_t* msa, int64_t msa_bytes, const cherry_fam_desc* fams, int n_fams,
-    const int32_t* pair_a, const int32_t* pair_b, const double* pair_t, const int32_t* pair_fam,
-    int64_t n_pairs, const double* rate_vals, int64_t n_rate_vals, const uint16_t* group_cat,
-    int64_t n_groups, const cherry_tile* tiles, int n_tiles, const double* grid, int K, int S,
-    int r_pad, int directed, double* counts_out, int64_t* h2d_bytes, int64_t* d2h_bytes) {
-  if (!msa || !fams || !pair_a || !pair_b || !pair_t || !pair_fam || !rate_vals || !group_cat ||
+    const int32_t* pair_a, const int32_t* pair_b, const double* pair_t, int64_t n_pairs,
+    const double* rate_vals, int64_t n_rate_vals, const uint16_t* group_cat, int64_t n_groups,
+    const cherry_tile* tiles, int n_tiles, const double* grid, int K, int S, int r_pad, int directed,
+    double* counts_out, int64_t* h2d_bytes, int64_t* d2h_bytes) {
+  if (!msa || !fams || !pair_a || !pair_b || !pair_t || !rate_vals || !group_cat ||
       !tiles || !grid || !counts_out)
     return cherry::fail(CHERRY_EINVAL, "count_lg_host: null pointer argument");
   if (K <= 0 || K > CHERRY_MAX_BUCKETS)
@@ -88,7 +88,7 @@ extern "C" int cherry_count_lg_host(
   const size_t o_msa = carve((size_t)msa_bytes);
   const size_t o_fams = carve((size_t)n_fams * sizeof(cherry_fam_desc));
   const size_t o_pa = carve((size_t)n_pairs * 4), o_pb = carve((size_t)n_pairs * 4);
-  const size_t o_pt = carve((size_t)n_pairs * 8), o_pf = carve((size_t)n_pairs * 4);
+  const size_t o_pt = carve((size_t)n_pairs * 8);
   const size_t o_rv = carve((size_t)n_rate_vals * 8);
   const size_t o_gc = carve((size_t)n_groups * 2);
   const size_t o_tl = carve((size_t)n_tiles * sizeof(cherry_tile));
@@ -122,7 +122,6 @@ extern "C" int cherry_count_lg_host(
   CHERRY_CUDA(H2D(o_pa, pair_a, (size_t)n_pairs * 4));
   CHERRY_CUDA(H2D(o_pb, pair_b, (size_t)n_pairs * 4));
   CHERRY_CUDA(H2D(o_pt, pair_t, (size_t)n_pairs * 8));
-  CHERRY_CUDA(H2D(o_pf, pair_fam, (size_t)n_pairs * 4));
   CHERRY_CUDA(H2D(o_rv, rate_vals, (size_t)n_rate_vals * 8));
   CHERRY_CUDA(H2D(o_gc, group_cat, (size_t)n_groups * 2));
   CHERRY_CUDA(H2D(o_tl, tiles, (size_t)n_tiles * sizeof(cherry_tile)));
@@ -130,10 +129,10 @@ extern "C" int cherry_count_lg_host(
   CHERRY_CUDA(cudaEventRecord(s.events[n_seg], s.copy_stream));
   CHERRY_CUDA(cudaStreamWaitEvent(s.compute_stream, s.events[n_seg], 0));
   CHERRY_CUDA(cudaMemsetAsync(w + o_raw, 0, nb * 8, s.compute_stream));
-  rc = cherry_build_bucket_table((const double*)(w + o_pt), (const int32_t*)(w + o_pf),
-                                 (const cherry_fam_desc*)(w + o_fams), (const double*)(w + o_rv),
-                                 (const double*)(w + o_grid), K, n_pairs, r_pad,
-                                 (uint8_t*)(w + o_tab), s.compute_stream);
+  rc = cherry_build_bucket_table_tiles((const double*)(w + o_pt), (const cherry_tile*)(w + o_tl), n_tiles,
+                                       (const cherry_fam_desc*)(w + o_fams), (const double*)(w + o_rv),
+                                       (const double*)(w + o_grid), K, r_pad, (uint8_t*)(w + o_tab),
+                                       s.compute_stream);
   if (rc) return rc;
 
   int tile_pos = 0;
@@ -163,7 +162,7 @@ extern "C" int cherry_count_lg_host(
                               s.compute_stream));
   CHERRY_CUDA(cudaStreamSynchronize(s.compute_stream));
   if (h2d_bytes)
-    *h2d_bytes = msa_bytes + (int64_t)n_fams * (int64_t)sizeof(cherry_fam_desc) + n_pairs * 20 +
+    *h2d_bytes = msa_bytes + (int64_t)n_fams * (int64_t)sizeof(cherry_fam_desc) + n_pairs * 16 +
                  n_rate_vals * 8 + n_groups * 2 + (int64_t)n_tiles * (int64_t)sizeof(cherry_tile) +
                  (int64_t)K * 8;
   if (d2h_bytes) *d2h_bytes = (int64_t)nb * 8;

@@ -14,14 +14,15 @@
 // 16; LG columns are sorted by site-rate category and each category is padded to a
 // multiple of 4 sites, so that every aligned 32-bit word of a row has ONE category and the
 // bucket of (pair, word) is a single byte lookup tab[pair][category].
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace {
 
 constexpr int kCountThreads = 1024;  // one CTA per SM, 32 warps to cover HBM latency
 constexpr int kMaxSmemBytes = 227 * 1024;
+// Padding cells per bucket of the LG shared-memory histogram (address-stream simulation: 2.92 -> 2.80
+// wavefronts per reduction; sweep in profiles/ab/r02_count_lg_ab_v3.txt).
+constexpr int kLgBucketPad = 5;
 
 __device__ __forceinline__ uint4 ld_stream16(const uint8_t* p) {
   uint4 r;
@@ -53,71 +54,14 @@ __device__ __forceinline__ int quantize_bucket(double t, const double* __restric
   return (el < er) ? lo - 1 : lo;
 }
 
-// The same function with the binary search replaced by a guess: the grids in use are geometric
-// (center * step^i, rounded to 8 decimals), so floor((log2 t - log2 q0) * (K-1)/log2(q[K-1]/q0))
-// is within one of the lower bound; the two loops then walk to the exact lower bound (first index
-// with q[lo] >= t) for ANY ascending grid, so the result is the binary search's by construction.
-__device__ __forceinline__ int quantize_bucket_guess(double t, const double* __restrict__ q, int K, float log2_q0,
-                                                     float inv_log2_step) {
-  if (t < q[0] || t > q[K - 1]) return -1;
-  int lo = t == t ? (int)((__log2f((float)t) - log2_q0) * inv_log2_step) : 0;
-  lo = max(0, min(K - 1, lo));
-  while (lo > 0 && q[lo - 1] >= t) --lo;
-  while (lo < K && q[lo] < t) ++lo;
-  if (lo == 0) return 0;
-  const double left = q[lo - 1], right = q[lo];
-  const double tt = __dmul_rn(t, t), lr = __dmul_rn(left, right);
-  if (fabs(tt - lr) > 1e-12 * lr) return (tt < lr) ? lo - 1 : lo;
-  const double el = __dsub_rn(__ddiv_rn(t, left), 1.0);
-  const double er = __dsub_rn(__ddiv_rn(right, t), 1.0);
-  return (el < er) ? lo - 1 : lo;
-}
-
-// One thread per pair: all r_pad entries of its row (r_pad is a multiple of 4, the row is
-// written as 32-bit words).
-__global__ void bucket_table_kernel(const double* __restrict__ pair_t,
-                                    const int32_t* __restrict__ pair_fam,
-                                    const cherry_fam_desc* __restrict__ fams,
-                                    const double* __restrict__ rate_vals,
-                                    const double* __restrict__ grid, int K, int64_t n_pairs,
-                                    int r_pad, uint8_t* __restrict__ tab) {
-  extern __shared__ double sgrid[];
-  for (int i = threadIdx.x; i < K; i += blockDim.x) sgrid[i] = grid[i];
-  __syncthreads();
-  const float log2_q0 = sgrid[0] > 0.0 ? log2f((float)sgrid[0]) : 0.0f;
-  const float span = K > 1 && sgrid[0] > 0.0 ? log2f((float)(sgrid[K - 1] / sgrid[0])) : 0.0f;
-  const float inv_log2_step = span > 0.0f ? (float)(K - 1) / span : 0.0f;
-  for (int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; p < n_pairs;
-       p += (int64_t)gridDim.x * blockDim.x) {
-    const cherry_fam_desc* fd = fams + pair_fam[p];
-    const int n_rates = fd->n_rates;
-    const double* __restrict__ rv = rate_vals + fd->rate_off;
-    const double t0 = pair_t[p];
-    uint32_t* __restrict__ row = reinterpret_cast<uint32_t*>(tab + p * r_pad);
-    for (int r0 = 0; r0 < r_pad; r0 += 4) {
-      uint32_t word = 0;
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        uint32_t out = CHERRY_NO_BUCKET;
-        if (r0 + k < n_rates) {
-          const int b = quantize_bucket_guess(__dmul_rn(t0, rv[r0 + k]), sgrid, K, log2_q0, inv_log2_step);
-          if (b >= 0) out = (uint32_t)b;
-        }
-        word |= out << (8 * k);
-      }
-      row[r0 >> 2] = word;
-    }
-  }
-}
-
 // Decision boundaries of the quantisation: for every pair of neighbouring grid points (left, right) the
 // reference's predicate  t/left - 1 < right/t - 1  (IEEE division and subtraction, utils.py:35-56 ==
 // _count_transitions.cpp:295-307) is monotone in t -- the rounded quotients are monotone -- so there is ONE
 // smallest double bnd in (left, right] for which it is false, and  bucket(t) = #{i : bnd[i] <= t}.  The
 // boundary is found by bisection on the bit patterns of the doubles with the predicate itself, so the
 // result is the reference's by construction; quantising a value is then a float guess and two or three
-// double compares instead of ~110 instructions.  Grids with repeated or non-positive points keep the
-// general path (flag).
+// double compares instead of ~110 instructions.  Grids with repeated or non-positive points take the
+// binary search of quantize_bucket instead (flag).
 __device__ __forceinline__ bool quantization_predicate(double t, double left, double right) {
   return __dsub_rn(__ddiv_rn(t, left), 1.0) < __dsub_rn(__ddiv_rn(right, t), 1.0);
 }
@@ -150,9 +94,9 @@ __device__ __forceinline__ int quantize_by_boundaries(double t, float log2_t, co
   return b;
 }
 
-// The same table, one WARP per tile: a tile's pairs belong to ONE family, so the family's rate values are
+// The bucket table, one WARP per tile: a tile's pairs belong to ONE family, so the family's rate values are
 // read once per warp and a thread's only dependent load is its pair's branch length (coalesced); values are
-// quantised against the precomputed decision boundaries.
+// quantised against the precomputed decision boundaries.  Only the rows of pairs in `tiles` are written.
 __global__ void __launch_bounds__(256)
 bucket_table_tiles_kernel(const double* __restrict__ pair_t, const cherry_tile* __restrict__ tiles,
                           const cherry_fam_desc* __restrict__ fams, const double* __restrict__ rate_vals,
@@ -218,7 +162,7 @@ bucket_table_tiles_kernel(const double* __restrict__ pair_t, const cherry_tile* 
             uint32_t out = CHERRY_NO_BUCKET;
             if (r0 + k < n_rates) {
               const double x = __dmul_rn(t[u], wrate[r0 + k]);
-              const int b = use_general ? quantize_bucket_guess(x, sgrid, K, log2_q0, inv_log2_step)
+              const int b = use_general ? quantize_bucket(x, sgrid, K)
                                         : quantize_by_boundaries(x, lt + wlog[r0 + k], sgrid, sbnd, K, log2_q0, inv_log2_step);
               if (b >= 0) out = (uint32_t)b;
             }
@@ -490,26 +434,6 @@ int check_count_args(const void* msa, const void* fams, const void* pa, const vo
 
 extern "C" {
 
-int cherry_build_bucket_table(const double* pair_t, const int32_t* pair_fam,
-                              const cherry_fam_desc* fams, const double* rate_vals,
-                              const double* grid, int K, int64_t n_pairs, int r_pad,
-                              uint8_t* tab, void* stream) {
-  if (!pair_t || !pair_fam || !fams || !rate_vals || !grid || !tab)
-    return cherry::fail(CHERRY_EINVAL, "bucket_table: null pointer argument");
-  if (K <= 0 || K > CHERRY_MAX_BUCKETS)
-    return cherry::fail(CHERRY_ELIMIT, "bucket_table: K=%d outside 1..%d", K, CHERRY_MAX_BUCKETS);
-  if (n_pairs < 0 || r_pad <= 0) return cherry::fail(CHERRY_EINVAL, "bucket_table: bad sizes");
-  if (n_pairs == 0) return 0;
-  if (r_pad % 4 != 0) return cherry::fail(CHERRY_EINVAL, "bucket_table: r_pad must be a multiple of 4");
-  int blocks = (int)((n_pairs + 255) / 256);
-  int cap = cherry::sm_count() * 8;
-  if (blocks > cap) blocks = cap;
-  bucket_table_kernel<<<blocks, 256, K * sizeof(double), (cudaStream_t)stream>>>(
-      pair_t, pair_fam, fams, rate_vals, grid, K, n_pairs, r_pad, tab);
-  CHERRY_LAUNCH_CHECK("bucket_table_kernel");
-  return 0;
-}
-
 int cherry_count_lg(const uint8_t* msa, const cherry_fam_desc* fams, const int32_t* pair_a,
                     const int32_t* pair_b, const uint8_t* tab, int r_pad,
                     const uint16_t* group_cat, const cherry_tile* tiles, int n_tiles, int K,
@@ -519,8 +443,7 @@ int cherry_count_lg(const uint8_t* msa, const cherry_fam_desc* fams, const int32
   if (!group_cat) return cherry::fail(CHERRY_EINVAL, "count_lg: null group_cat");
   if (n_tiles == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
-  static const int pad_env = getenv("CHERRY_LG_BUCKET_PAD") ? atoi(getenv("CHERRY_LG_BUCKET_PAD")) : 5;  // A/B switch
-  int bstride = S * S + pad_env;
+  int bstride = S * S + kLgBucketPad;
   if (((size_t)K * bstride + 4) * sizeof(uint32_t) > (size_t)kMaxSmemBytes) bstride = S * S;
   const size_t hist_bytes = ((size_t)K * bstride + 4) * sizeof(uint32_t);  // + the junk word
   int grid = cherry::sm_count();
@@ -573,26 +496,6 @@ int cherry_build_bucket_table_tiles(const double* pair_t, const cherry_tile* til
       pair_t, tiles, fams, rate_vals, grid, K, n_tiles, r_pad, tab);
   CHERRY_LAUNCH_CHECK("bucket_table_tiles_kernel");
   return 0;
-}
-
-int cherry_count_lg_fused(const uint8_t* msa, const cherry_fam_desc* fams, const int32_t* pair_a,
-                          const int32_t* pair_b, const double* pair_t, const int32_t* pair_fam,
-                          const double* rate_vals, const double* grid, int64_t n_pairs, int r_pad,
-                          const uint16_t* group_cat, const cherry_tile* tiles, int n_tiles, int K, int S,
-                          uint8_t* tab_scratch, unsigned long long* counts, void* stream) {
-  if (!pair_t || !pair_fam || !rate_vals || !grid)
-    return cherry::fail(CHERRY_EINVAL, "count_lg_fused: null pointer argument");
-  if (r_pad <= 0 || r_pad % 4 != 0) return cherry::fail(CHERRY_EINVAL, "count_lg_fused: r_pad must be a positive multiple of 4");
-  int rc = check_count_args(msa, fams, pair_a, pair_b, msa /* tab not needed */, tiles, counts, n_tiles, K, S, r_pad);
-  if (rc) return rc;
-  if (!group_cat) return cherry::fail(CHERRY_EINVAL, "count_lg_fused: null group_cat");
-  if (n_tiles == 0) return 0;
-  if (!tab_scratch) return cherry::fail(CHERRY_EINVAL, "count_lg_fused: tab_scratch (n_pairs * r_pad bytes) is required");
-  (void)n_pairs;
-  (void)pair_fam;
-  rc = cherry_build_bucket_table_tiles(pair_t, tiles, n_tiles, fams, rate_vals, grid, K, r_pad, tab_scratch, stream);
-  if (rc) return rc;
-  return cherry_count_lg(msa, fams, pair_a, pair_b, tab_scratch, r_pad, group_cat, tiles, n_tiles, K, S, counts, stream);
 }
 
 int cherry_count_per_site(const uint8_t* xa, const uint8_t* xb, const double* t, int64_t n_cherries,

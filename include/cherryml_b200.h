@@ -10,7 +10,8 @@
  * What each entry point replaces in the reference (paths relative to the reference
  * checkout, songlab-cal/CherryML v0.2.0):
  *
- *   cherry_build_bucket_table  quantization_idx(), cherryml/utils.py:35-56 ==
+ *   cherry_build_bucket_table_tiles
+ *                              quantization_idx(), cherryml/utils.py:35-56 ==
  *                              counting/_count_transitions.cpp:295-307, evaluated once
  *                              per (pair, rate category) instead of once per site.
  *   cherry_count_lg            the per-site loop of _dfs()/_map_func(),
@@ -95,14 +96,6 @@ void cherry_reset_launch_count(void);
 
 /* ---------------------------------------------------------------- counting */
 
-/* tab[p * r_pad + r] = bucket of (pair_t[p] * rate_vals[fams[pair_fam[p]].rate_off + r])
- * for r < n_rates of that family, CHERRY_NO_BUCKET otherwise.  grid: K ascending fp64
- * quantization points.  fp64 throughout, bit-identical to the host definition. */
-int cherry_build_bucket_table(const double* pair_t, const int32_t* pair_fam,
-                              const cherry_fam_desc* fams, const double* rate_vals,
-                              const double* grid, int K, int64_t n_pairs, int r_pad,
-                              uint8_t* tab, void* stream);
-
 /* counts[b][x][y] += #sites of all pairs with bucket b, residue x on row pair_a, residue y
  * on row pair_b (raw, directed).  group_cat[fam.aux_off + g] is the rate category of
  * sites 4g..4g+3 of the family's (category-sorted, 4-aligned) columns.
@@ -112,28 +105,18 @@ int cherry_count_lg(const uint8_t* msa, const cherry_fam_desc* fams, const int32
                     const uint16_t* group_cat, const cherry_tile* tiles, int n_tiles, int K,
                     int S, unsigned long long* counts, void* stream);
 
-/* The same table as cherry_build_bucket_table for the pairs covered by `tiles`, built one warp per TILE
- * (a tile's pairs share a family: its rate values are read once per warp, a pair costs one coalesced load)
- * and quantised against precomputed decision boundaries: for neighbouring grid points (left, right) the
- * reference's predicate t/left - 1 < right/t - 1 is monotone in t, so its switch point is found once per
- * launch by bisection on the doubles with the predicate itself.  Bit-identical to the per-pair kernel. */
+/* The bucket table: for every pair p of every tile in `tiles` (tile.fam = the pair's family f),
+ * tab[p * r_pad + r] = bucket of (pair_t[p] * rate_vals[fams[f].rate_off + r]) for r < n_rates of f,
+ * CHERRY_NO_BUCKET for n_rates <= r < r_pad; rows of pairs in no tile are not written.  grid: K ascending
+ * fp64 quantization points.  fp64 throughout, bit-identical to the host definition.  Built one warp per
+ * TILE (a tile's pairs share a family: its rate values are read once per warp, a pair costs one coalesced
+ * load) and quantised against precomputed decision boundaries: for neighbouring grid points (left, right)
+ * the reference's predicate t/left - 1 < right/t - 1 is monotone in t, so its switch point is found once
+ * per launch by bisection on the doubles with the predicate itself (grids with repeated or non-positive
+ * points use a binary search instead).  r_pad: a positive multiple of 4. */
 int cherry_build_bucket_table_tiles(const double* pair_t, const cherry_tile* tiles, int n_tiles,
                                     const cherry_fam_desc* fams, const double* rate_vals, const double* grid,
                                     int K, int r_pad, uint8_t* tab, void* stream);
-
-/* cherry_build_bucket_table_tiles + cherry_count_lg in one call for batches that come with tiles: the
- * bucket table is built one warp per TILE (a tile's pairs share a family, so the family's rate values
- * are read once per warp and a pair costs one coalesced load instead of the pair -> family -> rates
- * chain of cherry_build_bucket_table: 0.17 ms -> see DESIGN.md for 8.4 M pairs), then counted.  Same
- * results, bit for bit.  Every pair must belong to exactly one tile (pair_fam is implied by the tiles).
- * tab_scratch: n_pairs * r_pad bytes of device scratch (the bucket table; valid after the call).
- * Replaces the per-site quantisation inside the reference's loop
- * (counting/_count_transitions.cpp:295-307 called from :368-381). */
-int cherry_count_lg_fused(const uint8_t* msa, const cherry_fam_desc* fams, const int32_t* pair_a,
-                          const int32_t* pair_b, const double* pair_t, const int32_t* pair_fam,
-                          const double* rate_vals, const double* grid, int64_t n_pairs, int r_pad,
-                          const uint16_t* group_cat, const cherry_tile* tiles, int n_tiles, int K, int S,
-                          uint8_t* tab_scratch, unsigned long long* counts, void* stream);
 
 /* One sorted pair as the co-transition kernel's producer reads it.  16 bytes. */
 typedef struct cherry_co_rec {
@@ -143,7 +126,9 @@ typedef struct cherry_co_rec {
 } cherry_co_rec;
 
 /* Counting sort of the pairs by their bucket tab[p * r_pad] (co-transitions: one bucket per
- * pair).  order: int32 [n_pairs] (out) = pair indices grouped by bucket, ascending bucket.
+ * pair).  Reads tab[p * r_pad] for every p < n_pairs: with a table from
+ * cherry_build_bucket_table_tiles, every such pair must lie in exactly one tile.
+ * order: int32 [n_pairs] (out) = pair indices grouped by bucket, ascending bucket.
  * recs: [n_pairs] (out, may be NULL) = the row addresses of order[]'s pairs, resolved here
  * through pair_fam / fams / pair_a / pair_b.
  * ws: int32 [2 * (K + 2)] (out / scratch): ws[b] = first position of bucket b in order[],
@@ -195,7 +180,7 @@ int cherry_symmetrize_co(const uint32_t* raw, int K, int S, int directed, double
  * to counts_out on the host.  Synchronises before returning. */
 int cherry_count_lg_host(const uint8_t* msa, int64_t msa_bytes, const cherry_fam_desc* fams,
                          int n_fams, const int32_t* pair_a, const int32_t* pair_b,
-                         const double* pair_t, const int32_t* pair_fam, int64_t n_pairs,
+                         const double* pair_t, int64_t n_pairs,
                          const double* rate_vals, int64_t n_rate_vals,
                          const uint16_t* group_cat, int64_t n_groups,
                          const cherry_tile* tiles, int n_tiles, const double* grid, int K,

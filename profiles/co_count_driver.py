@@ -7,7 +7,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 
 from cherryml_b200 import _lib
-from cherryml_b200.counting._device import build_bucket_table, count_raw, sorted_grid
+from cherryml_b200.counting._device import build_bucket_table_tiles, count_raw, sorted_grid
 from cherryml_b200.synthetic import as_device_batch, quantization_grid, synthetic_co
 
 fams = int(sys.argv[1]) if len(sys.argv) > 1 else 1024
@@ -17,7 +17,7 @@ grid = quantization_grid()
 K = len(grid)
 gd = torch.from_numpy(sorted_grid(grid)).to(device)
 dev = as_device_batch(synthetic_co(fams, 1024, 300, seed=11, device=device), device)
-tab = build_bucket_table(dev, gd, K)
+tab = build_bucket_table_tiles(dev, gd, K)
 lib = _lib.load()
 order = torch.empty(dev.n_pairs, dtype=torch.int32, device=device)
 recs = torch.empty(dev.n_pairs * 16, dtype=torch.uint8, device=device)

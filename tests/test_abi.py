@@ -49,6 +49,10 @@ def test_argument_validation_without_gpu():
     lib = _lib.load()
     assert lib.cherry_count_lg(0, 0, 0, 0, 0, 4, 0, 0, 1, 10, 20, 0, 0) == -1
     assert b"null pointer" in lib.cherry_last_error()
+    assert lib.cherry_build_bucket_table_tiles(0, 0, 1, 0, 0, 0, 10, 4, 0, 0) == -1
+    assert b"null pointer" in lib.cherry_last_error()
+    assert lib.cherry_count_lg_host(0, 16, 0, 1, 0, 0, 0, 1, 0, 4, 0, 1, 0, 1, 0, 10, 20, 4, 0, 0, 0, 0) == -1
+    assert b"null pointer" in lib.cherry_last_error()
     with pytest.raises(_lib.CherryError):
         _lib.check(lib.cherry_symmetrize_lg(0, 1, 1, 0, 0, 0), "cherry_symmetrize_lg")
 

@@ -266,6 +266,7 @@ def test_full_size_properties_co():
     exp = count_batch_oracle(batch, grid, 20, False, pair_slice=sl)
     d3 = copy.copy(dev)
     d3.n_pairs = 16 * n_pairs
+    d3.n_tiles = 16 * (dev.n_tiles // n_fams)
     got = symmetrize(count_raw(d3, grid_dev, K, 20), "co", K, 20, False).cpu().numpy()
     assert np.array_equal(got, exp)
 
@@ -336,19 +337,21 @@ def test_full_size_properties_lg():
     assert np.array_equal(got, exp)
 
 
-@pytest.mark.parametrize("path", ["per_pair", "per_tile", "per_tile_repeated_grid_point"])
-def test_bucket_table_at_bucket_boundaries(path):
-    """t*rate exactly at / a few ulps around the geometric midpoints and the grid points: the
-    product-based fast comparison (per-pair kernel) must fall back to the reference expression where
-    needed, and the per-tile kernel's precomputed decision boundaries (cherry_count_lg_fused) must be the
-    reference's switch points exactly; a grid with a repeated point takes its general path."""
+@pytest.mark.parametrize("grid_kind", ["geometric", "repeated_point", "zero_point"])
+def test_bucket_table_tiles_at_bucket_boundaries(grid_kind):
+    """t*rate exactly at / a few ulps around the geometric midpoints and the grid points: the table's
+    precomputed decision boundaries must be the reference's switch points exactly; a grid with a repeated
+    or a zero point takes the binary search, whose product-based fast comparison must fall back to the
+    reference expression where needed (at zero the products tie and the quotients are infinite)."""
     from cherryml_b200 import _lib
-    from cherryml_b200.counting._device import build_bucket_table
     from oracle.native import quantization_idx_c
 
-    grid = np.array(sorted(GRID_LG))
-    if path == "per_tile_repeated_grid_point":
-        grid = np.array(sorted(list(grid) + [grid[7], grid[40]]))
+    lg = np.array(sorted(GRID_LG))
+    grid = lg
+    if grid_kind == "repeated_point":
+        grid = np.array(sorted(list(lg) + [lg[7], lg[40]]))
+    elif grid_kind == "zero_point":
+        grid = np.concatenate([[0.0], lg])
     mids = np.sqrt(grid[:-1] * grid[1:])
     near = [mids, grid]
     for base in (mids, grid):
@@ -357,23 +360,18 @@ def test_bucket_table_at_bucket_boundaries(path):
             lo, hi = np.nextafter(lo, 0), np.nextafter(hi, np.inf)
             near += [lo, hi]
     ts = np.concatenate(near + [0.5 * (grid[:-1] + grid[1:]),
-                                np.exp(np.random.default_rng(0).uniform(np.log(grid[0] / 2), np.log(grid[-1] * 2), 5000))])
+                                np.exp(np.random.default_rng(0).uniform(np.log(lg[0] / 2), np.log(lg[-1] * 2), 5000))])
     syn = synthetic_lg(1, 2 * len(ts), 16, 4, seed=0)
     syn["pair_t"] = torch.from_numpy(ts.copy())
     rates = np.array([1.0, 0.5, 3.0, 1.0 / 3.0])
     syn["rate_vals"] = rates.copy()
     dev = as_device_batch(syn, "cuda")
     grid_dev = torch.from_numpy(grid).cuda()
-    if path == "per_pair":
-        tab = build_bucket_table(dev, grid_dev, len(grid))
-    else:
-        tab = torch.full((dev.n_pairs * dev.r_pad,), 77, dtype=torch.uint8, device="cuda")
-        out = torch.zeros((len(grid), 20, 20), dtype=torch.int64, device="cuda")
-        _lib.check(_lib.load().cherry_count_lg_fused(
-            _lib.ptr(dev.msa), _lib.ptr(dev.fams), _lib.ptr(dev.pair_a), _lib.ptr(dev.pair_b), _lib.ptr(dev.pair_t),
-            _lib.ptr(dev.pair_fam), _lib.ptr(dev.rate_vals), _lib.ptr(grid_dev), dev.n_pairs, dev.r_pad,
-            _lib.ptr(dev.aux), _lib.ptr(dev.tiles), dev.n_tiles, len(grid), 20, _lib.ptr(tab), _lib.ptr(out),
-            _lib.current_stream_ptr()), "cherry_count_lg_fused")
+    tab = torch.full((dev.n_pairs * dev.r_pad,), 77, dtype=torch.uint8, device="cuda")
+    _lib.check(_lib.load().cherry_build_bucket_table_tiles(
+        _lib.ptr(dev.pair_t), _lib.ptr(dev.tiles), dev.n_tiles, _lib.ptr(dev.fams), _lib.ptr(dev.rate_vals),
+        _lib.ptr(grid_dev), len(grid), dev.r_pad, _lib.ptr(tab), _lib.current_stream_ptr()),
+        "cherry_build_bucket_table_tiles")
     tab = tab.cpu().numpy().reshape(len(ts), 4)
     for i, t in enumerate(ts):
         for r in range(4):
