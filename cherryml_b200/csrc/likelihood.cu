@@ -13,6 +13,7 @@
 // of Pt, so a warp reads 32 consecutive doubles per step of the dot product instead of 32
 // different rows; the sum over k keeps its order.
 #include <cstdint>
+#include <vector>
 
 #include "common.cuh"
 
@@ -189,6 +190,262 @@ __global__ void transpose_matrices_kernel(const double* __restrict__ in, double*
   }
 }
 
+// ---------------------------------------------------------------- edge posteriors (c = 1, S <= 32)
+//
+// Inside/outside pruning for the exact gradient of the log-likelihood.  The CTAs of one launch
+// each hold G units of ONE rate category (units sorted by category, the last CTA of a category
+// padded with dead slots), so every edge has one matrix per CTA.  Three kernels:
+//   post_fwd:    the forward pass of tree_ll_kernel (same thread mapping, same arithmetic in the
+//                same order, so ll_out is bitwise the same), which also stores per node and unit
+//                the inside vector dp_i, the message M_i to the parent, and the sum of the
+//                messages of i's EARLIER siblings (the prefix; 0 for a first child);
+//   post_bwd:    reverse post-order (a parent before its children, the children last to first);
+//                the outside vector of child i of p is O_i = A_p + prefix_i + suffix_i, suffix_i
+//                being the running sum of the messages of i's LATER siblings (a depth stack, like
+//                acc of the forward), A_root = log pi, A_i(b) = log sum_a exp(O_i(a)) P_i[a][b].
+//                No "total minus M_i": a -inf message (zero-length branch, P = I) would give
+//                -inf - -inf.  Pr(parent = a, i = b | data_u) = exp(O_i(a)) P_i[a][b]
+//                exp(dp_i(b)) obs_i(b) / L_u; the CTA sums its units in unit order and writes one
+//                S x S partial per (CTA, edge), and the root posterior per CTA;
+//   post_reduce: W[m] = sum over the (edge, category) pairs of matrix m in (edge, category)
+//                order, and over the category's CTAs in CTA order.  No atomics: two runs give
+//                bitwise-identical W and root posteriors.
+struct PostArgs {
+  const cherry_ll_node* nodes;
+  const int32_t* p_index;  // [n_nodes][n_cats]
+  const double* P;         // [n_matrices][S][S], transposed as for tree_ll_kernel
+  const uint8_t* obs;      // [n_leaves][n_units]
+  const double* pi;        // [S]
+  const int32_t* unit_of;  // [n_ctas][G]: unit of the slot, -1 for padding
+  const int32_t* cta_cat;  // [n_ctas]
+  const int32_t* cat_cta;  // [n_cats + 1]: CTAs of category k are cat_cta[k] .. cat_cta[k+1]-1
+  const int32_t* m_off;    // [n_matrices + 1]
+  const int32_t* m_ent;    // [(n_nodes - 1) * n_cats]: node * n_cats + category, grouped by matrix
+  double* dp;              // [n_ctas][n_nodes][G][S]
+  double* msg;             // [n_ctas][n_nodes][G][S]
+  double* pre;             // [n_ctas][n_nodes][G][S]
+  double* stk;             // [n_ctas][2][max_depth + 1][G][S]: forward acc / backward A, backward suffix
+  double* part;            // [n_ctas][n_nodes][S][S]
+  double* root_part;       // [n_ctas][S]
+  double* ll_out;          // [n_units]
+  double* W_out;           // [n_matrices][S][S]
+  double* root_out;        // [S]
+  int n_nodes, n_cats, S, n_units, G, max_depth, n_matrices, n_ctas;
+};
+
+__global__ void tree_ll_post_fwd_kernel(PostArgs a) {
+  extern __shared__ double w[];  // [G][S]
+  const int S = a.S;
+  const int g = threadIdx.x / S, s = threadIdx.x - g * S;
+  const int u = g < a.G ? a.unit_of[blockIdx.x * a.G + g] : -1;
+  const bool live = u >= 0;
+  const int cat = a.cta_cat[blockIdx.x];
+  const size_t gs = (size_t)a.G * S;
+  const size_t mine = (live ? g : 0) * S + s;
+  double* acc = a.stk + (size_t)blockIdx.x * 2 * (a.max_depth + 1) * gs + mine;
+  double* dp = a.dp + (size_t)blockIdx.x * a.n_nodes * gs + mine;
+  double* msg = a.msg + (size_t)blockIdx.x * a.n_nodes * gs + mine;
+  double* pre = a.pre + (size_t)blockIdx.x * a.n_nodes * gs + mine;
+  double* wg = w + (live ? g : 0) * S;
+  for (int i = 0; i < a.n_nodes; ++i) {
+    const cherry_ll_node node = a.nodes[i];
+    const bool is_leaf = node.flags & 1;
+    const bool is_root = i == a.n_nodes - 1;
+    const double* col = a.P + (is_root || !live ? 0 : (size_t)a.p_index[(size_t)i * a.n_cats + cat] * S * S) + s;
+    double m = 0.0;
+    if (!is_leaf) {
+      const double v = live ? acc[(size_t)node.depth * gs] : 0.0;
+      if (live) {
+        wg[s] = v;
+        dp[(size_t)i * gs] = v;
+      }
+      __syncthreads();
+      double mx = -INFINITY;
+      if (live)
+        for (int k = 0; k < S; ++k) mx = fmax(mx, wg[k]);
+      __syncthreads();
+      if (live) wg[s] = exp(v - mx);
+      __syncthreads();
+      if (live) {
+        double sum = 0.0;
+        if (is_root) {
+          if (s == 0) {
+            for (int k = 0; k < S; ++k) sum += a.pi[k] * wg[k];
+            a.ll_out[u] = log(fmax(sum, 0.0)) + mx;
+          }
+        } else {
+          for (int k = 0; k < S; ++k) sum += col[(size_t)k * S] * wg[k];
+          m = log(fmax(sum, 0.0)) + mx;
+        }
+      }
+      __syncthreads();
+    } else if (live) {
+      const int x = a.obs[(size_t)node.obs_row * a.n_units + u];
+      double sum = 0.0;
+      if (is_root) {
+        if (s == 0) {
+          for (int k = 0; k < S; ++k) sum += (x == S || x == k) ? a.pi[k] : 0.0;
+          a.ll_out[u] = log(fmax(sum, 0.0));
+        }
+      } else {
+        if (x != S) {
+          sum = col[(size_t)x * S];
+        } else {
+          for (int k = 0; k < S; ++k) sum += col[(size_t)k * S];
+        }
+        m = log(fmax(sum, 0.0));
+      }
+    }
+    if (live && !is_root) {
+      double* dst = acc + (size_t)(node.depth - 1) * gs;
+      const bool first = node.flags & 2;
+      pre[(size_t)i * gs] = first ? 0.0 : *dst;
+      msg[(size_t)i * gs] = m;
+      *dst = first ? m : *dst + m;
+    }
+  }
+}
+
+__global__ void tree_ll_post_bwd_kernel(PostArgs a) {
+  extern __shared__ double w[];
+  const int S = a.S, G = a.G, SS = S * S;
+  double* Pt = w;             // [S][S] the edge's matrix, transposed: Pt[b * S + a] = P[a][b]
+  double* eo = Pt + SS;       // [G][S] O_i, then exp(O_i - max O_i)
+  double* ei = eo + G * S;    // [G][S] dp_i, then exp(dp_i - max dp_i) * obs_i
+  double* sc = ei + G * S;    // [G] exp(max O_i + max dp_i - log L_u)
+  const int g = threadIdx.x / S, s = threadIdx.x - g * S;
+  const int u = g < G ? a.unit_of[blockIdx.x * G + g] : -1;
+  const bool live = u >= 0;
+  const int cat = a.cta_cat[blockIdx.x];
+  const size_t gs = (size_t)G * S;
+  const size_t mine = (live ? g : 0) * S + s;
+  double* alpha = a.stk + (size_t)blockIdx.x * 2 * (a.max_depth + 1) * gs + mine;
+  double* sfx = alpha + (size_t)(a.max_depth + 1) * gs;
+  const double* dp = a.dp + (size_t)blockIdx.x * a.n_nodes * gs + mine;
+  const double* msg = a.msg + (size_t)blockIdx.x * a.n_nodes * gs + mine;
+  const double* pre = a.pre + (size_t)blockIdx.x * a.n_nodes * gs + mine;
+  const double ll = live ? a.ll_out[u] : 0.0;
+  for (int i = a.n_nodes - 1; i >= 0; --i) {
+    const cherry_ll_node node = a.nodes[i];
+    const bool is_leaf = node.flags & 1;
+    const int x = is_leaf && live ? a.obs[(size_t)node.obs_row * a.n_units + u] : S;
+    if (i == a.n_nodes - 1) {
+      // root: A = log pi; posterior pi_a exp(dp(a)) obs(a) / L
+      double r = 0.0;
+      if (live) {
+        if (is_leaf) {
+          r = (x == S || x == s) ? a.pi[s] * exp(-ll) : 0.0;
+        } else {
+          r = a.pi[s] * exp(dp[(size_t)i * gs] - ll);
+          alpha[0] = log(a.pi[s]);
+          sfx[0] = 0.0;
+        }
+      }
+      if (threadIdx.x < G * S) eo[threadIdx.x] = r;
+      __syncthreads();
+      if ((int)threadIdx.x < S) {
+        double t = 0.0;
+        for (int h = 0; h < G; ++h) t += eo[h * S + threadIdx.x];
+        a.root_part[(size_t)blockIdx.x * S + threadIdx.x] = t;
+      }
+      __syncthreads();
+      continue;
+    }
+    const double* Pm = a.P + (size_t)a.p_index[(size_t)i * a.n_cats + cat] * SS;
+    for (int e = threadIdx.x; e < SS; e += blockDim.x) Pt[e] = Pm[e];
+    const int d = node.depth;
+    double o = 0.0, v = 0.0;
+    if (live) {
+      o = alpha[(size_t)(d - 1) * gs] + pre[(size_t)i * gs] + sfx[(size_t)(d - 1) * gs];
+      sfx[(size_t)(d - 1) * gs] = sfx[(size_t)(d - 1) * gs] + msg[(size_t)i * gs];
+      if (!is_leaf) v = dp[(size_t)i * gs];
+      eo[g * S + s] = o;
+      ei[g * S + s] = v;
+    }
+    __syncthreads();
+    double mo = -INFINITY, mi = 0.0;
+    if (live) {
+      for (int k = 0; k < S; ++k) mo = fmax(mo, eo[g * S + k]);
+      if (!is_leaf) {
+        mi = -INFINITY;
+        for (int k = 0; k < S; ++k) mi = fmax(mi, ei[g * S + k]);
+      }
+      if (mo == -INFINITY) mo = 0.0;  // L_u = 0: every posterior is 0
+      if (mi == -INFINITY) mi = 0.0;
+    }
+    __syncthreads();
+    if (threadIdx.x < G * S) {
+      eo[threadIdx.x] = live ? exp(o - mo) : 0.0;
+      ei[threadIdx.x] = !live ? 0.0 : is_leaf ? ((x == S || x == s) ? 1.0 : 0.0) : exp(v - mi);
+      if (s == 0) sc[g] = live ? exp(mo + mi - ll) : 0.0;
+    }
+    __syncthreads();
+    if (live && !is_leaf) {
+      // A_i(s) = log sum_a exp(O_i(a)) P_i[a][s]; this node's children start with an empty suffix
+      double sum = 0.0;
+      for (int k = 0; k < S; ++k) sum += eo[g * S + k] * Pt[s * S + k];
+      alpha[(size_t)d * gs] = log(fmax(sum, 0.0)) + mo;
+      sfx[(size_t)d * gs] = 0.0;
+    }
+    double* part = a.part + ((size_t)blockIdx.x * a.n_nodes + i) * SS;
+    for (int e = threadIdx.x; e < SS; e += blockDim.x) {
+      const int ra = e / S, cb = e - ra * S;
+      double t = 0.0;
+      for (int h = 0; h < G; ++h) t += eo[h * S + ra] * ei[h * S + cb] * sc[h];
+      part[e] = t * Pt[cb * S + ra];
+    }
+    __syncthreads();
+  }
+}
+
+// block m < n_matrices: W[m]; block n_matrices: the root posterior
+__global__ void tree_ll_post_reduce_kernel(PostArgs a) {
+  const int SS = a.S * a.S, e = threadIdx.x, m = blockIdx.x;
+  if (m == a.n_matrices) {
+    if (e < a.S) {
+      double t = 0.0;
+      for (int c = 0; c < a.n_ctas; ++c) t += a.root_part[(size_t)c * a.S + e];
+      a.root_out[e] = t;
+    }
+    return;
+  }
+  if (e >= SS) return;
+  double t = 0.0;
+  for (int j = a.m_off[m]; j < a.m_off[m + 1]; ++j) {
+    const int ent = a.m_ent[j];
+    const int i = ent / a.n_cats, k = ent - i * a.n_cats;
+    for (int c = a.cat_cta[k]; c < a.cat_cta[k + 1]; ++c) t += a.part[((size_t)c * a.n_nodes + i) * SS + e];
+  }
+  a.W_out[(size_t)m * SS + e] = t;
+}
+
+// Launch layout of the posterior pass, from the host copies of unit_cat and p_index.
+struct PostLayout {
+  int G = 0, n_ctas = 0;
+  size_t doubles = 0, ints = 0;  // scratch: the doubles first, then the int32 tables
+};
+
+bool post_layout(int S, int n_nodes, int max_depth, int n_cats, int n_matrices, int n_units,
+                 const int32_t* unit_cat, PostLayout* L) {
+  if (S < 1 || S > 32 || n_nodes < 1 || max_depth < 0 || n_cats < 1 || n_matrices < 1 || n_units < 0) return false;
+  if (n_units > 0 && !unit_cat) return false;
+  L->G = cherry_tree_ll_units_per_block(S, 1);
+  std::vector<int64_t> count(n_cats, 0);
+  for (int u = 0; u < n_units; ++u) {
+    if (unit_cat[u] < 0 || unit_cat[u] >= n_cats) return false;
+    ++count[unit_cat[u]];
+  }
+  int64_t ctas = 0;
+  for (int k = 0; k < n_cats; ++k) ctas += (count[k] + L->G - 1) / L->G;
+  L->n_ctas = (int)ctas;
+  const size_t gs = (size_t)L->G * S;
+  L->doubles = (size_t)ctas * (3 * (size_t)n_nodes * gs + 2 * (size_t)(max_depth + 1) * gs +
+                               (size_t)n_nodes * S * S + S);
+  L->ints = (size_t)ctas * L->G + ctas + (n_cats + 1) + (n_matrices + 1) + (size_t)(n_nodes - 1) * n_cats +
+            (size_t)n_nodes * n_cats;
+  return true;
+}
+
 }  // namespace
 
 extern "C" {
@@ -264,6 +521,111 @@ int cherry_tree_log_likelihood(const cherry_ll_node* nodes, int n_nodes, const i
   }
   tree_ll_kernel<<<blocks, threads, smem, (cudaStream_t)stream>>>(a);
   CHERRY_LAUNCH_CHECK("tree_ll_kernel");
+  return CHERRY_OK;
+}
+
+size_t cherry_tree_ll_posterior_scratch_bytes(int S, int n_nodes, int max_depth, int n_cats, int n_matrices,
+                                              int n_units, const int32_t* unit_cat) {
+  PostLayout L;
+  if (!post_layout(S, n_nodes, max_depth, n_cats, n_matrices, n_units, unit_cat, &L)) return 0;
+  return L.doubles * sizeof(double) + L.ints * sizeof(int32_t);
+}
+
+int cherry_tree_ll_posterior(const cherry_ll_node* nodes, int n_nodes, int max_depth, const int32_t* p_index,
+                             int n_cats, const double* P, int n_matrices, const uint8_t* obs, const int32_t* unit_cat,
+                             const double* pi, int S, int n_units, void* scratch, size_t scratch_bytes,
+                             double* ll_out, double* W_out, double* root_out, void* stream_) {
+  if (!nodes || !p_index || !P || !obs || !unit_cat || !pi || !scratch || !ll_out || !W_out || !root_out)
+    return cherry::fail(CHERRY_EINVAL, "null pointer");
+  if (S > 32) return cherry::fail(CHERRY_ELIMIT, "the posterior pass supports S <= 32 states (%d)", S);
+  if (n_nodes < 1 || n_cats < 1 || S < 1 || max_depth < 0 || max_depth >= n_nodes || n_matrices < 1 || n_units < 0)
+    return cherry::fail(CHERRY_EINVAL, "bad sizes");
+  for (int i = 0; i + 1 < n_nodes; ++i)  // the root's entries are never read
+    for (int k = 0; k < n_cats; ++k)
+      if (p_index[(size_t)i * n_cats + k] < 0 || p_index[(size_t)i * n_cats + k] >= n_matrices)
+        return cherry::fail(CHERRY_EINVAL, "p_index[%d] out of range", i * n_cats + k);
+  PostLayout L;
+  if (!post_layout(S, n_nodes, max_depth, n_cats, n_matrices, n_units, unit_cat, &L))
+    return cherry::fail(CHERRY_EINVAL, "unit category out of range");
+  if (scratch_bytes < L.doubles * sizeof(double) + L.ints * sizeof(int32_t))
+    return cherry::fail(CHERRY_EINVAL, "scratch too small");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  const int G = L.G, n_ctas = L.n_ctas;
+  const size_t gs = (size_t)G * S;
+
+  // host tables: slots of each category's units in unit order, categories in order; matrix -> its
+  // (node, category) pairs in (node, category) order (a counting sort)
+  std::vector<int32_t> tab(L.ints);
+  int32_t* unit_of = tab.data();
+  int32_t* cta_cat = unit_of + (size_t)n_ctas * G;
+  int32_t* cat_cta = cta_cat + n_ctas;
+  int32_t* m_off = cat_cta + n_cats + 1;
+  int32_t* m_ent = m_off + n_matrices + 1;
+  int32_t* pidx = m_ent + (size_t)(n_nodes - 1) * n_cats;
+  std::vector<int32_t> count(n_cats, 0);
+  for (int u = 0; u < n_units; ++u) ++count[unit_cat[u]];
+  cat_cta[0] = 0;
+  for (int k = 0; k < n_cats; ++k) cat_cta[k + 1] = cat_cta[k] + (count[k] + G - 1) / G;
+  std::fill(unit_of, unit_of + (size_t)n_ctas * G, -1);
+  for (int k = 0; k < n_cats; ++k)
+    for (int c = cat_cta[k]; c < cat_cta[k + 1]; ++c) cta_cat[c] = k;
+  std::vector<int32_t> fill(n_cats, 0);
+  for (int u = 0; u < n_units; ++u) {
+    const int k = unit_cat[u];
+    unit_of[(size_t)cat_cta[k] * G + fill[k]++] = u;
+  }
+  std::fill(m_off, m_off + n_matrices + 1, 0);
+  for (int i = 0; i + 1 < n_nodes; ++i)
+    for (int k = 0; k < n_cats; ++k) ++m_off[p_index[(size_t)i * n_cats + k] + 1];
+  for (int m = 0; m < n_matrices; ++m) m_off[m + 1] += m_off[m];
+  std::vector<int32_t> next(m_off, m_off + n_matrices);
+  for (int i = 0; i + 1 < n_nodes; ++i)
+    for (int k = 0; k < n_cats; ++k) m_ent[next[p_index[(size_t)i * n_cats + k]]++] = i * n_cats + k;
+  std::copy(p_index, p_index + (size_t)n_nodes * n_cats, pidx);
+
+  double* base = reinterpret_cast<double*>(scratch);
+  int32_t* dtab = reinterpret_cast<int32_t*>(base + L.doubles);
+  // pageable source: the copy is staged before cudaMemcpyAsync returns, so `tab` may go out of scope
+  CHERRY_CUDA(cudaMemcpyAsync(dtab, tab.data(), L.ints * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
+
+  PostArgs a;
+  a.nodes = nodes;
+  a.p_index = dtab + (pidx - tab.data());
+  a.P = P;
+  a.obs = obs;
+  a.pi = pi;
+  a.unit_of = dtab;
+  a.cta_cat = dtab + (cta_cat - tab.data());
+  a.cat_cta = dtab + (cat_cta - tab.data());
+  a.m_off = dtab + (m_off - tab.data());
+  a.m_ent = dtab + (m_ent - tab.data());
+  a.dp = base;
+  a.msg = a.dp + (size_t)n_ctas * n_nodes * gs;
+  a.pre = a.msg + (size_t)n_ctas * n_nodes * gs;
+  a.stk = a.pre + (size_t)n_ctas * n_nodes * gs;
+  a.part = a.stk + (size_t)n_ctas * 2 * (max_depth + 1) * gs;
+  a.root_part = a.part + (size_t)n_ctas * n_nodes * S * S;
+  a.ll_out = ll_out;
+  a.W_out = W_out;
+  a.root_out = root_out;
+  a.n_nodes = n_nodes;
+  a.n_cats = n_cats;
+  a.S = S;
+  a.n_units = n_units;
+  a.G = G;
+  a.max_depth = max_depth;
+  a.n_matrices = n_matrices;
+  a.n_ctas = n_ctas;
+  const int threads = (int)((gs + 31) / 32 * 32);
+  if (n_ctas > 0) {
+    tree_ll_post_fwd_kernel<<<n_ctas, threads, gs * sizeof(double), stream>>>(a);
+    CHERRY_LAUNCH_CHECK("tree_ll_post_fwd_kernel");
+    const size_t smem = ((size_t)S * S + 2 * gs + G) * sizeof(double);
+    tree_ll_post_bwd_kernel<<<n_ctas, threads, smem, stream>>>(a);
+    CHERRY_LAUNCH_CHECK("tree_ll_post_bwd_kernel");
+  }
+  tree_ll_post_reduce_kernel<<<n_matrices + 1, (S * S + 31) / 32 * 32, 0, stream>>>(a);
+  CHERRY_LAUNCH_CHECK("tree_ll_post_reduce_kernel");
   return CHERRY_OK;
 }
 

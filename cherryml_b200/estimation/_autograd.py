@@ -104,9 +104,13 @@ class RateMatrix(torch.nn.Module):
         self.register_buffer("_iu", iu)
         self.register_buffer("mask", torch.tensor(m, dtype=torch.float64, device=dev))
 
+    def stationary_distribution(self) -> torch.Tensor:
+        """``pi = softmax(pi_logits)``, the stationary distribution of ``forward()``'s rate matrix."""
+        return torch.softmax(self._pi, dim=0)
+
     def forward(self) -> torch.Tensor:
         S = self.num_states
-        pi = torch.softmax(self._pi, dim=0)
+        pi = self.stationary_distribution()
         sym = torch.zeros((S, S), dtype=torch.float64, device=self.upper_diag.device)
         sym[self._iu[0], self._iu[1]] = torch.nn.functional.softplus(self.upper_diag)
         sym = (sym + sym.T) * self.mask

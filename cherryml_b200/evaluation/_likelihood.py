@@ -73,18 +73,24 @@ def _encode_leaves(msa: Dict[str, str], leaves: List[str], amino_acids: List[str
 def _matrices(Q: np.ndarray, exponents: np.ndarray, device) -> Tuple[torch.Tensor, np.ndarray]:
     """One expm per distinct exponent -> (the TRANSPOSED matrices [n_distinct, S, S] on the device, as the
     pruning kernel reads them, and the index of every exponent)."""
-    lib = _lib.load()
     uniq, inverse = np.unique(exponents, return_inverse=True)
+    return _expm_transposed(Q, uniq, device), inverse.astype(np.int32)
+
+
+def _expm_transposed(Q, exponents: np.ndarray, device) -> torch.Tensor:
+    """``[K, S, S]``: ``expm(exponents[k] * Q)`` TRANSPOSED, as the pruning kernels read it (``Q``: numpy or a
+    device tensor)."""
+    lib = _lib.load()
     S = Q.shape[0]
     chunk = _PAIR_EXPM_CHUNK if S > 32 else 1 << 16
     dev = torch.device(device)
-    out = torch.empty((len(uniq), S, S), dtype=torch.float64, device=dev)
-    for i in range(0, len(uniq), chunk):
-        part = expm_batched(Q, uniq[i: i + chunk], dev)
+    out = torch.empty((len(exponents), S, S), dtype=torch.float64, device=dev)
+    for i in range(0, len(exponents), chunk):
+        part = expm_batched(Q, exponents[i: i + chunk], dev)
         with torch.cuda.device(dev):
             _lib.check(lib.cherry_tree_ll_transpose(_lib.ptr(part), part.shape[0], S, _lib.ptr(out[i: i + chunk]),
                                                     _lib.current_stream_ptr()), "cherry_tree_ll_transpose")
-    return out, inverse.astype(np.int32)
+    return out
 
 
 def _prune(nodes, max_depth, p_index, n_cats, P, obs, unit_cat, pi, S, c, device) -> np.ndarray:
@@ -182,6 +188,121 @@ def dp_likelihood_computation(
             f.write(f"Time to populate_transition_mats: {t_expm}\nTime for dp: {t_dp}\n"
                     f"Total time: {time.time() - st_all}\n")
     return sum(lls), lls
+
+
+_GRAD_CHUNK = 1 << 16  # exponents per cherry_fit_loss_grad call (one S x S gradient piece each)
+
+
+class _SiteFamily:
+    """One family's independent sites on the device, for the posterior pass: the node table, the leaf
+    residues, the distinct ``branch length * site rate`` exponents and, on the host, which of them
+    each (node, rate category) uses and the category of every site."""
+
+    def __init__(self, tree: Tree, msa: Dict[str, str], site_rates: List[float], amino_acids: List[str], device):
+        nodes, lengths, leaves, self.max_depth = _tree_arrays(tree)
+        self.S = len(amino_acids)
+        if self.S > 32:
+            raise ValueError(f"the likelihood gradient supports up to 32 states ({self.S} given)")
+        cats = sorted(set(site_rates))
+        cat_of = {r: k for k, r in enumerate(cats)}
+        exps = (lengths[:, None] * np.array(cats)[None, :]).reshape(-1)  # as dp_likelihood_computation
+        self.exponents, inverse = np.unique(exps, return_inverse=True)
+        self.p_index = np.ascontiguousarray(inverse, dtype=np.int32)
+        self.unit_cat = np.array([cat_of[r] for r in site_rates], dtype=np.int32)
+        self.n_nodes, self.n_cats, self.n_units = len(nodes), len(cats), len(site_rates)
+        dev = torch.device(device)
+        self.device = dev
+        self.nodes = torch.from_numpy(nodes.view(np.uint8).reshape(-1)).to(dev)
+        self.obs = torch.from_numpy(np.ascontiguousarray(_encode_leaves(msa, leaves, amino_acids))).to(dev)
+
+    def posterior(self, P: torch.Tensor, pi: torch.Tensor):
+        """``cherry_tree_ll_posterior`` with the transposed matrices ``P`` of ``self.exponents`` and the root
+        distribution ``pi`` (device fp64): (per-site log-likelihoods [n_units], W [n_exponents, S, S],
+        root posterior sums [S])."""
+        lib = _lib.load()
+        S, n_m = self.S, len(self.exponents)
+        with torch.cuda.device(self.device):
+            nbytes = int(lib.cherry_tree_ll_posterior_scratch_bytes(S, self.n_nodes, self.max_depth, self.n_cats, n_m,
+                                                                   self.n_units, _lib.ptr(self.unit_cat)))
+            scratch = torch.empty(max(8, nbytes), dtype=torch.uint8, device=self.device)
+            f64 = dict(dtype=torch.float64, device=self.device)
+            ll = torch.empty(max(1, self.n_units), **f64)
+            W = torch.empty((n_m, S, S), **f64)
+            root = torch.empty(S, **f64)
+            _lib.check(
+                lib.cherry_tree_ll_posterior(_lib.ptr(self.nodes), self.n_nodes, self.max_depth, _lib.ptr(self.p_index),
+                                             self.n_cats, _lib.ptr(P), n_m, _lib.ptr(self.obs),
+                                             _lib.ptr(self.unit_cat), _lib.ptr(pi), S, self.n_units,
+                                             _lib.ptr(scratch), nbytes, _lib.ptr(ll), _lib.ptr(W), _lib.ptr(root),
+                                             _lib.current_stream_ptr()),
+                "cherry_tree_ll_posterior",
+            )
+        return ll[: self.n_units], W, root
+
+
+def _q_gradient(Q: torch.Tensor, t: torch.Tensor, W: torch.Tensor) -> torch.Tensor:
+    """``d/dQ sum_m <W_m, log expm(t_m Q)>`` with ``W`` held fixed: minus the summed output of
+    ``cherry_fit_loss_grad`` with ``C = W``, in calls of at most ``_GRAD_CHUNK`` exponents that share one
+    set of buffers.  (``W_m / P_m = d log L / d P_m``, so this is the gradient of the log-likelihood.)"""
+    import ctypes
+
+    from ..estimation._engine import FitArgs
+
+    lib = _lib.load()
+    S, K = int(Q.shape[-1]), int(t.numel())
+    dev = Q.device
+    f64 = dict(dtype=torch.float64, device=dev)
+    grad = torch.zeros((S, S), **f64)
+    if K == 0:
+        return grad
+    kc = min(K, _GRAD_CHUNK)
+    nbytes = ctypes.c_size_t(0)
+    _lib.check(lib.cherry_fit_workspace_bytes(S, kc, 1, ctypes.byref(nbytes)), "cherry_fit_workspace_bytes")
+    ws = torch.empty(max(8, nbytes.value), dtype=torch.uint8, device=dev)
+    dQ = torch.empty((kc, S, S), **f64)
+    lp = torch.empty(kc, **f64)
+    flag = torch.zeros(1, dtype=torch.int32, device=dev)
+    Qc = Q.detach().contiguous()
+    a = FitArgs()
+    a.S, a.n_problems = S, 1
+    a.Q, a.dQ_part, a.loss_part = _lib.ptr(Qc), _lib.ptr(dQ), _lib.ptr(lp)
+    a.workspace, a.workspace_bytes, a.status_flag = _lib.ptr(ws), nbytes.value, _lib.ptr(flag)
+    with torch.cuda.device(dev):
+        for k0 in range(0, K, kc):
+            k = min(kc, K - k0)
+            a.K, a.t, a.C = k, _lib.ptr(t[k0:]), _lib.ptr(W[k0:])
+            _lib.check(lib.cherry_fit_loss_grad(ctypes.byref(a), _lib.current_stream_ptr()), "cherry_fit_loss_grad")
+            grad -= dQ[:k].sum(dim=0)
+    if int(flag.item()) != 0:
+        raise _lib.CherryError(f"cherry_fit_loss_grad reported status {int(flag.item())}: exponent * rate beyond "
+                               "the supported range")
+    return grad
+
+
+def log_likelihood_gradient(
+    tree: Tree,
+    msa: Dict[str, str],
+    site_rates: List[float],
+    amino_acids: List[str],
+    pi: np.ndarray,
+    Q: np.ndarray,
+    device: str = "cuda",
+) -> Tuple[float, List[float], np.ndarray, np.ndarray]:
+    """Exact log-likelihood of one family of independent sites and its gradient:
+    ``(ll, lls, d ll / d Q [S, S], d ll / d pi [S])``, every entry of ``Q`` and ``pi`` taken as a free
+    variable.  ``lls`` equals ``dp_likelihood_computation``'s per-site values bit for bit.  Edge posteriors
+    come from the inside/outside pass ``cherry_tree_ll_posterior``, the ``Q`` gradient from the fit's exact
+    expm adjoint (``cherry_fit_loss_grad``) with the posteriors as counts.  S <= 32; no CPU fallback."""
+    dev = torch.device(device if str(device).startswith("cuda") else "cuda")
+    fam = _SiteFamily(tree, msa, site_rates, amino_acids, dev)
+    Q = np.asarray(Q, dtype=np.float64)
+    P = _expm_transposed(Q, fam.exponents, dev)
+    d_pi = torch.from_numpy(np.array(pi, dtype=np.float64).reshape(-1)).to(dev)
+    ll, W, root = fam.posterior(P, d_pi)
+    t = torch.from_numpy(fam.exponents).to(dev)
+    gQ = _q_gradient(torch.from_numpy(Q).to(dev), t, W)
+    lls = [float(x) for x in ll.cpu().numpy()]
+    return sum(lls), lls, gQ.cpu().numpy(), (root / d_pi).cpu().numpy()
 
 
 @cached_parallel_computation(

@@ -496,6 +496,27 @@ int cherry_tree_log_likelihood(const cherry_ll_node* nodes, int n_nodes, const i
                                int S, int c, int n_units, int max_depth, void* scratch, size_t scratch_bytes,
                                double* ll_out, void* stream);
 
+/* Edge posteriors for the exact gradient of the log-likelihood of independent sites (c = 1,
+ * S <= 32 states, else CHERRY_ELIMIT).  Inputs as for cherry_tree_log_likelihood, except that
+ * p_index [n_nodes][n_cats] and unit_cat [n_units] are HOST arrays (the launch groups units of
+ * one rate category per CTA and orders the reduction from them); P holds n_matrices matrices and
+ * every p_index entry of a non-root node must be below n_matrices.  Outputs (device):
+ *   ll_out[u]       bitwise what cherry_tree_log_likelihood writes for c = 1;
+ *   W_out[m][a][b]  sum over units u and edges (parent(i), i) with p_index[i*n_cats + unit_cat[u]]
+ *                   = m of Pr(parent(i) = a, i = b | data_u), overwritten (zero for a matrix no
+ *                   edge uses);
+ *   root_out[a]     sum over units of Pr(root = a | data_u), overwritten.
+ * d log L / d P_m = W_m / P_m, so d log L / d Q = sum_m d/dQ <W_m, log expm(t_m Q)> with W held
+ * fixed (cherry_fit_loss_grad with C = W gives minus that), and d log L / d pi_a = root_out[a] / pi_a.
+ * No floating-point atomics: two calls give bitwise-identical outputs.  Synchronises the host
+ * with the upload of its index tables (pageable cudaMemcpyAsync); the kernels run on `stream`. */
+size_t cherry_tree_ll_posterior_scratch_bytes(int S, int n_nodes, int max_depth, int n_cats, int n_matrices,
+                                              int n_units, const int32_t* unit_cat);
+int cherry_tree_ll_posterior(const cherry_ll_node* nodes, int n_nodes, int max_depth, const int32_t* p_index,
+                             int n_cats, const double* P, int n_matrices, const uint8_t* obs, const int32_t* unit_cat,
+                             const double* pi, int S, int n_units, void* scratch, size_t scratch_bytes,
+                             double* ll_out, double* W_out, double* root_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
