@@ -100,6 +100,8 @@ int cherry_fit_loss_grad(const cherry_fit_args* a, void* stream) {
   if (a->S > cherry::kSmallFitMaxS && getenv("CHERRY_FIT_TIMELINE"))
     return cherry::fit_large_timeline(*a, (cudaStream_t)stream);
   if (a->S <= cherry::kSmallFitMaxS) return cherry::fit_small_expm(*a, (cudaStream_t)stream);
+  // an arbitrary Q (no parameters): no cherry_fit_init has prepared this workspace for this K
+  if (!a->theta && (rc = cherry::fit_large_prepare(*a, (cudaStream_t)stream))) return rc;
   return cherry::fit_large_expm(*a, (cudaStream_t)stream);
 }
 

@@ -22,6 +22,7 @@ int fit_large_workspace_bytes(int S, int K, int n_problems, size_t* bytes);
 int fit_large_expm(const cherry_fit_args& a, cudaStream_t stream, bool training = false);
 int fit_large_symmetric_form(const cherry_fit_args& a);  // 1: the training evaluations of this workspace use it
 int fit_large_forward_only(const cherry_fit_args& a, double* P_out, cudaStream_t stream);
+int fit_large_prepare(const cherry_fit_args& a, cudaStream_t stream);  // uploads the plan of (S, K) (synchronous)
 int fit_large_update(const cherry_fit_args& a, int mode, cudaStream_t stream, const double* reduced = nullptr);
 int fit_large_timeline(const cherry_fit_args& a, cudaStream_t stream);
 int fit_large_read_schedule(const cherry_fit_args& a, int* s_out, double* mu_out);

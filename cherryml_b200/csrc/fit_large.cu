@@ -28,6 +28,7 @@
 #include <unordered_map>
 #include <vector>
 
+#include "dmma.cuh"
 #include "fit_common.cuh"
 #include "fit_internal.cuh"
 
@@ -74,11 +75,6 @@ struct GemmTask {
   int term_begin, n_terms, accumulate;
 };
 
-__device__ __forceinline__ void dmma884(double& d0, double& d1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-               : "+d"(d0), "+d"(d1)
-               : "d"(a), "d"(b));
-}
 __device__ __forceinline__ void cp_async16(double* smem_dst, const double* gmem_src) {
   const unsigned s = (unsigned)__cvta_generic_to_shared(smem_dst);
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(gmem_src));

@@ -16,6 +16,7 @@
 // batched per-site variant (_siterm/_cherryml_vectorized.py:264-293, 351-383).
 #include "common.cuh"
 
+#include "dmma.cuh"
 #include "fit_common.cuh"
 
 namespace {
@@ -25,12 +26,6 @@ using cherry::kMaxSquarings;
 
 constexpr int kSmallThreads = 512;  // 16 warps: one 8x8 output tile per warp up to S = 32
 constexpr int kMaxSmallS = 32;
-
-__device__ __forceinline__ void dmma884(double& d0, double& d1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-               : "+d"(d0), "+d"(d1)
-               : "d"(a), "d"(b));
-}
 
 // D = op(A) * op(B)  (+ D if ACC), all spad x spad with leading dimension ld, operands may
 // live in shared or global memory (generic pointers).  Fragment layouts of m8n8k4:

@@ -17,9 +17,23 @@ from .. import _lib
 from ..caching import cached_parallel_computation
 from ..io import (Tree, read_contact_map, read_msa, read_probability_distribution, read_rate_matrix, read_site_rates,
                   read_tree, write_log_likelihood)
-from ..markov_chain import expm_batched
+from ..markov_chain import LARGE_MAX_K, expm_batched
 
 _PAIR_EXPM_CHUNK = 128  # 400 x 400 exponentials per cherry_expm_batched call (bounds its workspace)
+
+
+def _contact_pairs(contact_map: Optional[np.ndarray]) -> List[Tuple[int, int]]:
+    """The contacting pairs ``(i, j)``, ``i < j``, in ``np.where`` order; every site in at most one pair."""
+    if contact_map is None:
+        return []
+    ii, jj = np.where(contact_map == 1)
+    pairs = [(int(i), int(j)) for i, j in zip(ii, jj) if i < j]
+    flat = [s for p in pairs for s in p]
+    if len(set(flat)) != len(flat):
+        raise Exception(
+            f"Each site can only be in contact with one other site. The contacting sites were: {pairs}"
+        )
+    return pairs
 
 
 def _tree_arrays(tree: Tree):
@@ -80,6 +94,12 @@ def _matrices(Q: np.ndarray, exponents: np.ndarray, device) -> Tuple[torch.Tenso
 def _expm_transposed(Q, exponents: np.ndarray, device) -> torch.Tensor:
     """``[K, S, S]``: ``expm(exponents[k] * Q)`` TRANSPOSED, as the pruning kernels read it (``Q``: numpy or a
     device tensor)."""
+    return _expm_chunked(Q, exponents, device, transpose=True)
+
+
+def _expm_chunked(Q, exponents: np.ndarray, device, transpose: bool) -> torch.Tensor:
+    """``[K, S, S]``: ``expm(exponents[k] * Q)``, transposed or not, in ``cherry_expm_batched`` calls of at most
+    ``_PAIR_EXPM_CHUNK`` exponents for S > 32."""
     lib = _lib.load()
     S = Q.shape[0]
     chunk = _PAIR_EXPM_CHUNK if S > 32 else 1 << 16
@@ -87,6 +107,9 @@ def _expm_transposed(Q, exponents: np.ndarray, device) -> torch.Tensor:
     out = torch.empty((len(exponents), S, S), dtype=torch.float64, device=dev)
     for i in range(0, len(exponents), chunk):
         part = expm_batched(Q, exponents[i: i + chunk], dev)
+        if not transpose:
+            out[i: i + chunk].copy_(part)
+            continue
         with torch.cuda.device(dev):
             _lib.check(lib.cherry_tree_ll_transpose(_lib.ptr(part), part.shape[0], S, _lib.ptr(out[i: i + chunk]),
                                                     _lib.current_stream_ptr()), "cherry_tree_ll_transpose")
@@ -141,17 +164,8 @@ def dp_likelihood_computation(
     st_all = time.time()
     S = len(amino_acids)
     num_sites = len(site_rates)
-    if contact_map is not None:
-        ii, jj = np.where(contact_map == 1)
-        pairs = [(int(i), int(j)) for i, j in zip(ii, jj) if i < j]
-    else:
-        pairs = []
-    flat = [s for p in pairs for s in p]
-    if len(set(flat)) != len(flat):
-        raise Exception(
-            f"Each site can only be in contact with one other site. The contacting sites were: {pairs}"
-        )
-    in_contact = set(flat)
+    pairs = _contact_pairs(contact_map)
+    in_contact = set(s for p in pairs for s in p)
     independent = [i for i in range(num_sites) if i not in in_contact]
     device = device_1 if str(device_1).startswith("cuda") else "cuda"
 
@@ -240,6 +254,53 @@ class _SiteFamily:
         return ll[: self.n_units], W, root
 
 
+class _PairFamily:
+    """One family's contacting pairs on the device, for the pair posterior pass: the node table, the leaf
+    residues of both sites of every pair (``dp_likelihood_computation``'s pair order), the distinct branch
+    lengths and, on the host, which of them each node uses."""
+
+    def __init__(self, tree: Tree, msa: Dict[str, str], contact_map: Optional[np.ndarray], amino_acids: List[str],
+                 device):
+        nodes, lengths, leaves, self.max_depth = _tree_arrays(tree)
+        self.S = len(amino_acids)
+        if self.S > 32:
+            raise ValueError(f"the pair likelihood gradient supports up to 32 states per site ({self.S} given)")
+        self.pairs = _contact_pairs(contact_map)
+        self.exponents, inverse = np.unique(lengths, return_inverse=True)
+        self.p_index = np.ascontiguousarray(inverse, dtype=np.int32)
+        self.nodes_host = nodes
+        self.n_nodes, self.n_pairs = len(nodes), len(self.pairs)
+        enc = _encode_leaves(msa, leaves, amino_acids)
+        obs = np.stack([enc[:, [i for i, _ in self.pairs]], enc[:, [j for _, j in self.pairs]]], axis=2)
+        dev = torch.device(device)
+        self.device = dev
+        self.obs = torch.from_numpy(np.ascontiguousarray(obs, dtype=np.uint8)).to(dev)
+
+    def posterior(self, P: torch.Tensor, pi: torch.Tensor):
+        """``cherry_tree_ll_pair_posterior`` with the (not transposed) matrices ``P`` of ``self.exponents`` and the
+        root distribution ``pi`` [S^2] (device fp64): (per-pair log-likelihoods [n_pairs], W [n_exponents, S^2,
+        S^2], root posterior sums [S^2])."""
+        lib = _lib.load()
+        Su, n_m = self.S * self.S, len(self.exponents)
+        with torch.cuda.device(self.device):
+            nbytes = int(lib.cherry_tree_ll_pair_posterior_scratch_bytes(self.S, self.n_nodes, self.max_depth,
+                                                                        self.n_pairs, n_m))
+            scratch = torch.empty(max(8, nbytes), dtype=torch.uint8, device=self.device)
+            f64 = dict(dtype=torch.float64, device=self.device)
+            ll = torch.empty(max(1, self.n_pairs), **f64)
+            W = torch.empty((n_m, Su, Su), **f64)
+            root = torch.empty(Su, **f64)
+            _lib.check(
+                lib.cherry_tree_ll_pair_posterior(self.nodes_host.ctypes.data, self.n_nodes, self.max_depth,
+                                                  self.p_index.ctypes.data, _lib.ptr(P), n_m, _lib.ptr(self.obs),
+                                                  _lib.ptr(pi), self.S, self.n_pairs, _lib.ptr(scratch), nbytes,
+                                                  _lib.ptr(ll), _lib.ptr(W), _lib.ptr(root),
+                                                  _lib.current_stream_ptr()),
+                "cherry_tree_ll_pair_posterior",
+            )
+        return ll[: self.n_pairs], W, root
+
+
 def _q_gradient(Q: torch.Tensor, t: torch.Tensor, W: torch.Tensor) -> torch.Tensor:
     """``d/dQ sum_m <W_m, log expm(t_m Q)>`` with ``W`` held fixed: minus the summed output of
     ``cherry_fit_loss_grad`` with ``C = W``, in calls of at most ``_GRAD_CHUNK`` exponents that share one
@@ -255,11 +316,13 @@ def _q_gradient(Q: torch.Tensor, t: torch.Tensor, W: torch.Tensor) -> torch.Tens
     grad = torch.zeros((S, S), **f64)
     if K == 0:
         return grad
-    kc = min(K, _GRAD_CHUNK)
+    # S > 32: at most CHERRY_LARGE_FIT_MAX_K exponents per call, and only dQ_part[0] (the sum over them) is written
+    small = S <= 32
+    kc = min(K, _GRAD_CHUNK if small else LARGE_MAX_K)
     nbytes = ctypes.c_size_t(0)
     _lib.check(lib.cherry_fit_workspace_bytes(S, kc, 1, ctypes.byref(nbytes)), "cherry_fit_workspace_bytes")
     ws = torch.empty(max(8, nbytes.value), dtype=torch.uint8, device=dev)
-    dQ = torch.empty((kc, S, S), **f64)
+    dQ = torch.empty((kc if small else 1, S, S), **f64)
     lp = torch.empty(kc, **f64)
     flag = torch.zeros(1, dtype=torch.int32, device=dev)
     Qc = Q.detach().contiguous()
@@ -272,7 +335,7 @@ def _q_gradient(Q: torch.Tensor, t: torch.Tensor, W: torch.Tensor) -> torch.Tens
             k = min(kc, K - k0)
             a.K, a.t, a.C = k, _lib.ptr(t[k0:]), _lib.ptr(W[k0:])
             _lib.check(lib.cherry_fit_loss_grad(ctypes.byref(a), _lib.current_stream_ptr()), "cherry_fit_loss_grad")
-            grad -= dQ[:k].sum(dim=0)
+            grad -= dQ[:k].sum(dim=0) if small else dQ[0]
     if int(flag.item()) != 0:
         raise _lib.CherryError(f"cherry_fit_loss_grad reported status {int(flag.item())}: exponent * rate beyond "
                                "the supported range")
@@ -301,6 +364,33 @@ def log_likelihood_gradient(
     ll, W, root = fam.posterior(P, d_pi)
     t = torch.from_numpy(fam.exponents).to(dev)
     gQ = _q_gradient(torch.from_numpy(Q).to(dev), t, W)
+    lls = [float(x) for x in ll.cpu().numpy()]
+    return sum(lls), lls, gQ.cpu().numpy(), (root / d_pi).cpu().numpy()
+
+
+def pair_log_likelihood_gradient(
+    tree: Tree,
+    msa: Dict[str, str],
+    contact_map: np.ndarray,
+    amino_acids: List[str],
+    pi_2: np.ndarray,
+    Q_2: np.ndarray,
+    device: str = "cuda",
+) -> Tuple[float, List[float], np.ndarray, np.ndarray]:
+    """Exact log-likelihood of the contacting pairs of one family under the co-evolution model ``(Q_2, pi_2)``
+    on ``S^2`` pair states, and its gradient: ``(ll, lls_per_pair, d ll / d Q_2 [S^2, S^2], d ll / d pi_2
+    [S^2])``.  Pairs are ``dp_likelihood_computation``'s (``i < j`` in ``np.where(contact_map == 1)`` order);
+    the independent sites of the family are not included (``log_likelihood_gradient`` gives them).  Edge
+    posteriors come from ``cherry_tree_ll_pair_posterior``, the ``Q_2`` gradient from the fit's exact expm
+    adjoint with the posteriors as counts.  S <= 32 per site; no CPU fallback."""
+    dev = torch.device(device if str(device).startswith("cuda") else "cuda")
+    fam = _PairFamily(tree, msa, contact_map, amino_acids, dev)
+    Q = np.array(Q_2, dtype=np.float64)
+    P = _expm_chunked(Q, fam.exponents, dev, transpose=False)
+    d_pi = torch.from_numpy(np.array(pi_2, dtype=np.float64).reshape(-1)).to(dev)
+    ll, W, root = fam.posterior(P, d_pi)
+    del P
+    gQ = _q_gradient(torch.from_numpy(Q).to(dev), torch.from_numpy(fam.exponents).to(dev), W)
     lls = [float(x) for x in ll.cpu().numpy()]
     return sum(lls), lls, gQ.cpu().numpy(), (root / d_pi).cpu().numpy()
 

@@ -307,7 +307,9 @@ int cherry_fit_epoch_local(const cherry_fit_args* args, double* packed, void* st
 int cherry_fit_epoch_update(const cherry_fit_args* args, const double* packed, void* stream);
 /* One evaluation without an optimiser step (tests, evaluation): writes loss_part[p*K+k] =
  * -<C_k, log expm(t_k Q_p)> and dQ_part[p*K+k] = its gradient with respect to Q_p (S <= 32).  For S > 32
- * only the sums over k are defined: loss_part[0] holds the whole loss, dQ_part[0] the whole gradient. */
+ * only the sums over k are defined: loss_part[0] holds the whole loss, dQ_part[0] the whole gradient; with
+ * args->theta null (an arbitrary Q, no fit) the call prepares the workspace itself (synchronous), as
+ * cherry_expm_batched does. */
 int cherry_fit_loss_grad(const cherry_fit_args* args, void* stream);
 
 /* P_out[p*K + k] = expm(t[p*K + k] * Q[p]) (fp64 [S][S] each) with the fit's forward algorithm.
@@ -516,6 +518,29 @@ int cherry_tree_ll_posterior(const cherry_ll_node* nodes, int n_nodes, int max_d
                              int n_cats, const double* P, int n_matrices, const uint8_t* obs, const int32_t* unit_cat,
                              const double* pi, int S, int n_units, void* scratch, size_t scratch_bytes,
                              double* ll_out, double* W_out, double* root_out, void* stream);
+
+/* Edge posteriors for the exact gradient of the log-likelihood of pairs of contacting sites (c = 2,
+ * Su = S*S states, state S*i + j; 1 <= S <= 32, else CHERRY_ELIMIT), every pair on the same matrices
+ * (no rate categories).  nodes [n_nodes] and p_index [n_nodes] are HOST arrays (the launch builds its
+ * level schedule from them); every p_index entry of a non-root node must be below n_matrices.  P:
+ * [n_matrices][Su][Su] as cherry_expm_batched writes it (NOT transposed); obs: uint8
+ * [n_leaves][n_pairs][2] residues (S = not in the alphabet); pi: [Su].  Outputs (device):
+ *   ll_out[u]       log-likelihood of pair u (what cherry_tree_log_likelihood gives for c = 2, up to
+ *                   the order of the sums);
+ *   W_out[m][a][b]  sum over pairs and over the edges (parent(i), i) with p_index[i] = m of
+ *                   Pr(parent(i) = a, i = b | data_u), overwritten (zero for a matrix no edge uses);
+ *   root_out[a]     sum over pairs of Pr(root = a | data_u), overwritten.
+ * A pair with likelihood 0 contributes no posterior mass.  d log L / d P_m = W_m / P_m, so the Q
+ * gradient is cherry_fit_loss_grad with C = W, as for cherry_tree_ll_posterior.  The pairs are the
+ * columns of FP64 tensor-core products, so each edge matrix is read once per product for every 16
+ * pairs.  No floating-point atomics: two calls give bitwise-identical outputs.  Synchronises the host
+ * with the upload of its index tables (pageable cudaMemcpyAsync); the kernels run on `stream`.
+ * The scratch size is 0 for sizes outside these limits. */
+size_t cherry_tree_ll_pair_posterior_scratch_bytes(int S, int n_nodes, int max_depth, int n_pairs, int n_matrices);
+int cherry_tree_ll_pair_posterior(const cherry_ll_node* nodes, int n_nodes, int max_depth, const int32_t* p_index,
+                                  const double* P, int n_matrices, const uint8_t* obs, const double* pi, int S,
+                                  int n_pairs, void* scratch, size_t scratch_bytes, double* ll_out, double* W_out,
+                                  double* root_out, void* stream);
 
 #ifdef __cplusplus
 }
