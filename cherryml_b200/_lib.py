@@ -99,6 +99,10 @@ _SIGNATURES = {
     "cherry_tree_ll_posterior_scratch_bytes": (ctypes.c_size_t, [c_int, c_int, c_int, c_int, c_int, c_int, _P]),
     "cherry_tree_ll_posterior": (c_int, [_P, c_int, c_int, _P, c_int, _P, c_int, _P, _P, _P, c_int, c_int, _P,
                                          ctypes.c_size_t, _P, _P, _P, _P]),
+    "cherry_tree_ll_edge_derivatives_scratch_bytes": (ctypes.c_size_t, [c_int, c_int, c_int, c_int, c_int, c_int,
+                                                                        _P]),
+    "cherry_tree_ll_edge_derivatives": (c_int, [_P, c_int, c_int, _P, c_int, _P, c_int, _P, _P, _P, _P, c_int, c_int,
+                                                _P, ctypes.c_size_t, _P, _P, _P, _P, _P]),
     "cherry_tree_ll_pair_posterior_scratch_bytes": (ctypes.c_size_t, [c_int, c_int, c_int, c_int, c_int]),
     "cherry_tree_ll_pair_posterior": (c_int, [_P, c_int, c_int, _P, _P, c_int, _P, _P, c_int, c_int, _P,
                                               ctypes.c_size_t, _P, _P, _P, _P]),

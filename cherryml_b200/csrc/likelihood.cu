@@ -210,6 +210,12 @@ __global__ void transpose_matrices_kernel(const double* __restrict__ in, double*
 //   post_reduce: W[m] = sum over the (edge, category) pairs of matrix m in (edge, category)
 //                order, and over the category's CTAs in CTA order.  No atomics: two runs give
 //                bitwise-identical W and root posteriors.
+// Edge derivatives (post_bwd<true> + dtau_reduce): with G_u[a][b] = d log L_u / d P[a][b] =
+// exp(O_i(a)) exp(dp_i(b)) obs_i(b) / L_u and dP/dtau = QP for P = expm(tau Q),
+//     d log L_u / d tau_i = sum_ab G_u[a][b] (QP)[a][b] = sc_u sum_s (Q^T eo_u)(s) (P ei_u)(s),
+// two S-vector mat-vecs per unit and edge and no division by P (P = I is harmless).  The CTA sums
+// its units in unit order into one scalar per (CTA, edge); dtau[i][k] sums the CTAs of category k
+// in CTA order.
 struct PostArgs {
   const cherry_ll_node* nodes;
   const int32_t* p_index;  // [n_nodes][n_cats]
@@ -230,6 +236,9 @@ struct PostArgs {
   double* ll_out;          // [n_units]
   double* W_out;           // [n_matrices][S][S]
   double* root_out;        // [S]
+  const double* Q;         // [S][S], not transposed (edge derivatives only)
+  double* dpart;           // [n_ctas][n_nodes] (edge derivatives only)
+  double* dtau_out;        // [n_nodes][n_cats] (edge derivatives only)
   int n_nodes, n_cats, S, n_units, G, max_depth, n_matrices, n_ctas;
 };
 
@@ -306,6 +315,7 @@ __global__ void tree_ll_post_fwd_kernel(PostArgs a) {
   }
 }
 
+template <bool kDtau>
 __global__ void tree_ll_post_bwd_kernel(PostArgs a) {
   extern __shared__ double w[];
   const int S = a.S, G = a.G, SS = S * S;
@@ -313,6 +323,11 @@ __global__ void tree_ll_post_bwd_kernel(PostArgs a) {
   double* eo = Pt + SS;       // [G][S] O_i, then exp(O_i - max O_i)
   double* ei = eo + G * S;    // [G][S] dp_i, then exp(dp_i - max dp_i) * obs_i
   double* sc = ei + G * S;    // [G] exp(max O_i + max dp_i - log L_u)
+  double* Qs = sc + G;        // kDtau: [S][S] Q, not transposed
+  double* prod = Qs + SS;     // kDtau: [G][S] (Q^T eo)(s) * (P ei)(s)
+  double* usum = prod + G * S;  // kDtau: [G] d log L_u / d tau of the edge
+  if constexpr (kDtau)
+    for (int e = threadIdx.x; e < SS; e += blockDim.x) Qs[e] = a.Q[e];  // read after the root's barriers
   const int g = threadIdx.x / S, s = threadIdx.x - g * S;
   const int u = g < G ? a.unit_of[blockIdx.x * G + g] : -1;
   const bool live = u >= 0;
@@ -387,6 +402,16 @@ __global__ void tree_ll_post_bwd_kernel(PostArgs a) {
       alpha[(size_t)d * gs] = log(fmax(sum, 0.0)) + mo;
       sfx[(size_t)d * gs] = 0.0;
     }
+    if constexpr (kDtau) {
+      if (threadIdx.x < G * S) {  // dead slots: eo = ei = 0
+        double qo = 0.0, pe = 0.0;
+        for (int k = 0; k < S; ++k) {
+          qo += Qs[k * S + s] * eo[g * S + k];
+          pe += Pt[k * S + s] * ei[g * S + k];
+        }
+        prod[threadIdx.x] = qo * pe;
+      }
+    }
     double* part = a.part + ((size_t)blockIdx.x * a.n_nodes + i) * SS;
     for (int e = threadIdx.x; e < SS; e += blockDim.x) {
       const int ra = e / S, cb = e - ra * S;
@@ -395,6 +420,19 @@ __global__ void tree_ll_post_bwd_kernel(PostArgs a) {
       part[e] = t * Pt[cb * S + ra];
     }
     __syncthreads();
+    if constexpr (kDtau) {
+      if (threadIdx.x < G * S && s == 0) {
+        double t = 0.0;
+        for (int k = 0; k < S; ++k) t += prod[g * S + k];
+        usum[g] = t * sc[g];
+      }
+      __syncthreads();
+      if (threadIdx.x == 0) {
+        double t = 0.0;
+        for (int h = 0; h < G; ++h) t += usum[h];
+        a.dpart[(size_t)blockIdx.x * a.n_nodes + i] = t;
+      }
+    }
   }
 }
 
@@ -419,14 +457,27 @@ __global__ void tree_ll_post_reduce_kernel(PostArgs a) {
   a.W_out[(size_t)m * SS + e] = t;
 }
 
+// dtau[i][k] = sum over the CTAs of category k, in CTA order, of the (CTA, edge i) derivatives;
+// the root's row is 0
+__global__ void tree_ll_dtau_reduce_kernel(PostArgs a) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= a.n_nodes * a.n_cats) return;
+  const int i = e / a.n_cats, k = e - i * a.n_cats;
+  double t = 0.0;
+  if (i + 1 < a.n_nodes)
+    for (int c = a.cat_cta[k]; c < a.cat_cta[k + 1]; ++c) t += a.dpart[(size_t)c * a.n_nodes + i];
+  a.dtau_out[e] = t;
+}
+
 // Launch layout of the posterior pass, from the host copies of unit_cat and p_index.
 struct PostLayout {
   int G = 0, n_ctas = 0;
   size_t doubles = 0, ints = 0;  // scratch: the doubles first, then the int32 tables
 };
 
+// dtau: the edge-derivative pass, which also keeps one double per (CTA, node)
 bool post_layout(int S, int n_nodes, int max_depth, int n_cats, int n_matrices, int n_units,
-                 const int32_t* unit_cat, PostLayout* L) {
+                 const int32_t* unit_cat, bool dtau, PostLayout* L) {
   if (S < 1 || S > 32 || n_nodes < 1 || max_depth < 0 || n_cats < 1 || n_matrices < 1 || n_units < 0) return false;
   if (n_units > 0 && !unit_cat) return false;
   L->G = cherry_tree_ll_units_per_block(S, 1);
@@ -440,11 +491,121 @@ bool post_layout(int S, int n_nodes, int max_depth, int n_cats, int n_matrices, 
   L->n_ctas = (int)ctas;
   const size_t gs = (size_t)L->G * S;
   L->doubles = (size_t)ctas * (3 * (size_t)n_nodes * gs + 2 * (size_t)(max_depth + 1) * gs +
-                               (size_t)n_nodes * S * S + S);
+                               (size_t)n_nodes * S * S + S + (dtau ? (size_t)n_nodes : 0));
   L->ints = (size_t)ctas * L->G + ctas + (n_cats + 1) + (n_matrices + 1) + (size_t)(n_nodes - 1) * n_cats +
             (size_t)n_nodes * n_cats;
   return true;
 }
+
+// The host part of both posterior entry points (checks after the null checks, layout, index tables,
+// upload, launches).  Q == nullptr: the edge posteriors alone; otherwise also dtau_out.
+int tree_ll_post_launch(const cherry_ll_node* nodes, int n_nodes, int max_depth, const int32_t* p_index, int n_cats,
+                        const double* P, int n_matrices, const uint8_t* obs, const int32_t* unit_cat, const double* pi,
+                        const double* Q, int S, int n_units, void* scratch, size_t scratch_bytes, double* ll_out,
+                        double* W_out, double* root_out, double* dtau_out, cudaStream_t stream) {
+  if (S > 32) return cherry::fail(CHERRY_ELIMIT, "the posterior pass supports S <= 32 states (%d)", S);
+  if (n_nodes < 1 || n_cats < 1 || S < 1 || max_depth < 0 || max_depth >= n_nodes || n_matrices < 1 || n_units < 0)
+    return cherry::fail(CHERRY_EINVAL, "bad sizes");
+  for (int i = 0; i + 1 < n_nodes; ++i)  // the root's entries are never read
+    for (int k = 0; k < n_cats; ++k)
+      if (p_index[(size_t)i * n_cats + k] < 0 || p_index[(size_t)i * n_cats + k] >= n_matrices)
+        return cherry::fail(CHERRY_EINVAL, "p_index[%d] out of range", i * n_cats + k);
+  PostLayout L;
+  if (!post_layout(S, n_nodes, max_depth, n_cats, n_matrices, n_units, unit_cat, Q != nullptr, &L))
+    return cherry::fail(CHERRY_EINVAL, "unit category out of range");
+  if (scratch_bytes < L.doubles * sizeof(double) + L.ints * sizeof(int32_t))
+    return cherry::fail(CHERRY_EINVAL, "scratch too small");
+  const int G = L.G, n_ctas = L.n_ctas;
+  const size_t gs = (size_t)G * S;
+
+  // host tables: slots of each category's units in unit order, categories in order; matrix -> its
+  // (node, category) pairs in (node, category) order (a counting sort)
+  std::vector<int32_t> tab(L.ints);
+  int32_t* unit_of = tab.data();
+  int32_t* cta_cat = unit_of + (size_t)n_ctas * G;
+  int32_t* cat_cta = cta_cat + n_ctas;
+  int32_t* m_off = cat_cta + n_cats + 1;
+  int32_t* m_ent = m_off + n_matrices + 1;
+  int32_t* pidx = m_ent + (size_t)(n_nodes - 1) * n_cats;
+  std::vector<int32_t> count(n_cats, 0);
+  for (int u = 0; u < n_units; ++u) ++count[unit_cat[u]];
+  cat_cta[0] = 0;
+  for (int k = 0; k < n_cats; ++k) cat_cta[k + 1] = cat_cta[k] + (count[k] + G - 1) / G;
+  std::fill(unit_of, unit_of + (size_t)n_ctas * G, -1);
+  for (int k = 0; k < n_cats; ++k)
+    for (int c = cat_cta[k]; c < cat_cta[k + 1]; ++c) cta_cat[c] = k;
+  std::vector<int32_t> fill(n_cats, 0);
+  for (int u = 0; u < n_units; ++u) {
+    const int k = unit_cat[u];
+    unit_of[(size_t)cat_cta[k] * G + fill[k]++] = u;
+  }
+  std::fill(m_off, m_off + n_matrices + 1, 0);
+  for (int i = 0; i + 1 < n_nodes; ++i)
+    for (int k = 0; k < n_cats; ++k) ++m_off[p_index[(size_t)i * n_cats + k] + 1];
+  for (int m = 0; m < n_matrices; ++m) m_off[m + 1] += m_off[m];
+  std::vector<int32_t> next(m_off, m_off + n_matrices);
+  for (int i = 0; i + 1 < n_nodes; ++i)
+    for (int k = 0; k < n_cats; ++k) m_ent[next[p_index[(size_t)i * n_cats + k]]++] = i * n_cats + k;
+  std::copy(p_index, p_index + (size_t)n_nodes * n_cats, pidx);
+
+  double* base = reinterpret_cast<double*>(scratch);
+  int32_t* dtab = reinterpret_cast<int32_t*>(base + L.doubles);
+  // pageable source: the copy is staged before cudaMemcpyAsync returns, so `tab` may go out of scope
+  CHERRY_CUDA(cudaMemcpyAsync(dtab, tab.data(), L.ints * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
+
+  PostArgs a;
+  a.nodes = nodes;
+  a.p_index = dtab + (pidx - tab.data());
+  a.P = P;
+  a.obs = obs;
+  a.pi = pi;
+  a.unit_of = dtab;
+  a.cta_cat = dtab + (cta_cat - tab.data());
+  a.cat_cta = dtab + (cat_cta - tab.data());
+  a.m_off = dtab + (m_off - tab.data());
+  a.m_ent = dtab + (m_ent - tab.data());
+  a.dp = base;
+  a.msg = a.dp + (size_t)n_ctas * n_nodes * gs;
+  a.pre = a.msg + (size_t)n_ctas * n_nodes * gs;
+  a.stk = a.pre + (size_t)n_ctas * n_nodes * gs;
+  a.part = a.stk + (size_t)n_ctas * 2 * (max_depth + 1) * gs;
+  a.root_part = a.part + (size_t)n_ctas * n_nodes * S * S;
+  a.dpart = a.root_part + (size_t)n_ctas * S;
+  a.ll_out = ll_out;
+  a.W_out = W_out;
+  a.root_out = root_out;
+  a.Q = Q;
+  a.dtau_out = dtau_out;
+  a.n_nodes = n_nodes;
+  a.n_cats = n_cats;
+  a.S = S;
+  a.n_units = n_units;
+  a.G = G;
+  a.max_depth = max_depth;
+  a.n_matrices = n_matrices;
+  a.n_ctas = n_ctas;
+  const int threads = (int)((gs + 31) / 32 * 32);
+  if (n_ctas > 0) {
+    tree_ll_post_fwd_kernel<<<n_ctas, threads, gs * sizeof(double), stream>>>(a);
+    CHERRY_LAUNCH_CHECK("tree_ll_post_fwd_kernel");
+    const size_t smem = ((size_t)S * S + 2 * gs + G) * sizeof(double);
+    if (Q) {
+      tree_ll_post_bwd_kernel<true><<<n_ctas, threads, smem + ((size_t)S * S + gs + G) * sizeof(double), stream>>>(a);
+    } else {
+      tree_ll_post_bwd_kernel<false><<<n_ctas, threads, smem, stream>>>(a);
+    }
+    CHERRY_LAUNCH_CHECK("tree_ll_post_bwd_kernel");
+  }
+  tree_ll_post_reduce_kernel<<<n_matrices + 1, (S * S + 31) / 32 * 32, 0, stream>>>(a);
+  CHERRY_LAUNCH_CHECK("tree_ll_post_reduce_kernel");
+  if (Q) {
+    const int n = n_nodes * n_cats;
+    tree_ll_dtau_reduce_kernel<<<(n + 255) / 256, 256, 0, stream>>>(a);
+    CHERRY_LAUNCH_CHECK("tree_ll_dtau_reduce_kernel");
+  }
+  return CHERRY_OK;
+}
+
 
 }  // namespace
 
@@ -527,106 +688,37 @@ int cherry_tree_log_likelihood(const cherry_ll_node* nodes, int n_nodes, const i
 size_t cherry_tree_ll_posterior_scratch_bytes(int S, int n_nodes, int max_depth, int n_cats, int n_matrices,
                                               int n_units, const int32_t* unit_cat) {
   PostLayout L;
-  if (!post_layout(S, n_nodes, max_depth, n_cats, n_matrices, n_units, unit_cat, &L)) return 0;
+  if (!post_layout(S, n_nodes, max_depth, n_cats, n_matrices, n_units, unit_cat, false, &L)) return 0;
   return L.doubles * sizeof(double) + L.ints * sizeof(int32_t);
 }
 
 int cherry_tree_ll_posterior(const cherry_ll_node* nodes, int n_nodes, int max_depth, const int32_t* p_index,
                              int n_cats, const double* P, int n_matrices, const uint8_t* obs, const int32_t* unit_cat,
                              const double* pi, int S, int n_units, void* scratch, size_t scratch_bytes,
-                             double* ll_out, double* W_out, double* root_out, void* stream_) {
+                             double* ll_out, double* W_out, double* root_out, void* stream) {
   if (!nodes || !p_index || !P || !obs || !unit_cat || !pi || !scratch || !ll_out || !W_out || !root_out)
     return cherry::fail(CHERRY_EINVAL, "null pointer");
-  if (S > 32) return cherry::fail(CHERRY_ELIMIT, "the posterior pass supports S <= 32 states (%d)", S);
-  if (n_nodes < 1 || n_cats < 1 || S < 1 || max_depth < 0 || max_depth >= n_nodes || n_matrices < 1 || n_units < 0)
-    return cherry::fail(CHERRY_EINVAL, "bad sizes");
-  for (int i = 0; i + 1 < n_nodes; ++i)  // the root's entries are never read
-    for (int k = 0; k < n_cats; ++k)
-      if (p_index[(size_t)i * n_cats + k] < 0 || p_index[(size_t)i * n_cats + k] >= n_matrices)
-        return cherry::fail(CHERRY_EINVAL, "p_index[%d] out of range", i * n_cats + k);
+  return tree_ll_post_launch(nodes, n_nodes, max_depth, p_index, n_cats, P, n_matrices, obs, unit_cat, pi, nullptr, S,
+                             n_units, scratch, scratch_bytes, ll_out, W_out, root_out, nullptr, (cudaStream_t)stream);
+}
+
+size_t cherry_tree_ll_edge_derivatives_scratch_bytes(int S, int n_nodes, int max_depth, int n_cats, int n_matrices,
+                                                     int n_units, const int32_t* unit_cat) {
   PostLayout L;
-  if (!post_layout(S, n_nodes, max_depth, n_cats, n_matrices, n_units, unit_cat, &L))
-    return cherry::fail(CHERRY_EINVAL, "unit category out of range");
-  if (scratch_bytes < L.doubles * sizeof(double) + L.ints * sizeof(int32_t))
-    return cherry::fail(CHERRY_EINVAL, "scratch too small");
-  cudaStream_t stream = (cudaStream_t)stream_;
-  const int G = L.G, n_ctas = L.n_ctas;
-  const size_t gs = (size_t)G * S;
+  if (!post_layout(S, n_nodes, max_depth, n_cats, n_matrices, n_units, unit_cat, true, &L)) return 0;
+  return L.doubles * sizeof(double) + L.ints * sizeof(int32_t);
+}
 
-  // host tables: slots of each category's units in unit order, categories in order; matrix -> its
-  // (node, category) pairs in (node, category) order (a counting sort)
-  std::vector<int32_t> tab(L.ints);
-  int32_t* unit_of = tab.data();
-  int32_t* cta_cat = unit_of + (size_t)n_ctas * G;
-  int32_t* cat_cta = cta_cat + n_ctas;
-  int32_t* m_off = cat_cta + n_cats + 1;
-  int32_t* m_ent = m_off + n_matrices + 1;
-  int32_t* pidx = m_ent + (size_t)(n_nodes - 1) * n_cats;
-  std::vector<int32_t> count(n_cats, 0);
-  for (int u = 0; u < n_units; ++u) ++count[unit_cat[u]];
-  cat_cta[0] = 0;
-  for (int k = 0; k < n_cats; ++k) cat_cta[k + 1] = cat_cta[k] + (count[k] + G - 1) / G;
-  std::fill(unit_of, unit_of + (size_t)n_ctas * G, -1);
-  for (int k = 0; k < n_cats; ++k)
-    for (int c = cat_cta[k]; c < cat_cta[k + 1]; ++c) cta_cat[c] = k;
-  std::vector<int32_t> fill(n_cats, 0);
-  for (int u = 0; u < n_units; ++u) {
-    const int k = unit_cat[u];
-    unit_of[(size_t)cat_cta[k] * G + fill[k]++] = u;
-  }
-  std::fill(m_off, m_off + n_matrices + 1, 0);
-  for (int i = 0; i + 1 < n_nodes; ++i)
-    for (int k = 0; k < n_cats; ++k) ++m_off[p_index[(size_t)i * n_cats + k] + 1];
-  for (int m = 0; m < n_matrices; ++m) m_off[m + 1] += m_off[m];
-  std::vector<int32_t> next(m_off, m_off + n_matrices);
-  for (int i = 0; i + 1 < n_nodes; ++i)
-    for (int k = 0; k < n_cats; ++k) m_ent[next[p_index[(size_t)i * n_cats + k]]++] = i * n_cats + k;
-  std::copy(p_index, p_index + (size_t)n_nodes * n_cats, pidx);
-
-  double* base = reinterpret_cast<double*>(scratch);
-  int32_t* dtab = reinterpret_cast<int32_t*>(base + L.doubles);
-  // pageable source: the copy is staged before cudaMemcpyAsync returns, so `tab` may go out of scope
-  CHERRY_CUDA(cudaMemcpyAsync(dtab, tab.data(), L.ints * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
-
-  PostArgs a;
-  a.nodes = nodes;
-  a.p_index = dtab + (pidx - tab.data());
-  a.P = P;
-  a.obs = obs;
-  a.pi = pi;
-  a.unit_of = dtab;
-  a.cta_cat = dtab + (cta_cat - tab.data());
-  a.cat_cta = dtab + (cat_cta - tab.data());
-  a.m_off = dtab + (m_off - tab.data());
-  a.m_ent = dtab + (m_ent - tab.data());
-  a.dp = base;
-  a.msg = a.dp + (size_t)n_ctas * n_nodes * gs;
-  a.pre = a.msg + (size_t)n_ctas * n_nodes * gs;
-  a.stk = a.pre + (size_t)n_ctas * n_nodes * gs;
-  a.part = a.stk + (size_t)n_ctas * 2 * (max_depth + 1) * gs;
-  a.root_part = a.part + (size_t)n_ctas * n_nodes * S * S;
-  a.ll_out = ll_out;
-  a.W_out = W_out;
-  a.root_out = root_out;
-  a.n_nodes = n_nodes;
-  a.n_cats = n_cats;
-  a.S = S;
-  a.n_units = n_units;
-  a.G = G;
-  a.max_depth = max_depth;
-  a.n_matrices = n_matrices;
-  a.n_ctas = n_ctas;
-  const int threads = (int)((gs + 31) / 32 * 32);
-  if (n_ctas > 0) {
-    tree_ll_post_fwd_kernel<<<n_ctas, threads, gs * sizeof(double), stream>>>(a);
-    CHERRY_LAUNCH_CHECK("tree_ll_post_fwd_kernel");
-    const size_t smem = ((size_t)S * S + 2 * gs + G) * sizeof(double);
-    tree_ll_post_bwd_kernel<<<n_ctas, threads, smem, stream>>>(a);
-    CHERRY_LAUNCH_CHECK("tree_ll_post_bwd_kernel");
-  }
-  tree_ll_post_reduce_kernel<<<n_matrices + 1, (S * S + 31) / 32 * 32, 0, stream>>>(a);
-  CHERRY_LAUNCH_CHECK("tree_ll_post_reduce_kernel");
-  return CHERRY_OK;
+int cherry_tree_ll_edge_derivatives(const cherry_ll_node* nodes, int n_nodes, int max_depth, const int32_t* p_index,
+                                    int n_cats, const double* P, int n_matrices, const uint8_t* obs,
+                                    const int32_t* unit_cat, const double* pi, const double* Q, int S, int n_units,
+                                    void* scratch, size_t scratch_bytes, double* ll_out, double* W_out,
+                                    double* root_out, double* dtau_out, void* stream) {
+  if (!nodes || !p_index || !P || !obs || !unit_cat || !pi || !Q || !scratch || !ll_out || !W_out || !root_out ||
+      !dtau_out)
+    return cherry::fail(CHERRY_EINVAL, "null pointer");
+  return tree_ll_post_launch(nodes, n_nodes, max_depth, p_index, n_cats, P, n_matrices, obs, unit_cat, pi, Q, S,
+                             n_units, scratch, scratch_bytes, ll_out, W_out, root_out, dtau_out, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -36,15 +36,17 @@ def _contact_pairs(contact_map: Optional[np.ndarray]) -> List[Tuple[int, int]]:
     return pairs
 
 
-def _tree_arrays(tree: Tree):
+def _tree_arrays(tree: Tree, with_names: bool = False):
     """Post-order node table for the kernel + per node branch length (one iterative walk; the
-    order is ``tree.postorder_traversal()``'s: children in edge order, then their parent)."""
+    order is ``tree.postorder_traversal()``'s: children in edge order, then their parent).  With
+    ``with_names`` the node names in that order come fifth."""
     kids_of = {v: tree.children(v) for v in tree.nodes()}
     depths: List[int] = []
     flags: List[int] = []
     obs_rows: List[int] = []
     lengths: List[float] = []
     leaves: List[str] = []
+    names: List[str] = []
     stack = [(tree.root(), 0, 0.0, 0, False)]
     while stack:
         v, d, length, first, expanded = stack.pop()
@@ -56,6 +58,7 @@ def _tree_arrays(tree: Tree):
             continue
         depths.append(d)
         lengths.append(length)
+        names.append(v)
         if kids:
             flags.append(first)
             obs_rows.append(-1)
@@ -67,6 +70,8 @@ def _tree_arrays(tree: Tree):
     nodes["depth"] = depths
     nodes["flags"] = flags
     nodes["obs_row"] = obs_rows
+    if with_names:
+        return nodes, np.array(lengths, dtype=np.float64), leaves, max(depths), names
     return nodes, np.array(lengths, dtype=np.float64), leaves, max(depths)
 
 
@@ -210,18 +215,19 @@ _GRAD_CHUNK = 1 << 16  # exponents per cherry_fit_loss_grad call (one S x S grad
 class _SiteFamily:
     """One family's independent sites on the device, for the posterior pass: the node table, the leaf
     residues, the distinct ``branch length * site rate`` exponents and, on the host, which of them
-    each (node, rate category) uses and the category of every site."""
+    each (node, rate category) uses and the category of every site.  ``names`` are the nodes in the
+    table's (post) order, ``lengths`` their branch lengths (the root's is not read) and ``rates`` the
+    sorted distinct site rates; ``set_lengths`` rebuilds the exponents for new branch lengths."""
 
     def __init__(self, tree: Tree, msa: Dict[str, str], site_rates: List[float], amino_acids: List[str], device):
-        nodes, lengths, leaves, self.max_depth = _tree_arrays(tree)
+        nodes, lengths, leaves, self.max_depth, self.names = _tree_arrays(tree, with_names=True)
         self.S = len(amino_acids)
         if self.S > 32:
             raise ValueError(f"the likelihood gradient supports up to 32 states ({self.S} given)")
         cats = sorted(set(site_rates))
         cat_of = {r: k for k, r in enumerate(cats)}
-        exps = (lengths[:, None] * np.array(cats)[None, :]).reshape(-1)  # as dp_likelihood_computation
-        self.exponents, inverse = np.unique(exps, return_inverse=True)
-        self.p_index = np.ascontiguousarray(inverse, dtype=np.int32)
+        self.rates = np.array(cats, dtype=np.float64)
+        self.set_lengths(lengths)
         self.unit_cat = np.array([cat_of[r] for r in site_rates], dtype=np.int32)
         self.n_nodes, self.n_cats, self.n_units = len(nodes), len(cats), len(site_rates)
         dev = torch.device(device)
@@ -229,29 +235,52 @@ class _SiteFamily:
         self.nodes = torch.from_numpy(nodes.view(np.uint8).reshape(-1)).to(dev)
         self.obs = torch.from_numpy(np.ascontiguousarray(_encode_leaves(msa, leaves, amino_acids))).to(dev)
 
+    def set_lengths(self, lengths: np.ndarray) -> None:
+        """New branch lengths [n_nodes] in ``names`` order: ``exponents`` and ``p_index`` from them."""
+        self.lengths = np.asarray(lengths, dtype=np.float64)
+        exps = (self.lengths[:, None] * self.rates[None, :]).reshape(-1)  # as dp_likelihood_computation
+        self.exponents, inverse = np.unique(exps, return_inverse=True)
+        self.p_index = np.ascontiguousarray(inverse, dtype=np.int32)
+
     def posterior(self, P: torch.Tensor, pi: torch.Tensor):
         """``cherry_tree_ll_posterior`` with the transposed matrices ``P`` of ``self.exponents`` and the root
         distribution ``pi`` (device fp64): (per-site log-likelihoods [n_units], W [n_exponents, S, S],
         root posterior sums [S])."""
+        return self._run(P, pi, None)
+
+    def edge_derivatives(self, P: torch.Tensor, pi: torch.Tensor, Q: torch.Tensor):
+        """``cherry_tree_ll_edge_derivatives``: ``posterior``'s outputs and ``dtau`` [n_nodes, n_cats], the
+        derivative of the log-likelihood with respect to ``length * rate`` of every (edge, rate category);
+        ``Q`` [S, S] (device fp64) is the rate matrix of ``P``."""
+        return self._run(P, pi, Q)
+
+    def _run(self, P: torch.Tensor, pi: torch.Tensor, Q: Optional[torch.Tensor]):
         lib = _lib.load()
         S, n_m = self.S, len(self.exponents)
         with torch.cuda.device(self.device):
-            nbytes = int(lib.cherry_tree_ll_posterior_scratch_bytes(S, self.n_nodes, self.max_depth, self.n_cats, n_m,
-                                                                   self.n_units, _lib.ptr(self.unit_cat)))
+            sizes = (S, self.n_nodes, self.max_depth, self.n_cats, n_m, self.n_units, _lib.ptr(self.unit_cat))
+            if Q is None:
+                nbytes = int(lib.cherry_tree_ll_posterior_scratch_bytes(*sizes))
+            else:
+                nbytes = int(lib.cherry_tree_ll_edge_derivatives_scratch_bytes(*sizes))
             scratch = torch.empty(max(8, nbytes), dtype=torch.uint8, device=self.device)
             f64 = dict(dtype=torch.float64, device=self.device)
             ll = torch.empty(max(1, self.n_units), **f64)
             W = torch.empty((n_m, S, S), **f64)
             root = torch.empty(S, **f64)
-            _lib.check(
-                lib.cherry_tree_ll_posterior(_lib.ptr(self.nodes), self.n_nodes, self.max_depth, _lib.ptr(self.p_index),
-                                             self.n_cats, _lib.ptr(P), n_m, _lib.ptr(self.obs),
-                                             _lib.ptr(self.unit_cat), _lib.ptr(pi), S, self.n_units,
-                                             _lib.ptr(scratch), nbytes, _lib.ptr(ll), _lib.ptr(W), _lib.ptr(root),
-                                             _lib.current_stream_ptr()),
-                "cherry_tree_ll_posterior",
-            )
-        return ll[: self.n_units], W, root
+            head = (_lib.ptr(self.nodes), self.n_nodes, self.max_depth, _lib.ptr(self.p_index), self.n_cats,
+                    _lib.ptr(P), n_m, _lib.ptr(self.obs), _lib.ptr(self.unit_cat), _lib.ptr(pi))
+            tail = (S, self.n_units, _lib.ptr(scratch), nbytes, _lib.ptr(ll), _lib.ptr(W), _lib.ptr(root))
+            if Q is None:
+                _lib.check(lib.cherry_tree_ll_posterior(*head, *tail, _lib.current_stream_ptr()),
+                           "cherry_tree_ll_posterior")
+                return ll[: self.n_units], W, root
+            dtau = torch.empty((self.n_nodes, self.n_cats), **f64)
+            Q = Q.contiguous()
+            _lib.check(lib.cherry_tree_ll_edge_derivatives(*head, _lib.ptr(Q), *tail, _lib.ptr(dtau),
+                                                           _lib.current_stream_ptr()),
+                       "cherry_tree_ll_edge_derivatives")
+        return ll[: self.n_units], W, root, dtau
 
 
 class _PairFamily:
@@ -366,6 +395,31 @@ def log_likelihood_gradient(
     gQ = _q_gradient(torch.from_numpy(Q).to(dev), t, W)
     lls = [float(x) for x in ll.cpu().numpy()]
     return sum(lls), lls, gQ.cpu().numpy(), (root / d_pi).cpu().numpy()
+
+
+def branch_length_gradient(
+    tree: Tree,
+    msa: Dict[str, str],
+    site_rates: List[float],
+    amino_acids: List[str],
+    pi: np.ndarray,
+    Q: np.ndarray,
+    device: str = "cuda",
+) -> Tuple[float, List[float], Dict[str, float]]:
+    """Exact log-likelihood of one family of independent sites and its derivative with respect to every
+    branch length: ``(ll, lls, {child node: d ll / d length of the edge above it})``.  ``lls`` equals
+    ``dp_likelihood_computation``'s per-site values bit for bit.  One pass of
+    ``cherry_tree_ll_edge_derivatives`` gives ``d ll / d (length * rate_k)`` per edge and rate category;
+    the length derivative is their sum weighted by the rates.  S <= 32; no CPU fallback."""
+    dev = torch.device(device if str(device).startswith("cuda") else "cuda")
+    fam = _SiteFamily(tree, msa, site_rates, amino_acids, dev)
+    Q = np.array(Q, dtype=np.float64, order="C")  # the kernel reads Q row-major (a DataFrame's array is not)
+    P = _expm_transposed(Q, fam.exponents, dev)
+    d_pi = torch.from_numpy(np.array(pi, dtype=np.float64).reshape(-1)).to(dev)
+    ll, _, _, dtau = fam.edge_derivatives(P, d_pi, torch.from_numpy(Q).to(dev))
+    dlen = dtau.cpu().numpy() @ fam.rates
+    lls = [float(x) for x in ll.cpu().numpy()]
+    return sum(lls), lls, {v: float(dlen[i]) for i, v in enumerate(fam.names[:-1])}
 
 
 def pair_log_likelihood_gradient(

@@ -519,6 +519,24 @@ int cherry_tree_ll_posterior(const cherry_ll_node* nodes, int n_nodes, int max_d
                              const double* pi, int S, int n_units, void* scratch, size_t scratch_bytes,
                              double* ll_out, double* W_out, double* root_out, void* stream);
 
+/* cherry_tree_ll_posterior plus the derivative of the log-likelihood with respect to every branch
+ * exponent.  Inputs and limits as for cherry_tree_ll_posterior, plus Q: device fp64 [S][S], NOT
+ * transposed, the rate matrix the matrices P were made from (P = expm(tau Q)).  Outputs: ll_out,
+ * W_out and root_out exactly as cherry_tree_ll_posterior writes them, and (device)
+ *   dtau_out[i][k]  d log L / d tau for the edge above node i in rate category k (tau = branch length
+ *                   * rate_k), summed over that category's units; the root's row is 0.
+ * With dP/dtau = QP it is sum over units of (Q^T eo_u) . (P ei_u) (outside and inside vectors of
+ * the edge): no division by P, so zero-length branches are fine.  d log L / d length_i =
+ * sum_k rate_k dtau_out[i][k].  Null Q or dtau_out gives CHERRY_EINVAL.  No floating-point atomics:
+ * two calls give bitwise-identical outputs.  The scratch size is 0 for sizes outside the limits. */
+size_t cherry_tree_ll_edge_derivatives_scratch_bytes(int S, int n_nodes, int max_depth, int n_cats, int n_matrices,
+                                                     int n_units, const int32_t* unit_cat);
+int cherry_tree_ll_edge_derivatives(const cherry_ll_node* nodes, int n_nodes, int max_depth, const int32_t* p_index,
+                                    int n_cats, const double* P, int n_matrices, const uint8_t* obs,
+                                    const int32_t* unit_cat, const double* pi, const double* Q, int S, int n_units,
+                                    void* scratch, size_t scratch_bytes, double* ll_out, double* W_out,
+                                    double* root_out, double* dtau_out, void* stream);
+
 /* Edge posteriors for the exact gradient of the log-likelihood of pairs of contacting sites (c = 2,
  * Su = S*S states, state S*i + j; 1 <= S <= 32, else CHERRY_ELIMIT), every pair on the same matrices
  * (no rate categories).  nodes [n_nodes] and p_index [n_nodes] are HOST arrays (the launch builds its
