@@ -18,7 +18,8 @@ import numpy as np
 import torch
 
 from .. import caching
-from ..evaluation._likelihood import _expm_chunked, _expm_transposed, _PairFamily, _q_gradient, _SiteFamily
+from ..evaluation._likelihood import (_expm_chunked, _expm_transposed, _exponent_union, _PairFamily, _q_gradient,
+                                      _SiteFamily)
 from ..io import (read_contact_map, read_mask_matrix, read_msa, read_rate_matrix, read_site_rates, read_tree,
                   write_rate_matrix)
 from ._autograd import RateMatrix
@@ -42,11 +43,9 @@ class TreeLikelihoodData:
                         read_site_rates(os.path.join(site_rates_dir, f + ".txt")), amino_acids, dev)
             for f in families
         ]
-        self.exponents, inverse = np.unique(np.concatenate([f.exponents for f in self.fams]), return_inverse=True)
+        self.exponents, rows = _exponent_union(self.fams)
         self.t = torch.from_numpy(self.exponents).to(dev)
-        # per family: the rows of the union its own exponents are (sorted, distinct)
-        offs = np.cumsum([0] + [len(f.exponents) for f in self.fams])
-        self.rows = [torch.from_numpy(inverse[offs[i]: offs[i + 1]]).to(dev) for i in range(len(self.fams))]
+        self.rows = [torch.from_numpy(r).to(dev) for r in rows]
         self.n_sites = sum(f.n_units for f in self.fams)
         self.timing = {"expm": 0.0, "posterior": 0.0, "loss_grad": 0.0}
 
@@ -182,6 +181,23 @@ def _adam_best_iterate(data, num_states: int, n_units: int, initialization_path:
     return best_ll, best_Q
 
 
+def _write_stage_files(out_dir: str, states: List[str], best_Q: np.ndarray, best_ll: float, num_epochs: int,
+                       n_families: int, units: str, start: float, t_setup: float, tm: dict) -> None:
+    """A maximum-likelihood stage's ``result.txt`` (``best_Q`` labelled with ``states``), ``log_likelihood.txt``
+    and ``profiling.txt``; ``units`` describes the data (units and distinct exponents), ``start`` is the
+    stage's ``time.time()`` at entry and ``tm`` the data's phase timings."""
+    os.makedirs(out_dir, exist_ok=True)
+    write_rate_matrix(best_Q, states, os.path.join(out_dir, "result.txt"))
+    with open(os.path.join(out_dir, "log_likelihood.txt"), "w") as f:
+        f.write(f"{best_ll!r}\n")
+    total = time.time() - start
+    with open(os.path.join(out_dir, "profiling.txt"), "w") as f:
+        f.write(f"Total time: {total} seconds for {num_epochs} epochs over {n_families} families ({units})\n"
+                f"Set-up (read and encode): {t_setup}\nexpm: {tm['expm']}\nposterior: {tm['posterior']}\n"
+                f"loss_grad: {tm['loss_grad']}\n"
+                f"host and rest: {total - t_setup - tm['expm'] - tm['posterior'] - tm['loss_grad']}\n")
+
+
 @caching.cached_computation(
     output_dirs=["output_rate_matrix_dir"],
     exclude_args=["device"],
@@ -211,18 +227,8 @@ def tree_likelihood_mle(
     t_setup = time.time() - start
     best_ll, best_Q = _adam_best_iterate(data, len(amino_acids), data.n_sites, initialization_path, mask_path,
                                          num_epochs, learning_rate, dev)
-    os.makedirs(output_rate_matrix_dir, exist_ok=True)
-    write_rate_matrix(best_Q, amino_acids, os.path.join(output_rate_matrix_dir, "result.txt"))
-    with open(os.path.join(output_rate_matrix_dir, "log_likelihood.txt"), "w") as f:
-        f.write(f"{best_ll!r}\n")
-    total = time.time() - start
-    tm = data.timing
-    with open(os.path.join(output_rate_matrix_dir, "profiling.txt"), "w") as f:
-        f.write(f"Total time: {total} seconds for {num_epochs} epochs over {len(families)} families "
-                f"({data.n_sites} sites, {len(data.exponents)} distinct exponents)\n"
-                f"Set-up (read and encode): {t_setup}\nexpm: {tm['expm']}\nposterior: {tm['posterior']}\n"
-                f"loss_grad: {tm['loss_grad']}\n"
-                f"host and rest: {total - t_setup - tm['expm'] - tm['posterior'] - tm['loss_grad']}\n")
+    _write_stage_files(output_rate_matrix_dir, amino_acids, best_Q, best_ll, num_epochs, len(families),
+                       f"{data.n_sites} sites, {len(data.exponents)} distinct exponents", start, t_setup, data.timing)
 
 
 @caching.cached_computation(
@@ -257,15 +263,5 @@ def coevolution_tree_likelihood_mle(
     states = [a + b for a in amino_acids for b in amino_acids]
     best_ll, best_Q = _adam_best_iterate(data, len(states), data.n_pairs, initialization_path, mask_path,
                                          num_epochs, learning_rate, dev)
-    os.makedirs(output_rate_matrix_dir, exist_ok=True)
-    write_rate_matrix(best_Q, states, os.path.join(output_rate_matrix_dir, "result.txt"))
-    with open(os.path.join(output_rate_matrix_dir, "log_likelihood.txt"), "w") as f:
-        f.write(f"{best_ll!r}\n")
-    total = time.time() - start
-    tm = data.timing
-    with open(os.path.join(output_rate_matrix_dir, "profiling.txt"), "w") as f:
-        f.write(f"Total time: {total} seconds for {num_epochs} epochs over {len(families)} families "
-                f"({data.n_pairs} pairs, {data.n_exponents} distinct branch lengths)\n"
-                f"Set-up (read and encode): {t_setup}\nexpm: {tm['expm']}\nposterior: {tm['posterior']}\n"
-                f"loss_grad: {tm['loss_grad']}\n"
-                f"host and rest: {total - t_setup - tm['expm'] - tm['posterior'] - tm['loss_grad']}\n")
+    _write_stage_files(output_rate_matrix_dir, states, best_Q, best_ll, num_epochs, len(families),
+                       f"{data.n_pairs} pairs, {data.n_exponents} distinct branch lengths", start, t_setup, data.timing)

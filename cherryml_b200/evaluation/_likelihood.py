@@ -283,6 +283,14 @@ class _SiteFamily:
         return ll[: self.n_units], W, root, dtau
 
 
+def _exponent_union(fams: List[_SiteFamily]) -> Tuple[np.ndarray, List[np.ndarray]]:
+    """The sorted distinct exponents of all ``fams``, and per family the rows of that union its own
+    (sorted, distinct) exponents are."""
+    union, inverse = np.unique(np.concatenate([f.exponents for f in fams]), return_inverse=True)
+    offs = np.cumsum([0] + [len(f.exponents) for f in fams])
+    return union, [inverse[offs[i]: offs[i + 1]] for i in range(len(fams))]
+
+
 class _PairFamily:
     """One family's contacting pairs on the device, for the pair posterior pass: the node table, the leaf
     residues of both sites of every pair (``dp_likelihood_computation``'s pair order), the distinct branch

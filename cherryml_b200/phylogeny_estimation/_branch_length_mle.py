@@ -14,7 +14,7 @@ import numpy as np
 import torch
 
 from ..caching import cached_parallel_computation
-from ..evaluation._likelihood import _expm_transposed, _SiteFamily
+from ..evaluation._likelihood import _expm_transposed, _exponent_union, _SiteFamily
 from ..io import (Tree, read_msa, read_rate_matrix, read_site_rates, read_tree, write_log_likelihood,
                   write_site_rates, write_tree)
 from ..markov_chain import compute_stationary_distribution
@@ -52,16 +52,15 @@ class _BranchLengthData:
         lengths = [self.lengths(f) for f in range(len(self.fams))]
         for fam, ln in zip(self.fams, lengths):
             fam.set_lengths(ln)
-        union, inverse = np.unique(np.concatenate([f.exponents for f in self.fams]), return_inverse=True)
-        offs = np.cumsum([0] + [len(f.exponents) for f in self.fams])
+        union, rows = _exponent_union(self.fams)
         t1 = time.perf_counter()
         P = _expm_transposed(self.Q, union, self.dev)
         torch.cuda.synchronize(self.dev)
         t2 = time.perf_counter()
         outs = []
-        for i, fam in enumerate(self.fams):
-            rows = torch.from_numpy(inverse[offs[i]: offs[i + 1]]).to(self.dev)
-            ll, _, _, dtau = fam.edge_derivatives(P.index_select(0, rows), self.d_pi, self.d_Q)
+        for fam, r in zip(self.fams, rows):
+            P_f = P.index_select(0, torch.from_numpy(r).to(self.dev))
+            ll, _, _, dtau = fam.edge_derivatives(P_f, self.d_pi, self.d_Q)
             outs.append((ll.cpu().numpy(), dtau.cpu().numpy()))  # the copies synchronise
         t3 = time.perf_counter()
         res = []

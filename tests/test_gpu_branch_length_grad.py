@@ -1,7 +1,7 @@
 """Exact branch-length gradient of the tree log-likelihood (cherry_tree_ll_edge_derivatives) and the
 maximum-likelihood branch-length stage built on it (phylogeny_estimation.branch_length_mle).
 
-CPU: the numpy oracle (oracle.branch_length_grad_oracle.branch_length_gradient) against central finite
+CPU: the numpy oracle (oracle.likelihood_grad_oracle.branch_length_gradient) against central finite
 differences of the likelihood oracle and the pulley principle, and the new C entry point's argument checks
 and scratch formula.
 GPU: dtau and the length gradient against the oracle (1e-9 relative), ll / W / root bitwise equal to
@@ -18,11 +18,9 @@ import pytest
 
 from cherryml_b200 import _lib
 from cherryml_b200.io import Tree
-from tests._ll_cases import AA, rate_matrix
+from tests._ll_cases import (AA, DNA, _demo_family, _model, _random_msa, _random_reversible, _random_tree, _rates,
+                             _scratch_formula, _simulate_family, _synthetic_cases, _write_families, rate_matrix)
 from tests.conftest import GOLDEN
-from tests.test_gpu_tree_likelihood_grad import (DNA, _demo_family, _model, _random_msa, _random_reversible,
-                                                 _random_tree, _rates, _scratch_formula, _synthetic_cases,
-                                                 _write_families)
 
 
 def _with_length(tree: Tree, child: str, length: float) -> Tree:
@@ -48,7 +46,7 @@ def _fd_cases():
 
 @pytest.mark.parametrize("case", _fd_cases(), ids=lambda c: c[0])
 def test_oracle_length_gradient_matches_finite_differences(case):
-    from oracle.branch_length_grad_oracle import branch_length_gradient
+    from oracle.likelihood_grad_oracle import branch_length_gradient
     from oracle.likelihood_oracle import log_likelihood
 
     _, tree, msa, rates, alphabet, model = case
@@ -79,7 +77,7 @@ def _pulley_case(S, seed):
 def test_oracle_pulley_principle(S):
     """Reversible Q, pi stationary: moving the root along its two edges does not change L, so the two
     edges under a root of degree two have equal derivatives."""
-    from oracle.branch_length_grad_oracle import branch_length_gradient
+    from oracle.likelihood_grad_oracle import branch_length_gradient
 
     tree, msa, rates, alphabet = _pulley_case(S, seed=S)
     Q, pi = _random_reversible(S, seed=31)
@@ -153,7 +151,7 @@ def _gpu_both(tree, msa, rates, alphabet, pi, Q):
 
 def _check_against_oracle(tree, msa, rates, alphabet, Q, pi):
     from cherryml_b200.evaluation import branch_length_gradient, dp_likelihood_computation
-    from oracle.branch_length_grad_oracle import branch_length_gradient as oracle_gradient
+    from oracle.likelihood_grad_oracle import branch_length_gradient as oracle_gradient
 
     names, cats, post, der = _gpu_both(tree, msa, rates, alphabet, pi, Q)
     for x, y in zip(post, der[:3]):  # ll, W, root: the posterior pass's, bit for bit
@@ -226,23 +224,6 @@ def test_pulley_principle_on_gpu(S):
 
 # ------------------------------------------------------------------ GPU: the stage
 
-def _simulate(tree, Q, pi, rates, rng):
-    """Sites evolved down `tree` under (Q, pi) with the given per-site rates."""
-    from scipy.linalg import expm
-
-    L = len(rates)
-    cats = sorted(set(rates))
-    cat = np.array([cats.index(r) for r in rates])
-    states = {tree.root(): rng.choice(len(pi), L, p=pi)}
-    for v in reversed(tree.postorder_traversal()):
-        if v == tree.root():
-            continue
-        p, length = tree.parent(v)
-        cdf = np.cumsum(np.stack([expm(length * r * Q) for r in cats]), axis=2)
-        states[v] = np.minimum((rng.random(L)[:, None] > cdf[cat, states[p]]).sum(axis=1), len(pi) - 1)
-    return {v: "".join(AA[s] for s in states[v]) for v in tree.leaves()}
-
-
 def _scaled(tree, rng, sigma):
     """`tree` with every length multiplied by exp(N(0, sigma))."""
     out = Tree()
@@ -274,9 +255,7 @@ def simulated(tmp_path_factory):
     pi = compute_stationary_distribution(Q)
     truth, fams = {}, {}
     for i in range(3):
-        t = _random_tree(16, rng)
-        rates = [float(r) for r in rng.choice([0.5, 1.0, 2.0], N_SITES)]
-        msa = _simulate(t, Q, pi, rates, rng)
+        t, msa, rates = _simulate_family(Q, pi, 16, N_SITES, rng)
         truth[f"sim{i}"] = t
         fams[f"sim{i}"] = (_scaled(t, rng, 0.5), msa, rates)
     dirs = _write_families(root, fams)

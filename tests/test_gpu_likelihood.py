@@ -13,7 +13,7 @@ pytestmark = pytest.mark.gpu
 from cherryml_b200.evaluation import compute_log_likelihoods, dp_likelihood_computation
 from cherryml_b200.io import (Tree, write_msa, write_probability_distribution, write_rate_matrix, write_site_rates,
                               write_tree)
-from tests._ll_cases import AA, fasttree_kats, golden_cases
+from tests._ll_cases import AA, _caterpillar, fasttree_kats, golden_cases
 
 
 @pytest.mark.parametrize("kat", fasttree_kats(), ids=lambda k: k[0])
@@ -42,25 +42,6 @@ def test_matches_reference_function_and_oracle(i):
                                  c["pi2"], c["Q2"])
     assert abs(ll - ll_o) <= 1e-10 * abs(ll_o)
     np.testing.assert_allclose(lls, lls_o, rtol=1e-9, atol=1e-11)
-
-
-def _caterpillar(n_leaves, rng):
-    """Maximally deep tree (depth n_leaves - 1) with a multifurcation at the root."""
-    t = Tree()
-    t.add_node("n0")
-    prev = "n0"
-    for i in range(n_leaves - 1):
-        leaf, nxt = f"L{i}", f"n{i + 1}"
-        t.add_node(leaf)
-        t.add_edge(prev, leaf, float(rng.lognormal(-2, 1)))
-        if i == n_leaves - 2:
-            t.add_node(f"L{i + 1}")
-            t.add_edge(prev, f"L{i + 1}", float(rng.lognormal(-2, 1)))
-        else:
-            t.add_node(nxt)
-            t.add_edge(prev, nxt, float(rng.lognormal(-2, 1)))
-            prev = nxt
-    return t
 
 
 def test_deep_tree_many_sites_against_oracle():

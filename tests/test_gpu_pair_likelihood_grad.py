@@ -15,26 +15,12 @@ import pytest
 
 from cherryml_b200 import _lib
 from cherryml_b200.io import Tree
-from tests._ll_cases import AA, golden_cases, rate_matrix
+from tests._ll_cases import (AA, DNA, _caterpillar, _random_reversible, _random_tree, _star_of_cherries, golden_cases,
+                             rate_matrix)
 from tests.conftest import GOLDEN
-
-DNA = list("ACGT")
 
 
 # ------------------------------------------------------------------ fixtures
-
-def _random_reversible(n, seed, mask=None):
-    rng = np.random.default_rng(seed)
-    pi = rng.dirichlet(np.full(n, 5.0))
-    sym = rng.uniform(0.2, 2.0, (n, n))
-    sym = (sym + sym.T) / 2
-    if mask is not None:
-        sym = sym * mask
-    Q = sym * pi[None, :]
-    np.fill_diagonal(Q, 0.0)
-    np.fill_diagonal(Q, -Q.sum(axis=1))
-    return Q / -np.sum(pi * np.diag(Q)), pi
-
 
 def _coupled(S, seed):
     """A random reversible pair model on S^2 states that is not a product of two site models."""
@@ -42,55 +28,6 @@ def _coupled(S, seed):
 
     Q, _ = _random_reversible(S * S, seed)
     return Q, compute_stationary_distribution(Q)
-
-
-def _random_tree(n_leaves, rng, root_children=2, zero_branch=False):
-    t = Tree()
-    names = [f"L{i}" for i in range(n_leaves)]
-    t.add_nodes(names)
-    edges, pool, k = [], list(names), 0
-    while len(pool) > root_children:
-        a, b = rng.choice(len(pool), 2, replace=False)
-        p = f"n{k}"
-        k += 1
-        t.add_node(p)
-        edges += [(p, pool[a], float(rng.lognormal(-2, 0.8))), (p, pool[b], float(rng.lognormal(-2, 0.8)))]
-        pool = [x for i, x in enumerate(pool) if i not in (a, b)] + [p]
-    t.add_node("root")
-    edges += [("root", x, float(rng.lognormal(-2, 0.8))) for x in pool]
-    if zero_branch:
-        edges[0] = (edges[0][0], edges[0][1], 0.0)
-    t.add_edges(edges)
-    return t
-
-
-def _caterpillar(n_leaves, rng):
-    t = Tree()
-    t.add_node("n0")
-    prev = "n0"
-    for i in range(n_leaves - 1):
-        leaf, nxt = f"L{i}", f"n{i + 1}"
-        t.add_node(leaf)
-        t.add_edge(prev, leaf, float(rng.lognormal(-2, 1)))
-        if i == n_leaves - 2:
-            t.add_node(f"L{i + 1}")
-            t.add_edge(prev, f"L{i + 1}", float(rng.lognormal(-2, 1)))
-        else:
-            t.add_node(nxt)
-            t.add_edge(prev, nxt, float(rng.lognormal(-2, 1)))
-            prev = nxt
-    return t
-
-
-def _star_of_cherries(n_cherries, rng):
-    t = Tree()
-    t.add_node("root")
-    for c in range(n_cherries):
-        p, a, b = f"c{c}", f"c{c}a", f"c{c}b"
-        t.add_nodes([p, a, b])
-        t.add_edges([("root", p, float(rng.lognormal(-3, 1))), (p, a, float(rng.lognormal(-2, 1))),
-                     (p, b, float(rng.lognormal(-2, 1)))])
-    return t
 
 
 def _two_leaves(rng):
@@ -133,7 +70,7 @@ def _scratch_formula(S, n_nodes, n_pairs, n_matrices):
 
 @pytest.mark.parametrize("S", [2, 3, 4])
 def test_pair_oracle_matches_finite_differences(S):
-    from oracle.pair_likelihood_grad_oracle import pair_log_likelihood_gradient
+    from oracle.likelihood_grad_oracle import pair_log_likelihood_gradient
     from oracle.likelihood_oracle import log_likelihood
 
     rng = np.random.default_rng(S)
@@ -179,8 +116,7 @@ def _pi_block_sums(g2, pi, S):
 
 def test_pair_oracle_reduces_to_sites_under_product_model():
     from cherryml_b200.markov_chain import chain_product
-    from oracle.likelihood_grad_oracle import log_likelihood_gradient
-    from oracle.pair_likelihood_grad_oracle import pair_log_likelihood_gradient
+    from oracle.likelihood_grad_oracle import log_likelihood_gradient, pair_log_likelihood_gradient
 
     rng = np.random.default_rng(3)
     S = 4
@@ -290,7 +226,7 @@ def _rel(a, b):
 @pytest.mark.parametrize("case", _oracle_cases(), ids=lambda c: c[0])
 def test_pair_posterior_and_gradient_against_oracle(case):
     from cherryml_b200.evaluation import pair_log_likelihood_gradient
-    from oracle.pair_likelihood_grad_oracle import pair_log_likelihood_gradient as oracle_gradient
+    from oracle.likelihood_grad_oracle import pair_log_likelihood_gradient as oracle_gradient
 
     _, tree, alphabet, n_pairs, kind = case
     rng = np.random.default_rng(n_pairs)
