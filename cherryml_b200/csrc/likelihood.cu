@@ -45,7 +45,7 @@ __device__ __forceinline__ void ll_stage_batch(uint32_t stage_u32, uint32_t slot
   asm volatile("cp.async.commit_group;" ::: "memory");
 }
 
-__global__ void tree_ll_kernel(LlArgs a) {
+__device__ __forceinline__ void tree_ll_body(const LlArgs& a) {
   extern __shared__ double w[];  // [G][Su], then [G][32] partial maxima, then (Su > 64) the staging slots
   double* red = w + (size_t)a.G * a.Su;
   double* stage = red + (size_t)a.G * 32 + threadIdx.x;  // [2][kLlBatch][blockDim.x], this thread's column
@@ -173,6 +173,13 @@ __global__ void tree_ll_kernel(LlArgs a) {
     }
   }
 }
+
+__global__ void tree_ll_kernel(LlArgs a) { tree_ll_body(a); }
+
+// The same pass for CTAs beyond tree_ll_kernel's register budget: it takes 96 registers a thread, so 64 K
+// registers hold 672 threads, fewer than the G * Su of a pair model with S >= 26 (Su >= 676).  Held to 64
+// registers, it launches up to 1024 threads.
+__global__ void __launch_bounds__(1024) tree_ll_wide_kernel(LlArgs a) { tree_ll_body(a); }
 
 // out[m][k][s] = in[m][s][k], 32 x 32 tiles through shared memory (both sides coalesced)
 __global__ void transpose_matrices_kernel(const double* __restrict__ in, double* __restrict__ out, int Su) {
@@ -673,14 +680,24 @@ int cherry_tree_log_likelihood(const cherry_ll_node* nodes, int n_nodes, const i
   size_t smem = (size_t)a.G * (Su + 32) * sizeof(double);
   const size_t staging = (size_t)2 * kLlBatch * threads * sizeof(double);
   a.staged = Su > 64 && smem + staging <= 227 * 1024;
+  // tree_ll_kernel's largest launchable CTA, which its register count decides (0 if unknown: always wide)
+  static const int narrow_max_threads = [] {
+    cudaFuncAttributes attr;
+    return cudaFuncGetAttributes(&attr, tree_ll_kernel) == cudaSuccess ? attr.maxThreadsPerBlock : 0;
+  }();
+  const bool wide = threads > narrow_max_threads;
   if (a.staged) {
     smem += staging;
-    const int rc = cherry::check_cuda(
-        cudaFuncSetAttribute(tree_ll_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024),
-        "cudaFuncSetAttribute(tree_ll_kernel)");
+    const int rc = cherry::check_cuda(cudaFuncSetAttribute(wide ? tree_ll_wide_kernel : tree_ll_kernel,
+                                                           cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024),
+                                      "cudaFuncSetAttribute(tree_ll_kernel)");
     if (rc != 0) return rc;
   }
-  tree_ll_kernel<<<blocks, threads, smem, (cudaStream_t)stream>>>(a);
+  if (wide) {
+    tree_ll_wide_kernel<<<blocks, threads, smem, (cudaStream_t)stream>>>(a);
+  } else {
+    tree_ll_kernel<<<blocks, threads, smem, (cudaStream_t)stream>>>(a);
+  }
   CHERRY_LAUNCH_CHECK("tree_ll_kernel");
   return CHERRY_OK;
 }
